@@ -20,6 +20,9 @@ same metagenome (different reads, same strains/sites).
 `e2e_bam` : a synthetic coordinate-sorted BAM of the same reads (bounded sample) through util.load_from_bam:
             reads/s with the per-stage seconds (file read, inflate, record scan, depth cap, CIGAR walks, gather,
             GPU ingestion).
+
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs) as .npy files, so that two builds
+can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -34,6 +37,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: the bench leaves it as the build left it
 
 import numpy as np  # noqa: E402
 
@@ -41,6 +45,7 @@ from gretel_b200 import synth  # noqa: E402
 
 METRIC = "snp_pair_observations_per_sec"
 UNIT = "obs/s"
+DUMP_BYTES = 64 << 20                   # --dump-outputs: budget of all files together
 
 
 def b_obs(k_mean):
@@ -255,6 +260,29 @@ def recovery_cpu_baseline(device):
 
 
 # ----------------------------------------------------------------------------------- our arm
+def dump_outputs(out_dir, h, N, W):
+    """What the last timed step left in ``h``, as the caller of the ingestion receives it: ``totals.npy`` (slices,
+    crumbs, covered SNPs, sentinel increments) and ``band.npy``, the step's counts as the float32 band [N+2][W][7][7]
+    that Hansel.band() returns once they are folded into an empty matrix.  The counts are copied without folding
+    them, so the rest of the run is unchanged.  A band over the budget keeps a fixed, seeded sample of its rows;
+    ``band_rows.npy`` lists the rows kept."""
+    import torch
+    from gretel_b200 import dist as gdist
+    totals = np.array(h.ingest_totals(), dtype=np.float64)
+    cptr, cn, _, _ = h.counts_buffer()
+    assert cn == (N + 2) * W * 49, "pending counts do not have the band's shape"
+    cnt = torch.as_tensor(gdist._DevBuf(cptr, cn, "<i4"), device=torch.device("cuda", h.device)).cpu().numpy()
+    cnt = cnt.view(np.uint32).reshape(N + 2, W, 7, 7)
+    rows = np.arange(N + 2)
+    fit = (DUMP_BYTES - (1 << 20)) // (W * 49 * 4)      # 1 MB left for the row list, the totals and the headers
+    if fit < N + 2:
+        rows = np.sort(np.random.default_rng(20260000).choice(N + 2, size=fit, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "band.npy"), cnt[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "band_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "totals.npy"), totals)
+
+
 def measure_other_config(name, args, device):
     """One more BASELINE.json ingestion config on this GPU: inputs resident, K steps of clear + pair expansion timed with
     CUDA events on the library's stream, then the independent per-row recount (as parity_probe)."""
@@ -522,6 +550,8 @@ def run_ours(args):
         step_ms = [a.elapsed_time(b) for a, b in ev]
         total_ms = float(sum(step_ms))
         serial_ms = None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, h, N, W)
     # kernel-only duration (events inside the library, on the launching stream) for the roofline
     for _ in range(3):
         h.reset_counts()
@@ -615,7 +645,7 @@ def run_ours(args):
             dt = float(tt.item())
         return crumbs * steps / dt, dt / steps
 
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     # (the 1 kHz NVML sampling thread stays off here: its driver calls delay the ~100 CUDA API calls of a step; the
     # clocks line describes the device-timed region above)
     e2e_value, e2e_step_s = time_e2e(args.e2e_format, e2e_steps)
@@ -914,7 +944,13 @@ def main():
     ap.add_argument("--no-other-configs", dest="other_configs", action="store_false", default=True,
                     help="skip the device-timed figures of configs[1] (HIV-like) and configs[3] (ONT-like) in the default line")
     ap.add_argument("--ref-sample", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the last step's totals and counts as .npy files into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm keeps no outputs")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -30,7 +30,9 @@ def needs_build():
     if not os.path.exists(LIB_PATH):
         return True
     t = os.path.getmtime(LIB_PATH)
-    deps = [os.path.join(_HERE, "csrc", f) for f in os.listdir(os.path.join(_HERE, "csrc"))]
+    # sources only: build_lib writes csrc/ptxas.log after the library, which must not make it stale
+    deps = [os.path.join(_HERE, "csrc", f) for f in os.listdir(os.path.join(_HERE, "csrc"))
+            if f.endswith((".cu", ".cuh", ".cpp", ".h"))]
     deps.append(os.path.join(_ROOT, "include", "hanselx.h"))
     return any(os.path.getmtime(d) > t for d in deps)
 

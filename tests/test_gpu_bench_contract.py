@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -38,6 +39,41 @@ def test_bench_line_contract():
     b = j["e2e_bam"]
     assert b["reads_per_s"] > 0 and b["same_totals_as_packed_arrays"] and 0 < b["gpu_share"] < 1
     assert set(b["stage_seconds"]) >= {"read", "inflate", "scan", "walk", "gather", "gpu_ingest"}
+
+
+def _dumped(d):
+    names = sorted(os.listdir(d))
+    assert names == ["band.npy", "band_rows.npy", "totals.npy"]
+    assert sum(os.path.getsize(os.path.join(d, n)) for n in names) <= 64 << 20
+    return {n[:-4]: np.load(os.path.join(d, n)) for n in names}
+
+
+def test_dump_outputs(tmp_path):
+    """--dump-outputs writes the last timed step's totals and counts, identical from run to run."""
+    args = ("--reads", "200000", "--steps", "2", "--warmup", "1", "--recover-paths", "0", "--no-cpu-baseline",
+            "--bam-reads", "0")
+    j = _run(*args, "--dump-outputs", str(tmp_path / "a"))
+    _run(*args, "--dump-outputs", str(tmp_path / "b"))
+    a, b = _dumped(tmp_path / "a"), _dumped(tmp_path / "b")
+    assert a["band"].dtype == np.float32 and a["totals"].dtype == np.float64 and a["band_rows"].dtype == np.float64
+    assert j["steps"] == 2 and j["e2e"]["steps"] == 2
+    assert a["band"].shape == (j["parity_probe"]["rows"], j["band_w"], 7, 7)
+    assert np.array_equal(a["band_rows"], np.arange(j["parity_probe"]["rows"]))
+    assert a["totals"][1] == j["observations_per_step"] == j["parity_probe"]["n_crumbs"]
+    assert a["band"].sum(dtype=np.float64) == j["parity_probe"]["band_sum"]
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+
+
+def test_dump_outputs_samples_a_large_band(tmp_path):
+    """A band over 64 MB (80 SNPs per read: band_w 110, 206 MB) is cut to a seeded sample of whole rows."""
+    j = _run("--workload", "mid", "--reads", "20000", "--steps", "1", "--warmup", "1", "--recover-paths", "0",
+             "--no-cpu-baseline", "--bam-reads", "0", "--dump-outputs", str(tmp_path))
+    d = _dumped(tmp_path)
+    rows = d["band_rows"].astype(np.int64)
+    assert 0 < len(rows) < j["parity_probe"]["rows"] and np.all(np.diff(rows) > 0)
+    assert d["band"].shape == (len(rows), j["band_w"], 7, 7) and d["band"].sum() > 0
+    assert d["totals"][1] == j["observations_per_step"]
 
 
 def test_reference_arm_contract():
