@@ -141,31 +141,17 @@ void free_all(hx_matrix *h) {
     hx_l2_free(h);
     hx_wire_free(h);
     if (h->d_peer_tbl) cudaFree(h->d_peer_tbl);
-    if (h->band) cudaFreeAsync(h->band, h->stream);
+    cudaStream_t st = h->stream;
+    h->band.release(st);
     release_counts(h);
-    if (h->d_totals) cudaFreeAsync(h->d_totals, h->stream);
-    if (h->d_err) cudaFreeAsync(h->d_err, h->stream);
-    if (h->s_rank) cudaFreeAsync(h->s_rank, h->stream);
-    if (h->s_off) cudaFreeAsync(h->s_off, h->stream);
-    if (h->s_codes) cudaFreeAsync(h->s_codes, h->stream);
-    if (h->s_klen) cudaFreeAsync(h->s_klen, h->stream);
-    if (h->s_codes4) cudaFreeAsync(h->s_codes4, h->stream);
-    if (h->s_scan) cudaFreeAsync(h->s_scan, h->stream);
-    if (h->scnt) cudaFreeAsync(h->scnt, h->stream);
-    if (h->vseen) cudaFreeAsync(h->vseen, h->stream);
-    if (h->d_path) cudaFreeAsync(h->d_path, h->stream);
-    if (h->d_stats) cudaFreeAsync(h->d_stats, h->stream);
-    if (h->d_site) cudaFreeAsync(h->d_site, h->stream);
-    if (h->d_partials) cudaFreeAsync(h->d_partials, h->stream);
-    if (h->d_spec) cudaFreeAsync(h->d_spec, h->stream);
-    if (h->d_terms) cudaFreeAsync(h->d_terms, h->stream);
-    if (h->d_flags) cudaFreeAsync(h->d_flags, h->stream);
-    if (h->d_run_end) cudaFreeAsync(h->d_run_end, h->stream);
-    if (h->d_run_list) cudaFreeAsync(h->d_run_list, h->stream);
-    if (h->d_jobs) cudaFreeAsync(h->d_jobs, h->stream);
-    if (h->d_misc) cudaFreeAsync(h->d_misc, h->stream);
-    if (h->d_pack) cudaFreeAsync(h->d_pack, h->stream);
-    if (h->stream) cudaStreamSynchronize(h->stream);
+    h->d_totals.release(st); h->d_err.release(st);
+    h->s_rank.release(st); h->s_off.release(st); h->s_codes.release(st);
+    h->s_klen.release(st); h->s_codes4.release(st); h->s_scan.release(st);
+    h->scnt.release(st); h->vseen.release(st); h->d_path.release(st); h->d_stats.release(st); h->d_site.release(st);
+    h->d_partials.release(st); h->d_spec.release(st); h->d_terms.release(st); h->d_flags.release(st);
+    h->d_run_end.release(st); h->d_run_list.release(st); h->d_jobs.release(st); h->d_misc.release(st);
+    h->d_pack.release(st);
+    if (st) cudaStreamSynchronize(st);
     free(h->h_pinned);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
@@ -235,18 +221,11 @@ bool park(hx_matrix *h) {
 
 int reset_parked(hx_matrix *h) {
     HX_CUDA(cudaSetDevice(h->device));
-    HX_CUDA(hx_fill_async(h->band, 0, sizeof(float) * (size_t)h->band_elems, h->stream));
-    HX_CUDA(hx_fill_async(h->d_totals, 0, 8 * sizeof(unsigned long long), h->stream));
-    HX_CUDA(hx_fill_async(h->d_err, 0, sizeof(int), h->stream));
-    HX_CUDA(hx_fill_async(h->d_flags, 0, 8 * sizeof(int), h->stream));
-    h->counts_dirty = true;
-    h->ev_rec = false;
-    h->launches = 0;
-    h->ingest_kernel = 0;
-    h->ingest_sms = 0;
-    h->wire_next = 0;
-    h->sum_busy[0] = h->sum_busy[1] = false;
-    h->last_ms[0] = h->last_ms[1] = h->last_ms[2] = 0.0f;
+    HX_CUDA(hx_fill_async(h->band.p, 0, sizeof(float) * (size_t)h->band_elems, h->stream));
+    HX_CUDA(hx_fill_async(h->d_totals.p, 0, 8 * sizeof(unsigned long long), h->stream));
+    HX_CUDA(hx_fill_async(h->d_err.p, 0, sizeof(int), h->stream));
+    HX_CUDA(hx_fill_async(h->d_flags.p, 0, 8 * sizeof(int), h->stream));
+    h->use = {};
     return HX_OK;
 }
 }  // namespace
@@ -269,7 +248,7 @@ int hx_create(int32_t n_snps, int32_t band_w, int32_t device, hx_matrix **out) {
     h->W = band_w;
     h->device = device;
     h->band_elems = ((int64_t)n_snps + 2) * band_w * HX_CELL;
-    h->counts_dirty = true;
+    h->use = {};
 #define HX_TRY(call)                                                                     \
     do {                                                                                 \
         cudaError_t e__ = (call);                                                        \
@@ -290,20 +269,20 @@ int hx_create(int32_t n_snps, int32_t band_w, int32_t device, hx_matrix **out) {
     h->own_stream = true;
     HX_TRY(cudaEventCreate(&h->ev0));
     HX_TRY(cudaEventCreate(&h->ev1));
-    HX_TRY(cudaMallocAsync((void **)&h->band, sizeof(float) * (size_t)h->band_elems, h->stream));
-    HX_TRY(hx_fill_async(h->band, 0, sizeof(float) * (size_t)h->band_elems, h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->d_totals, 8 * sizeof(unsigned long long), h->stream));
-    HX_TRY(hx_fill_async(h->d_totals, 0, 8 * sizeof(unsigned long long), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->d_err, sizeof(int), h->stream));
-    HX_TRY(hx_fill_async(h->d_err, 0, sizeof(int), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->scnt, sizeof(double) * 8 * ((size_t)n_snps + 2), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->vseen, sizeof(int32_t) * ((size_t)n_snps + 2), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->d_site, sizeof(double) * 6 * ((size_t)n_snps + 2), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->d_flags, 8 * sizeof(int), h->stream));
-    HX_TRY(hx_fill_async(h->d_flags, 0, 8 * sizeof(int), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->d_misc, 32 * sizeof(double), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->d_run_end, sizeof(int64_t) * ((size_t)n_snps + 2), h->stream));
-    HX_TRY(cudaMallocAsync((void **)&h->d_run_list, sizeof(int64_t) * (((size_t)n_snps + 3) / 2 + (size_t)n_snps + 2 + 2), h->stream));
+    HX_TRY(h->band.grow(sizeof(float) * (size_t)h->band_elems, h->stream));
+    HX_TRY(hx_fill_async(h->band.p, 0, sizeof(float) * (size_t)h->band_elems, h->stream));
+    HX_TRY(h->d_totals.grow(8 * sizeof(unsigned long long), h->stream));
+    HX_TRY(hx_fill_async(h->d_totals.p, 0, 8 * sizeof(unsigned long long), h->stream));
+    HX_TRY(h->d_err.grow(sizeof(int), h->stream));
+    HX_TRY(hx_fill_async(h->d_err.p, 0, sizeof(int), h->stream));
+    HX_TRY(h->scnt.grow(sizeof(double) * 8 * ((size_t)n_snps + 2), h->stream));
+    HX_TRY(h->vseen.grow(sizeof(int32_t) * ((size_t)n_snps + 2), h->stream));
+    HX_TRY(h->d_site.grow(sizeof(double) * 6 * ((size_t)n_snps + 2), h->stream));
+    HX_TRY(h->d_flags.grow(8 * sizeof(int), h->stream));
+    HX_TRY(hx_fill_async(h->d_flags.p, 0, 8 * sizeof(int), h->stream));
+    HX_TRY(h->d_misc.grow(32 * sizeof(double), h->stream));
+    HX_TRY(h->d_run_end.grow(sizeof(int64_t) * ((size_t)n_snps + 2), h->stream));
+    HX_TRY(h->d_run_list.grow(sizeof(int64_t) * (((size_t)n_snps + 3) / 2 + (size_t)n_snps + 2 + 2), h->stream));
     h->h_pinned = calloc(1, 256);     // scalars come back through pageable memory: a pinned allocation per
                                       // matrix costs more (cudaMallocHost/cudaFreeHost) than it saves
     if (!h->h_pinned) { free_all(h); return HX_E_NOMEM; }
@@ -328,12 +307,12 @@ int hx_copy(const hx_matrix *src, hx_matrix **out) {
     if (rc) return rc;
     hx_matrix *h = *out;
     HX_CUDA(cudaStreamSynchronize(src->stream));
-    HX_CUDA(cudaMemcpyAsync(h->band, src->band, sizeof(float) * (size_t)src->band_elems,
+    HX_CUDA(cudaMemcpyAsync(h->band.p, src->band.p, sizeof(float) * (size_t)src->band_elems,
                             cudaMemcpyDeviceToDevice, h->stream));
-    HX_CUDA(cudaMemcpyAsync(h->d_totals, src->d_totals, 8 * sizeof(unsigned long long),
+    HX_CUDA(cudaMemcpyAsync(h->d_totals.p, src->d_totals.p, 8 * sizeof(unsigned long long),
                             cudaMemcpyDeviceToDevice, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
-    h->ingest_kernel = src->ingest_kernel;
+    h->use.ingest_kernel = src->use.ingest_kernel;
     return HX_OK;
 }
 
@@ -375,20 +354,20 @@ int hx_ensure_counts_buffer(hx_matrix *h) {
     h->cnt_elems = h->band_elems;
     HX_CUDA(cudaMallocAsync((void **)&h->cnt, sizeof(uint32_t) * (size_t)h->cnt_elems, h->stream));
     HX_CUDA(hx_fill_async(h->cnt, 0, sizeof(uint32_t) * (size_t)h->cnt_elems, h->stream));
-    h->cnt_fresh = true;
+    h->use.cnt_fresh = true;
     return HX_OK;
 }
 extern "C" {
 
 int hx_set_ingest_kernel(hx_matrix *h, int which) {
     HX_CHECK_ARG(h && which >= 0 && which <= 7);
-    h->ingest_kernel = which;
+    h->use.ingest_kernel = which;
     return HX_OK;
 }
 
 int hx_set_ingest_sms(hx_matrix *h, int n_sms) {
     HX_CHECK_ARG(h && n_sms >= 0);
-    h->ingest_sms = n_sms;
+    h->use.ingest_sms = n_sms;
     return HX_OK;
 }
 
@@ -408,13 +387,13 @@ int hx_ingest_totals(hx_matrix *h, int64_t totals[4]) {
     HX_CUDA(cudaSetDevice(h->device));
     unsigned long long *hp = (unsigned long long *)h->h_pinned;
     int *he = (int *)(hp + 8);
-    HX_CUDA(cudaMemcpyAsync(hp, h->d_totals, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
-    HX_CUDA(cudaMemcpyAsync(he, h->d_err, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    if (h->prepass_ran) HX_CUDA(cudaMemcpyAsync(he + 1, h->d_flags + 4, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(hp, h->d_totals.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(he, h->d_err.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (h->use.prepass_ran) HX_CUDA(cudaMemcpyAsync(he + 1, h->d_flags.p + 4, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
-    if (h->prepass_ran && he[1] == 0) hx_note_unsorted();
+    if (h->use.prepass_ran && he[1] == 0) hx_note_unsorted();
     hx_wire_trace_dump();
-    if (h->ev_rec) cudaEventElapsedTime(&h->last_ms[0], h->ev0, h->ev1);
+    if (h->use.ev_rec) cudaEventElapsedTime(&h->use.last_ms[0], h->ev0, h->ev1);
     for (int i = 0; i < 4; ++i) totals[i] = (int64_t)hp[i];
     if (*he) {
         hx_set_error("ingest: invalid packed read(s): %s%s",
@@ -451,20 +430,9 @@ int hx_ingest_host(hx_matrix *h, const int32_t *rank, const int64_t *off, const 
         HX_CHECK_ARG(rank && off && codes);
         const int64_t n_codes = off[n_reads] - off[0];
         HX_CHECK_ARG(n_codes >= 0);
-        if (n_reads > h->cap_reads) {
-            if (h->s_rank) cudaFreeAsync(h->s_rank, h->stream);
-            if (h->s_off) cudaFreeAsync(h->s_off, h->stream);
-            h->s_rank = nullptr; h->s_off = nullptr; h->cap_reads = 0;
-            HX_CUDA(cudaMallocAsync((void **)&h->s_rank, sizeof(int32_t) * (size_t)n_reads, h->stream));
-            HX_CUDA(cudaMallocAsync((void **)&h->s_off, sizeof(int64_t) * ((size_t)n_reads + 1) + 16, h->stream));
-            h->cap_reads = n_reads;
-        }
-        if (n_codes > h->cap_codes) {
-            if (h->s_codes) cudaFreeAsync(h->s_codes, h->stream);
-            h->s_codes = nullptr; h->cap_codes = 0;
-            HX_CUDA(cudaMallocAsync((void **)&h->s_codes, (size_t)n_codes + 16, h->stream));
-            h->cap_codes = n_codes;
-        }
+        HX_CUDA(h->s_rank.grow(sizeof(int32_t) * n_reads, h->stream));
+        HX_CUDA(h->s_off.grow(sizeof(int64_t) * (n_reads + 1) + 16, h->stream));
+        HX_CUDA(h->s_codes.grow(n_codes + 16, h->stream));
         int rc = hx_ensure_counts_buffer(h);
         if (rc) return rc;
         const int n_chunks = n_reads >= 200000 && !(pipe_env && !strcmp(pipe_env, "off")) ? 4 : 1;
@@ -484,15 +452,15 @@ int hx_ingest_host(hx_matrix *h, const int32_t *rank, const int64_t *off, const 
                 b = std::lower_bound(off + a, off + n_reads, target) - off;
                 if (b <= a) continue;
             }
-            HX_CUDA(cudaMemcpyAsync(h->s_rank + a, rank + a, sizeof(int32_t) * (size_t)(b - a), cudaMemcpyHostToDevice, cs));
-            HX_CUDA(cudaMemcpyAsync(h->s_off + a, off + a, sizeof(int64_t) * (size_t)(b - a + 1), cudaMemcpyHostToDevice, cs));
-            HX_CUDA(cudaMemcpyAsync(h->s_codes + (off[a] - off[0]), codes + off[a], (size_t)(off[b] - off[a]), cudaMemcpyHostToDevice, cs));
+            HX_CUDA(cudaMemcpyAsync(h->s_rank.p + a, rank + a, sizeof(int32_t) * (size_t)(b - a), cudaMemcpyHostToDevice, cs));
+            HX_CUDA(cudaMemcpyAsync(h->s_off.p + a, off + a, sizeof(int64_t) * (size_t)(b - a + 1), cudaMemcpyHostToDevice, cs));
+            HX_CUDA(cudaMemcpyAsync(h->s_codes.p + (off[a] - off[0]), codes + off[a], (size_t)(off[b] - off[a]), cudaMemcpyHostToDevice, cs));
             if (n_chunks > 1) {
                 HX_CUDA(cudaEventRecord(h->host_ev, cs));
                 HX_CUDA(cudaStreamWaitEvent(h->stream, h->host_ev, 0));
             }
             // kernels index codes by absolute offsets: bias the base pointer by off[0]
-            rc = hx_launch_ingest(h, h->s_rank + a, h->s_off + a, h->s_codes - off[0], b - a);
+            rc = hx_launch_ingest(h, h->s_rank.p + a, h->s_off.p + a, h->s_codes.p - off[0], b - a);
             if (rc) return rc;
             a = b;
         }
@@ -508,57 +476,31 @@ int hx_ingest_host_compact(hx_matrix *h, const int32_t *rank, const uint16_t *kl
         HX_CHECK_ARG(rank && klen && (codes4 || n_codes == 0));
         cudaStream_t st = h->stream;
         const int64_t n_words = (n_codes + 7) / 8;          // 32-bit words of packed nibbles
-        if (n_reads > h->cap_reads) {
-            if (h->s_rank) cudaFreeAsync(h->s_rank, st);
-            if (h->s_off) cudaFreeAsync(h->s_off, st);
-            h->s_rank = nullptr; h->s_off = nullptr; h->cap_reads = 0;
-            HX_CUDA(cudaMallocAsync((void **)&h->s_rank, sizeof(int32_t) * (size_t)n_reads, st));
-            HX_CUDA(cudaMallocAsync((void **)&h->s_off, sizeof(int64_t) * ((size_t)n_reads + 1), st));
-            h->cap_reads = n_reads;
-        }
-        if (n_words * 8 > h->cap_codes) {
-            if (h->s_codes) cudaFreeAsync(h->s_codes, st);
-            h->s_codes = nullptr; h->cap_codes = 0;
-            HX_CUDA(cudaMallocAsync((void **)&h->s_codes, (size_t)n_words * 8 + 16, st));
-            h->cap_codes = n_words * 8;
-        }
-        if (n_reads > h->cap_klen) {
-            if (h->s_klen) cudaFreeAsync(h->s_klen, st);
-            h->s_klen = nullptr; h->cap_klen = 0;
-            HX_CUDA(cudaMallocAsync((void **)&h->s_klen, sizeof(uint16_t) * (size_t)n_reads, st));
-            h->cap_klen = n_reads;
-        }
-        if (n_words > h->cap_codes4) {
-            if (h->s_codes4) cudaFreeAsync(h->s_codes4, st);
-            h->s_codes4 = nullptr; h->cap_codes4 = 0;
-            HX_CUDA(cudaMallocAsync((void **)&h->s_codes4, sizeof(uint32_t) * (size_t)n_words, st));
-            h->cap_codes4 = n_words;
-        }
         constexpr int ITEMS = 16;
         const int64_t n1 = n_reads + 1;
         const int64_t nblk = (n1 + 256 * ITEMS - 1) / (256 * ITEMS);
-        if (nblk > h->cap_scan) {
-            if (h->s_scan) cudaFreeAsync(h->s_scan, st);
-            h->s_scan = nullptr; h->cap_scan = 0;
-            HX_CUDA(cudaMallocAsync((void **)&h->s_scan, sizeof(int64_t) * (size_t)nblk, st));
-            h->cap_scan = nblk;
-        }
-        HX_CUDA(cudaMemcpyAsync(h->s_rank, rank, sizeof(int32_t) * (size_t)n_reads, cudaMemcpyHostToDevice, st));
-        HX_CUDA(cudaMemcpyAsync(h->s_klen, klen, sizeof(uint16_t) * (size_t)n_reads, cudaMemcpyHostToDevice, st));
+        HX_CUDA(h->s_rank.grow(sizeof(int32_t) * n_reads, st));
+        HX_CUDA(h->s_off.grow(sizeof(int64_t) * n1 + 16, st));
+        HX_CUDA(h->s_codes.grow(n_words * 8 + 16, st));
+        HX_CUDA(h->s_klen.grow(sizeof(uint16_t) * n_reads, st));
+        HX_CUDA(h->s_codes4.grow(sizeof(uint32_t) * n_words, st));
+        HX_CUDA(h->s_scan.grow(sizeof(int64_t) * nblk, st));
+        HX_CUDA(cudaMemcpyAsync(h->s_rank.p, rank, sizeof(int32_t) * (size_t)n_reads, cudaMemcpyHostToDevice, st));
+        HX_CUDA(cudaMemcpyAsync(h->s_klen.p, klen, sizeof(uint16_t) * (size_t)n_reads, cudaMemcpyHostToDevice, st));
         if (n_codes)
-            HX_CUDA(cudaMemcpyAsync(h->s_codes4, codes4, (size_t)((n_codes + 1) / 2), cudaMemcpyHostToDevice, st));
+            HX_CUDA(cudaMemcpyAsync(h->s_codes4.p, codes4, (size_t)((n_codes + 1) / 2), cudaMemcpyHostToDevice, st));
         // off = exclusive scan of klen (n+1 entries, off[n] = n_codes); codes = one byte per nibble
-        k_widen_klen<<<(unsigned)((n1 + 255) / 256), 256, 0, st>>>(h->s_klen, n_reads, h->s_off);
-        k_scan_partials<int64_t, 0, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(h->s_off, n1, h->s_scan);
-        k_scan_spine<int64_t, 0><<<1, 32, 0, st>>>(h->s_scan, nblk, nullptr);
-        k_scan_apply<int64_t, 0, ITEMS, true><<<(unsigned)nblk, 256, 0, st>>>(h->s_off, n1, h->s_scan, h->s_off);
+        k_widen_klen<<<(unsigned)((n1 + 255) / 256), 256, 0, st>>>(h->s_klen.p, n_reads, h->s_off.p);
+        k_scan_partials<int64_t, 0, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(h->s_off.p, n1, h->s_scan.p);
+        k_scan_spine<int64_t, 0><<<1, 32, 0, st>>>(h->s_scan.p, nblk, nullptr);
+        k_scan_apply<int64_t, 0, ITEMS, true><<<(unsigned)nblk, 256, 0, st>>>(h->s_off.p, n1, h->s_scan.p, h->s_off.p);
         if (n_words)
-            k_unpack_nibbles<<<(unsigned)((n_words + 255) / 256), 256, 0, st>>>(h->s_codes4, n_words, (uint2 *)h->s_codes);
-        h->launches += 5;
+            k_unpack_nibbles<<<(unsigned)((n_words + 255) / 256), 256, 0, st>>>(h->s_codes4.p, n_words, (uint2 *)h->s_codes.p);
+        h->use.launches += 5;
         HX_CUDA(cudaGetLastError());
         int rc = hx_ensure_counts_buffer(h);
         if (rc) return rc;
-        rc = hx_launch_ingest(h, h->s_rank, h->s_off, h->s_codes, n_reads);
+        rc = hx_launch_ingest(h, h->s_rank.p, h->s_off.p, h->s_codes.p, n_reads);
         if (rc) return rc;
     }
     return hx_ingest_totals(h, totals);
@@ -570,9 +512,9 @@ int hx_counts_buffer(hx_matrix *h, void **d_counts, int64_t *n_u32, void **d_tot
     int rc = hx_ensure_counts_buffer(h);
     if (rc) return rc;
     *d_counts = h->cnt;
-    h->cnt_fresh = false;                 // the caller may write through the pointer (until the next hx_reset_counts)
+    h->use.cnt_fresh = false;             // the caller may write through the pointer (until the next hx_reset_counts)
     *n_u32 = h->cnt_elems;
-    *d_totals = h->d_totals;
+    *d_totals = h->d_totals.p;
     *n_i64 = 4;
     return HX_OK;
 }
@@ -585,61 +527,56 @@ int hx_counts_pack(hx_matrix *h, int32_t world, void **d_packed, int64_t *n_u32)
     const int64_t n_pairs = h->band_elems / HX_CELL;
     const int64_t flag_at = (n_pairs * HX_PACK_WORDS + 3) & ~(int64_t)3;      // 16-byte aligned trailer
     const int64_t words = flag_at + 4;
-    if (words > h->cap_pack) {
-        if (h->d_pack) cudaFreeAsync(h->d_pack, h->stream);
-        h->d_pack = nullptr; h->cap_pack = 0;
-        HX_CUDA(cudaMallocAsync((void **)&h->d_pack, sizeof(uint32_t) * (size_t)words, h->stream));
-        h->cap_pack = words;
-    }
-    HX_CUDA(hx_fill_async(h->d_pack + n_pairs * HX_PACK_WORDS, 0, (size_t)(words - n_pairs * HX_PACK_WORDS) * 4, h->stream));
+    HX_CUDA(h->d_pack.grow(sizeof(uint32_t) * words, h->stream));
+    HX_CUDA(hx_fill_async(h->d_pack.p + n_pairs * HX_PACK_WORDS, 0, (size_t)(words - n_pairs * HX_PACK_WORDS) * 4, h->stream));
     const int64_t n_w = n_pairs * HX_PACK_WORDS;
     k_pack_counts<<<(unsigned)((n_w + 255) / 256), 256, 0, h->stream>>>(h->cnt, n_pairs, 65535u / (uint32_t)world,
-                                                                        h->d_pack, flag_at);
-    h->launches++;
+                                                                        h->d_pack.p, flag_at);
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
-    *d_packed = h->d_pack;
+    *d_packed = h->d_pack.p;
     *n_u32 = words;
     return HX_OK;
 }
 
 int hx_counts_unpack(hx_matrix *h, int32_t *overflowed) {
-    HX_CHECK_ARG(h && overflowed && h->d_pack && h->cnt);
+    HX_CHECK_ARG(h && overflowed && h->d_pack.p && h->cnt);
     HX_CUDA(cudaSetDevice(h->device));
     const int64_t n_pairs = h->band_elems / HX_CELL;
     const int64_t flag_at = (n_pairs * HX_PACK_WORDS + 3) & ~(int64_t)3;
     const int64_t n_w = n_pairs * HX_PACK_WORDS;
-    h->cnt_fresh = false;
-    k_unpack_counts<<<(unsigned)((n_w + 255) / 256), 256, 0, h->stream>>>(h->d_pack, n_pairs, h->cnt, flag_at);
-    h->launches++;
+    h->use.cnt_fresh = false;
+    k_unpack_counts<<<(unsigned)((n_w + 255) / 256), 256, 0, h->stream>>>(h->d_pack.p, n_pairs, h->cnt, flag_at);
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     uint32_t *hp = (uint32_t *)h->h_pinned + 40;
-    HX_CUDA(cudaMemcpyAsync(hp, h->d_pack + flag_at, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(hp, h->d_pack.p + flag_at, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     *overflowed = *hp != 0;
     return HX_OK;
 }
 
 int hx_counts_unpack_async(hx_matrix *h, void *stream) {
-    HX_CHECK_ARG(h && h->d_pack && h->cnt);
+    HX_CHECK_ARG(h && h->d_pack.p && h->cnt);
     HX_CUDA(cudaSetDevice(h->device));
     const int64_t n_pairs = h->band_elems / HX_CELL;
     const int64_t flag_at = (n_pairs * HX_PACK_WORDS + 3) & ~(int64_t)3;
     const int64_t n_w = n_pairs * HX_PACK_WORDS;
-    h->cnt_fresh = false;
+    h->use.cnt_fresh = false;
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-    k_unpack_counts<<<(unsigned)((n_w + 255) / 256), 256, 0, st>>>(h->d_pack, n_pairs, h->cnt, flag_at);
-    h->launches++;
+    k_unpack_counts<<<(unsigned)((n_w + 255) / 256), 256, 0, st>>>(h->d_pack.p, n_pairs, h->cnt, flag_at);
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }
 
 int hx_counts_pack_overflowed(hx_matrix *h, int32_t *overflowed) {
-    HX_CHECK_ARG(h && overflowed && h->d_pack);
+    HX_CHECK_ARG(h && overflowed && h->d_pack.p);
     HX_CUDA(cudaSetDevice(h->device));
     const int64_t n_pairs = h->band_elems / HX_CELL;
     const int64_t flag_at = (n_pairs * HX_PACK_WORDS + 3) & ~(int64_t)3;
     uint32_t *hp = (uint32_t *)h->h_pinned + 40;
-    HX_CUDA(cudaMemcpyAsync(hp, h->d_pack + flag_at, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(hp, h->d_pack.p + flag_at, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     *overflowed = *hp != 0;
     return HX_OK;
@@ -657,10 +594,10 @@ int hx_counts_max(hx_matrix *h, uint32_t *max_count) {
     HX_CUDA(cudaSetDevice(h->device));
     int rc = hx_ensure_counts_buffer(h);
     if (rc) return rc;
-    uint32_t *d_out = reinterpret_cast<uint32_t *>(h->d_flags + 6);
+    uint32_t *d_out = reinterpret_cast<uint32_t *>(h->d_flags.p + 6);
     HX_CUDA(hx_fill_async(d_out, 0, sizeof(uint32_t), h->stream));
     k_counts_max<<<592, 256, 0, h->stream>>>(h->cnt, h->cnt_elems, d_out);
-    h->launches++;
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     uint32_t *hp = (uint32_t *)h->h_pinned + 41;
     HX_CUDA(cudaMemcpyAsync(hp, d_out, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
@@ -678,7 +615,7 @@ int hx_counts_ipc_export(hx_matrix *h, int32_t world, void *handle_out) {
     h->cnt_elems = rows_per * world * h->W * HX_CELL;          // padded so that every rank owns rows_per rows
     HX_CUDA(cudaMalloc((void **)&h->cnt, sizeof(uint32_t) * (size_t)h->cnt_elems));   // IPC needs a plain allocation
     h->cnt_ipc = true;
-    h->cnt_fresh = false;
+    h->use.cnt_fresh = false;
     HX_CUDA(hx_fill_async(h->cnt, 0, sizeof(uint32_t) * (size_t)h->cnt_elems, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     cudaIpcMemHandle_t hd;
@@ -729,12 +666,12 @@ int hx_reset_counts(hx_matrix *h) {
         const size_t want = (n16 + 255) / 256;
         const unsigned grid = (unsigned)(want < 1 ? 1 : (want > 148 * 16 ? 148 * 16 : want));
         k_reset_counts<<<grid, 256, 0, h->stream>>>(reinterpret_cast<uint4 *>(h->cnt), sizeof(uint32_t) * (size_t)h->cnt_elems,
-                                                    h->d_totals, h->d_err);
+                                                    h->d_totals.p, h->d_err.p);
         HX_CUDA(cudaGetLastError());
-        h->cnt_fresh = true;
+        h->use.cnt_fresh = true;
     } else {
-        HX_CUDA(hx_fill_async(h->d_totals, 0, 8 * sizeof(unsigned long long), h->stream));
-        HX_CUDA(hx_fill_async(h->d_err, 0, sizeof(int), h->stream));
+        HX_CUDA(hx_fill_async(h->d_totals.p, 0, 8 * sizeof(unsigned long long), h->stream));
+        HX_CUDA(hx_fill_async(h->d_err.p, 0, sizeof(int), h->stream));
     }
     return HX_OK;
 }
@@ -744,12 +681,12 @@ int hx_finalize_counts(hx_matrix *h) {
     if (!h->cnt) return HX_OK;
     HX_CUDA(cudaSetDevice(h->device));
     const int64_t n = h->band_elems;
-    k_fold_counts<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->cnt, h->band, n);
-    h->launches++;
+    k_fold_counts<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->cnt, h->band.p, n);
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     if (h->cnt_ipc) HX_CUDA(cudaStreamSynchronize(h->stream));   // a shared allocation is freed with cudaFree
     release_counts(h);                                           // (stream-ordered otherwise: no host wait here)
-    h->counts_dirty = true;
+    h->use.counts_dirty = true;
     return HX_OK;
 }
 
@@ -759,9 +696,9 @@ int hx_add_observation(hx_matrix *h, int a, int b, int32_t i, int32_t j, float a
     int rc = in_band(h, a, b, i, j);
     if (rc) { hx_set_error("add_observation(%d,%d,%d,%d): outside band/arguments", a, b, i, j); return rc; }
     HX_CUDA(cudaSetDevice(h->device));
-    k_add_one<<<1, 1, 0, h->stream>>>(h->band + hx_cell_off(h->W, i, j) + a * HX_NSYM + b, amount);
-    h->launches++;
-    h->counts_dirty = true;
+    k_add_one<<<1, 1, 0, h->stream>>>(h->band.p + hx_cell_off(h->W, i, j) + a * HX_NSYM + b, amount);
+    h->use.launches++;
+    h->use.counts_dirty = true;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }
@@ -774,7 +711,7 @@ int hx_get_observation(hx_matrix *h, int a, int b, int32_t i, int32_t j, float *
     HX_CUDA(cudaSetDevice(h->device));
     const int64_t o = hx_cell_off(h->W, i, j) + a * HX_NSYM + b;
     float v = 0.0f;
-    HX_CUDA(cudaMemcpyAsync(&v, h->band + o, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(&v, h->band.p + o, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     if (h->cnt) {       // counts not folded yet: report the sum
         uint32_t c = 0;
@@ -794,11 +731,11 @@ int hx_reweight_observation(hx_matrix *h, int a, int b, int32_t i, int32_t j, do
     if (rc) { hx_set_error("reweight_observation(%d,%d,%d,%d): bad arguments", a, b, i, j); return rc; }
     if (h->cnt) { hx_set_error("reweight_observation: call hx_finalize_counts first"); return HX_E_STATE; }
     HX_CUDA(cudaSetDevice(h->device));
-    k_reweight_one<<<1, 1, 0, h->stream>>>(h->band + hx_cell_off(h->W, i, j) + a * HX_NSYM + b, ratio, h->d_misc + 16);
-    h->launches++;
-    h->counts_dirty = true;
+    k_reweight_one<<<1, 1, 0, h->stream>>>(h->band.p + hx_cell_off(h->W, i, j) + a * HX_NSYM + b, ratio, h->d_misc.p + 16);
+    h->use.launches++;
+    h->use.counts_dirty = true;
     HX_CUDA(cudaGetLastError());
-    HX_CUDA(cudaMemcpyAsync(removed, h->d_misc + 16, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(removed, h->d_misc.p + 16, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     return HX_OK;
 }
@@ -808,7 +745,7 @@ int hx_band_to_host(hx_matrix *h, float *out) {
     HX_CHECK_ARG(h && out);
     if (h->cnt) { hx_set_error("band_to_host: call hx_finalize_counts first"); return HX_E_STATE; }
     HX_CUDA(cudaSetDevice(h->device));
-    HX_CUDA(cudaMemcpyAsync(out, h->band, sizeof(float) * (size_t)h->band_elems, cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(out, h->band.p, sizeof(float) * (size_t)h->band_elems, cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     return HX_OK;
 }
@@ -817,9 +754,9 @@ int hx_band_from_host(hx_matrix *h, const float *in) {
     HX_CHECK_ARG(h && in);
     if (h->cnt) { hx_set_error("band_from_host: call hx_finalize_counts first"); return HX_E_STATE; }
     HX_CUDA(cudaSetDevice(h->device));
-    HX_CUDA(cudaMemcpyAsync(h->band, in, sizeof(float) * (size_t)h->band_elems, cudaMemcpyHostToDevice, h->stream));
+    HX_CUDA(cudaMemcpyAsync(h->band.p, in, sizeof(float) * (size_t)h->band_elems, cudaMemcpyHostToDevice, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
-    h->counts_dirty = true;
+    h->use.counts_dirty = true;
     return HX_OK;
 }
 
@@ -842,13 +779,13 @@ int hx_to_dense(hx_matrix *h, float *out) {
 
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms) {
     HX_CHECK_ARG(h && ms && which >= 0 && which < 3);
-    *ms = h->last_ms[which];
+    *ms = h->use.last_ms[which];
     return HX_OK;
 }
 
 int hx_launch_count(const hx_matrix *h, int64_t *n) {
     HX_CHECK_ARG(h && n);
-    *n = h->launches;
+    *n = h->use.launches;
     return HX_OK;
 }
 

@@ -31,11 +31,34 @@ struct HxCnt {
 #endif
 };
 
+// A stream-ordered device buffer of T that grows on demand; all zero is empty (hx_matrix is calloc'ed).  cap is the
+// size of the allocation in bytes.  grow() allocates exactly the bytes asked for: a caller that wants headroom adds it.
+template <class T>
+struct HxDevBuf {
+    T *p;
+    int64_t cap;
+    // bytes > cap: free the old block (its contents are not kept) and allocate `bytes` on st; *grew is set if so
+    cudaError_t grow(int64_t bytes, cudaStream_t st, bool *grew = nullptr) {
+        if (bytes <= cap) return cudaSuccess;
+        if (grew) *grew = true;
+        release(st);
+        const cudaError_t e = cudaMallocAsync((void **)&p, (size_t)bytes, st);
+        if (e != cudaSuccess) { p = nullptr; return e; }
+        cap = bytes;
+        return cudaSuccess;
+    }
+    void release(cudaStream_t st) {
+        if (p) cudaFreeAsync(p, st);
+        p = nullptr;
+        cap = 0;
+    }
+};
+
 #define HX_WIRE_SETS 3
 // One staging set of the dense wire format (wire.cu): raw shipped bytes + the rebuilt packed arrays
 struct hx_wire_set {
-    void *raw; int32_t *rank; int64_t *off; uint8_t *codes; int64_t *partials, *run_end;
-    int64_t cap_raw, cap_rank, cap_off, cap_codes, cap_partials, cap_run_end;
+    HxDevBuf<uint8_t> raw; HxDevBuf<int32_t> rank; HxDevBuf<int64_t> off; HxDevBuf<uint8_t> codes;
+    HxDevBuf<int64_t> partials, run_end;
     cudaEvent_t copied, decoded, consumed;
 };
 
@@ -44,62 +67,57 @@ struct hx_matrix {
     int64_t band_elems;              // (N+2)*W*49
     cudaStream_t stream;
     bool own_stream;
-    float *band;                     // float32 working matrix (what the Hansel surface reads)
+    HxDevBuf<float> band;            // float32 working matrix (what the Hansel surface reads)
     uint32_t *cnt;                   // integer counts being ingested (lazily allocated)
-    bool cnt_fresh;                  // cnt is still all zero (nothing ingested / received since it was cleared)
     bool cnt_ipc;                    // cnt is a plain cudaMalloc allocation shared through CUDA IPC
     int64_t cnt_elems;               // allocated uint32 elements (>= band_elems; padded for the fused exchange)
     uint32_t *peer_host[HX_MAX_PEERS];   // fused exchange: every rank's cnt (own entry = local pointer)
     uint32_t **d_peer_tbl;           // the same table on the device
     int peer_world, peer_rows_per;
     void *ipc_opened[HX_MAX_PEERS];  // pointers returned by cudaIpcOpenMemHandle (to close)
-    unsigned long long *d_totals;    // [8] slices, crumbs, covered, sentinels, -, -, -, -
-    int *d_err;                      // ingestion error bits
+    HxDevBuf<unsigned long long> d_totals;   // [8] slices, crumbs, covered, sentinels, -, -, -, -
+    HxDevBuf<int> d_err;             // ingestion error bits
     // staging for hx_ingest_host
-    int32_t *s_rank; int64_t *s_off; uint8_t *s_codes;
-    int64_t cap_reads, cap_codes;
-    uint16_t *s_klen; uint32_t *s_codes4; int64_t *s_scan;     // compact wire format staging
-    int64_t cap_klen, cap_codes4, cap_scan;
-    hx_wire_set wire[HX_WIRE_SETS]; int wire_next;   // dense wire format: rotating staging sets
+    HxDevBuf<int32_t> s_rank; HxDevBuf<int64_t> s_off; HxDevBuf<uint8_t> s_codes;
+    HxDevBuf<uint16_t> s_klen; HxDevBuf<uint32_t> s_codes4; HxDevBuf<int64_t> s_scan;   // compact wire format staging
+    hx_wire_set wire[HX_WIRE_SETS];  // dense wire format: rotating staging sets
     cudaStream_t copy_stream, decode_stream; // host->device copies / decode kernels of the dense format
     uint8_t *pin[2]; int64_t pin_cap[2]; cudaEvent_t pin_ev[2]; bool pin_busy[2];   // pinned encode buffers of hx_ingest_host
     // recovery scratch
-    double *scnt;                    // (N+2)*8 per-site counts + total
-    int32_t *vseen;                  // (N+2) valid symbols seen per site
-    bool counts_dirty;
-    uint8_t *d_path;                 // path buffer(s)
-    int64_t cap_path;
-    double *d_stats;                 // per-iteration stats
-    int64_t cap_stats;
-    double *d_site;                  // 2 x 3*(N+2) per-site log10 marginal (cur), (orig), marginal (alternating haplotypes)
+    HxDevBuf<double> scnt;           // (N+2)*8 per-site counts + total
+    HxDevBuf<int32_t> vseen;         // (N+2) valid symbols seen per site
+    HxDevBuf<uint8_t> d_path;        // path buffer(s)
+    HxDevBuf<double> d_stats;        // per-iteration stats
+    HxDevBuf<double> d_site;         // 2 x 3*(N+2) per-site log10 marginal (cur), (orig), marginal (alternating haplotypes)
     cudaStream_t sum_stream;         // the ordered log10 sums of a haplotype run here, off the critical path
     cudaEvent_t sum_done[2], site_ready;
-    bool sum_busy[2];
-    double *d_terms;                 // walk tables: (N+2)*Lw*49 log10 lookback terms + (N+2)*8 log10 marginals
-    int64_t cap_terms;
-    uint8_t *d_spec;                 // speculative block paths, majority-allele guess and block flags of the walk
-    int64_t cap_spec;
-    double *d_partials;              // block partials of the reweight reduction
-    int64_t cap_partials;
-    int *d_flags;                    // [0] hole site / abort flag, [1..] misc
-    int64_t *d_run_end;              // (N+1) end (exclusive) of the run of reads with each rank
-    int64_t *d_run_list;             // compact run list for the tensor-core kernel: ranks (int32), stops (int64), count
-    void *d_jobs;                    // per-CTA job tables of the tensor-core kernel (ingest_umma.cu)
-    int64_t cap_jobs;
-    double *d_misc;                  // small outputs (weights etc.)
-    uint32_t *d_pack;                // packed counts for the cross-GPU exchange (api.cu)
-    int64_t cap_pack;
+    HxDevBuf<double> d_terms;        // walk tables: (N+2)*Lw*49 log10 lookback terms + (N+2)*8 log10 marginals
+    HxDevBuf<uint8_t> d_spec;        // speculative block paths, majority-allele guess and block flags of the walk
+    HxDevBuf<double> d_partials;     // block partials of the reweight reduction
+    HxDevBuf<int> d_flags;           // [0] hole site / abort flag, [1..] misc
+    HxDevBuf<int64_t> d_run_end;     // (N+1) end (exclusive) of the run of reads with each rank
+    HxDevBuf<int64_t> d_run_list;    // compact run list for the tensor-core kernel: ranks (int32), stops (int64), count
+    HxDevBuf<int4> d_jobs;           // per-CTA job tables of the tensor-core kernel (ingest_umma.cu)
+    HxDevBuf<double> d_misc;         // small outputs (weights etc.)
+    HxDevBuf<uint32_t> d_pack;       // packed counts for the cross-GPU exchange (api.cu)
     void *h_pinned;                  // small host buffer for D2H of scalars
-    int ingest_kernel;
-    int ingest_sms;                  // SMs the persistent ingestion kernels may use (0 = all)
     void *lr_scratch;                // long-read ingestion scratch (ingest_long.cu)
     void *l2_scratch;                // long-read tensor-core ingestion scratch (ingest_lumma.cu)
     cudaEvent_t ev0, ev1;
     cudaEvent_t host_ev;             // orders the chunked host->device copies of hx_ingest_host
-    bool ev_rec;                     // ev0/ev1 have been recorded at least once
-    bool prepass_ran;                // d_flags[4] holds the sortedness verdict of the last ingestion launch
-    float last_ms[3];
-    int64_t launches;
+    // State of one use of the handle.  A new matrix and a parked one taken back by hx_create both start from `use = {}`.
+    struct Use {
+        int64_t launches = 0;
+        int ingest_kernel = 0;
+        int ingest_sms = 0;          // SMs the persistent ingestion kernels may use (0 = all)
+        bool counts_dirty = true;    // scnt / vseen do not reflect the band yet
+        bool cnt_fresh = false;      // cnt is still all zero (nothing ingested / received since it was cleared)
+        bool ev_rec = false;         // ev0/ev1 have been recorded at least once
+        bool prepass_ran = false;    // d_flags[4] holds the sortedness verdict of the last ingestion launch
+        int wire_next = 0;           // the next staging set of the dense wire format
+        bool sum_busy[2] = {};       // sum_done[b] marks ordered sums not yet joined into the main stream
+        float last_ms[3] = {};
+    } use;
 };
 
 void hx_set_error(const char *fmt, ...);

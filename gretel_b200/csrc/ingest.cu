@@ -770,11 +770,11 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
                          int64_t n_reads, int64_t *run_end, const int *ok) {
     if (n_reads <= 0) return HX_OK;
     const bool presorted = run_end != nullptr;
-    if (!presorted) run_end = h->d_run_end;
+    if (!presorted) run_end = h->d_run_end.p;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    if (h->ingest_sms > 0 && h->ingest_sms < sms) sms = h->ingest_sms;
-    const int *sorted_flag = presorted ? ok : h->d_flags + 4;
+    if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
+    const int *sorted_flag = presorted ? ok : h->d_flags.p + 4;
     constexpr int GBLOCK = 256;
     const int64_t gwant = (n_reads + (GBLOCK / 32) - 1) / (GBLOCK / 32);
     const int ggrid = (int)(gwant < (int64_t)sms * 8 ? gwant : (int64_t)sms * 8);
@@ -782,55 +782,55 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
     // crumbs in a read are all distinct cells, so W+1 bounds the SNPs per read
     const int kmax = h->W + 1;
     const bool bs_possible = kmax >= 2 && kmax <= BS_KMAX;
-    const bool use_bs = (h->ingest_kernel == 2 || h->ingest_kernel == 4 || h->ingest_kernel == 5 || h->ingest_kernel == 6)
-                            ? bs_possible : (h->ingest_kernel == 0 && bs_possible);
+    const bool use_bs = (h->use.ingest_kernel == 2 || h->use.ingest_kernel == 4 || h->use.ingest_kernel == 5 || h->use.ingest_kernel == 6)
+                            ? bs_possible : (h->use.ingest_kernel == 0 && bs_possible);
     // tensor-core kernel (ingest_umma.cu): default for rank-sorted reads of at most 32 SNPs
     // (auto: when a rank's run of reads is deep enough to fill MMAs - measured: 1000 reads per rank 0.42 vs 0.63 ms,
     // 20 reads per rank 0.25 vs 0.19 ms against the bit-sliced kernel)
     const bool use_umma = use_bs && hx_umma_possible(h) &&
-                          (h->ingest_kernel == 6 || (h->ingest_kernel == 0 && n_reads >= 64 * ((int64_t)h->N + 1)));
+                          (h->use.ingest_kernel == 6 || (h->use.ingest_kernel == 0 && n_reads >= 64 * ((int64_t)h->N + 1)));
     const bool fused = h->peer_world > 1;
-    const bool use_long = !use_bs && (h->ingest_kernel == 3 || (h->ingest_kernel == 0 && kmax >= 2));
+    const bool use_long = !use_bs && (h->use.ingest_kernel == 3 || (h->use.ingest_kernel == 0 && kmax >= 2));
     // long-read tensor-core kernel (ingest_lumma.cu): default for wide reads unless its one-hot scratch would be huge
-    const bool use_lumma = kmax >= 2 && (h->ingest_kernel == 7 ||
-                                         (h->ingest_kernel == 0 && !use_bs &&
+    const bool use_lumma = kmax >= 2 && (h->use.ingest_kernel == 7 ||
+                                         (h->use.ingest_kernel == 0 && !use_bs &&
                                           hx_lumma_scratch_bytes(h, n_reads) <= ((int64_t)24 << 30)));
 
     // unsorted short reads: once this process has met some, the counting-sort tensor-core kernel is queued as the
     // fallback (it runs only if the pre-pass says "not sorted"); before that, and when its scratch would be huge, one
     // RED per pair (k1_pairs_red)
-    const bool lumma_fallback = !presorted && use_bs && !use_lumma && h->ingest_kernel == 0 && hx_unsorted_seen() &&
+    const bool lumma_fallback = !presorted && use_bs && !use_lumma && h->use.ingest_kernel == 0 && hx_unsorted_seen() &&
                                 hx_lumma_scratch_bytes(h, n_reads) <= ((int64_t)24 << 30);
-    h->prepass_ran = !presorted && !use_lumma && (use_long || use_bs);
+    h->use.prepass_ran = !presorted && !use_lumma && (use_long || use_bs);
     HX_CUDA(cudaEventRecord(h->ev0, h->stream));
     if (use_lumma) {
         int rc = hx_launch_ingest_lumma(h, d_rank, d_off, d_codes, n_reads, presorted ? ok : nullptr);
         if (rc) return rc;
     } else if (use_long) {
         if (!presorted) {
-            HX_CUDA(hx_fill_async(h->d_flags + 4, 1, sizeof(int), h->stream));     // non-zero = sorted
-            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, h->d_flags + 4,
-                                                                                run_end, h->d_err);
-            h->launches++;
+            HX_CUDA(hx_fill_async(h->d_flags.p + 4, 1, sizeof(int), h->stream));     // non-zero = sorted
+            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, h->d_flags.p + 4,
+                                                                                run_end, h->d_err.p);
+            h->use.launches++;
         }
         int rc = hx_launch_ingest_long(h, d_rank, d_off, d_codes, n_reads, sorted_flag);
         if (rc) return rc;
         if (!presorted) {
             k1_pairs_red<GBLOCK><<<ggrid, GBLOCK, 0, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W,
-                                                                  hx_cnt_ref(h), h->d_totals, h->d_err, sorted_flag, 0);
-            h->launches++;
+                                                                  hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag, 0);
+            h->use.launches++;
         }
     } else if (!use_bs) {
         k1_pairs_red<GBLOCK><<<ggrid, GBLOCK, 0, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, hx_cnt_ref(h),
-                                                              h->d_totals, h->d_err, sorted_flag, presorted ? 2 : 1);
-        h->launches++;
+                                                              h->d_totals.p, h->d_err.p, sorted_flag, presorted ? 2 : 1);
+        h->use.launches++;
     } else {
         if (!presorted) {
             // flag: non-zero = sorted; run_end: -1 = no reads of that rank (the tensor-core kernel walks it)
-            k_prepass_init<<<(unsigned)((h->N + 2 + 255) / 256), 256, 0, h->stream>>>(h->d_flags + 4, run_end, use_umma ? h->N + 2 : 0);
-            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, h->d_flags + 4,
-                                                                                run_end, h->d_err);
-            h->launches += 2;
+            k_prepass_init<<<(unsigned)((h->N + 2 + 255) / 256), 256, 0, h->stream>>>(h->d_flags.p + 4, run_end, use_umma ? h->N + 2 : 0);
+            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, h->d_flags.p + 4,
+                                                                                run_end, h->d_err.p);
+            h->use.launches += 2;
         }
         const int npairs = kmax * (kmax - 1) / 2;
         if (use_umma) {
@@ -839,7 +839,7 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
         } else
         // measured (B200): the warp-specialised variant wins for wide reads (config 2: 0.097 vs 0.118 ms),
         // the barrier-phased one for narrow reads (config 3: 0.725 vs 0.751 ms)
-        if (h->ingest_kernel == 5 || (h->ingest_kernel != 4 && kmax > 32)) {
+        if (h->use.ingest_kernel == 5 || (h->use.ingest_kernel != 4 && kmax > 32)) {
             // warp-specialised: pw pair-owning warps + bw builder warps
             const int np = npairs > 512 ? 2 : 1;
             const int pw = ((npairs + np - 1) / np + 31) / 32;
@@ -860,7 +860,7 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
         const int64_t max_useful = (n_reads + 255) / 256;                                                      \
         if (grid > max_useful) grid = max_useful;                                                              \
         kern<<<(unsigned)grid, block, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax,    \
-                                                         gb, pw, hx_cnt_ref(h), h->d_totals, h->d_err, sorted_flag,   \
+                                                         gb, pw, hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag, \
                                                          run_end);                                        \
     } while (0)
             if (np == 2) HX_WS_LAUNCH(14, 2, 1024, 1);
@@ -886,7 +886,7 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
         const int64_t max_useful = (n_reads + 255) / 256;   /* no thinner than 256 reads per CTA */            \
         if (grid > max_useful) grid = max_useful;                                                              \
         kern<<<(unsigned)grid, block, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax,    \
-                                                         gb, hx_cnt_ref(h), h->d_totals, h->d_err, sorted_flag,       \
+                                                         gb, hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag,   \
                                                          run_end);                                        \
     } while (0)
         if (np == 2) HX_BS_LAUNCH(14, 2, 1024, 1);
@@ -894,22 +894,22 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
         else HX_BS_LAUNCH(8, 1, 512, 2);
 #undef HX_BS_LAUNCH
         }
-        h->launches++;
+        h->use.launches++;
         // fallback for unsorted input: runs only when the flag says the bit-sliced kernel declined
         if (lumma_fallback) {
-            k_flag_not<<<1, 32, 0, h->stream>>>(h->d_flags + 4, h->d_flags + 5);
-            h->launches++;
-            int rc = hx_launch_ingest_lumma(h, d_rank, d_off, d_codes, n_reads, h->d_flags + 5);
+            k_flag_not<<<1, 32, 0, h->stream>>>(h->d_flags.p + 4, h->d_flags.p + 5);
+            h->use.launches++;
+            int rc = hx_launch_ingest_lumma(h, d_rank, d_off, d_codes, n_reads, h->d_flags.p + 5);
             if (rc) return rc;
         } else if (!presorted) {
             k1_pairs_red<GBLOCK><<<ggrid, GBLOCK, 0, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W,
-                                                                  hx_cnt_ref(h), h->d_totals, h->d_err, sorted_flag, 0);
-            h->launches++;
+                                                                  hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag, 0);
+            h->use.launches++;
         }
     }
-    h->cnt_fresh = false;
+    h->use.cnt_fresh = false;
     HX_CUDA(cudaGetLastError());
     HX_CUDA(cudaEventRecord(h->ev1, h->stream));
-    h->ev_rec = true;
+    h->use.ev_rec = true;
     return HX_OK;
 }

@@ -348,36 +348,23 @@ k_lr_tiles_staged(const uint4 *__restrict__ planes, const int64_t *__restrict__ 
     if ((threadIdx.x & 31) == 0 && crumbs) atomicAdd(&totals[1], crumbs);
 }
 
-template <typename T>
-int grow(T **p, int64_t *cap, int64_t need, cudaStream_t st) {
-    if (*cap >= need) return HX_OK;
-    if (*p) cudaFreeAsync(*p, st);
-    *p = nullptr;
-    *cap = 0;
-    HX_CUDA(cudaMallocAsync((void **)p, sizeof(T) * (size_t)need, st));
-    *cap = need;
-    return HX_OK;
-}
-
 }  // namespace
 
 // Scratch owned by the matrix for this path (freed in hx_destroy through hx_lr_free).
 struct hx_lr_scratch {
-    int32_t *g_lo = nullptr, *g_hi = nullptr, *g_hipm = nullptr;
-    int64_t *g_len = nullptr, *g_off = nullptr, *first_reach = nullptr, *first_after = nullptr;
-    int64_t *part64 = nullptr; int32_t *part32 = nullptr; int64_t *d_total = nullptr;
-    uint4 *planes = nullptr;
-    int64_t cap_groups = 0, cap_sites = 0, cap_part = 0, cap_planes = 0, cap_lo = 0, cap_hi = 0, cap_hipm = 0,
-            cap_len = 0, cap_off = 0, cap_fr = 0, cap_fa = 0, cap_p32 = 0, cap_tot = 0;
+    HxDevBuf<int32_t> g_lo, g_hi, g_hipm;
+    HxDevBuf<int64_t> g_len, g_off, first_reach, first_after;
+    HxDevBuf<int64_t> part64; HxDevBuf<int32_t> part32; HxDevBuf<int64_t> d_total;
+    HxDevBuf<uint4> planes;
 };
 
 void hx_lr_free(hx_matrix *h) {
     hx_lr_scratch *s = (hx_lr_scratch *)h->lr_scratch;
     if (!s) return;
-    void *ptrs[] = {s->g_lo, s->g_hi, s->g_hipm, s->g_len, s->g_off, s->first_reach, s->first_after,
-                    s->part64, s->part32, s->d_total, s->planes};
-    for (void *p : ptrs)
-        if (p) cudaFreeAsync(p, h->stream);
+    cudaStream_t st = h->stream;
+    s->g_lo.release(st); s->g_hi.release(st); s->g_hipm.release(st); s->g_len.release(st); s->g_off.release(st);
+    s->first_reach.release(st); s->first_after.release(st);
+    s->part64.release(st); s->part32.release(st); s->d_total.release(st); s->planes.release(st);
     delete s;
     h->lr_scratch = nullptr;
 }
@@ -391,56 +378,55 @@ int hx_launch_ingest_long(hx_matrix *h, const int32_t *d_rank, const int64_t *d_
     const int64_t ng = (n_reads + 31) >> 5;
     constexpr int ITEMS = 16;
     const int64_t nblk = (ng + 256 * ITEMS - 1) / (256 * ITEMS);
-    int rc;
-    if ((rc = grow(&s->g_lo, &s->cap_lo, ng, st))) return rc;
-    if ((rc = grow(&s->g_hi, &s->cap_hi, ng, st))) return rc;
-    if ((rc = grow(&s->g_hipm, &s->cap_hipm, ng, st))) return rc;
-    if ((rc = grow(&s->g_len, &s->cap_len, ng, st))) return rc;
-    if ((rc = grow(&s->g_off, &s->cap_off, ng, st))) return rc;
-    if ((rc = grow(&s->first_reach, &s->cap_fr, (int64_t)N + 1, st))) return rc;
-    if ((rc = grow(&s->first_after, &s->cap_fa, (int64_t)N + 1, st))) return rc;
-    if ((rc = grow(&s->part64, &s->cap_part, nblk, st))) return rc;
-    if ((rc = grow(&s->part32, &s->cap_p32, nblk, st))) return rc;
-    if ((rc = grow(&s->d_total, &s->cap_tot, 1, st))) return rc;
+    HX_CUDA(s->g_lo.grow(sizeof(int32_t) * ng, st));
+    HX_CUDA(s->g_hi.grow(sizeof(int32_t) * ng, st));
+    HX_CUDA(s->g_hipm.grow(sizeof(int32_t) * ng, st));
+    HX_CUDA(s->g_len.grow(sizeof(int64_t) * ng, st));
+    HX_CUDA(s->g_off.grow(sizeof(int64_t) * ng, st));
+    HX_CUDA(s->first_reach.grow(sizeof(int64_t) * ((int64_t)N + 1), st));
+    HX_CUDA(s->first_after.grow(sizeof(int64_t) * ((int64_t)N + 1), st));
+    HX_CUDA(s->part64.grow(sizeof(int64_t) * nblk, st));
+    HX_CUDA(s->part32.grow(sizeof(int32_t) * nblk, st));
+    HX_CUDA(s->d_total.grow(sizeof(int64_t), st));
 
-    k_lr_frames<<<(unsigned)((ng * 32 + 255) / 256), 256, 0, st>>>(d_rank, d_off, n_reads, N, W, s->g_lo, s->g_len,
-                                                                   s->g_hi, h->d_err);
-    k_lr_fix_empty<<<(unsigned)((ng + 255) / 256), 256, 0, st>>>(s->g_lo, s->g_len, ng, d_rank, n_reads);
+    k_lr_frames<<<(unsigned)((ng * 32 + 255) / 256), 256, 0, st>>>(d_rank, d_off, n_reads, N, W, s->g_lo.p, s->g_len.p,
+                                                                   s->g_hi.p, h->d_err.p);
+    k_lr_fix_empty<<<(unsigned)((ng + 255) / 256), 256, 0, st>>>(s->g_lo.p, s->g_len.p, ng, d_rank, n_reads);
     // plane offsets = exclusive sum of the frame lengths; running max of the group ends
-    k_scan_partials<int64_t, 0, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(s->g_len, ng, s->part64);
-    k_scan_spine<int64_t, 0><<<1, 32, 0, st>>>(s->part64, nblk, s->d_total);
-    k_scan_apply<int64_t, 0, ITEMS, true><<<(unsigned)nblk, 256, 0, st>>>(s->g_len, ng, s->part64, s->g_off);
-    k_scan_partials<int32_t, 1, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(s->g_hi, ng, s->part32);
-    k_scan_spine<int32_t, 1><<<1, 32, 0, st>>>(s->part32, nblk, nullptr);
-    k_scan_apply<int32_t, 1, ITEMS, false><<<(unsigned)nblk, 256, 0, st>>>(s->g_hi, ng, s->part32, s->g_hipm);
-    h->launches += 8;
+    k_scan_partials<int64_t, 0, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(s->g_len.p, ng, s->part64.p);
+    k_scan_spine<int64_t, 0><<<1, 32, 0, st>>>(s->part64.p, nblk, s->d_total.p);
+    k_scan_apply<int64_t, 0, ITEMS, true><<<(unsigned)nblk, 256, 0, st>>>(s->g_len.p, ng, s->part64.p, s->g_off.p);
+    k_scan_partials<int32_t, 1, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(s->g_hi.p, ng, s->part32.p);
+    k_scan_spine<int32_t, 1><<<1, 32, 0, st>>>(s->part32.p, nblk, nullptr);
+    k_scan_apply<int32_t, 1, ITEMS, false><<<(unsigned)nblk, 256, 0, st>>>(s->g_hi.p, ng, s->part32.p, s->g_hipm.p);
+    h->use.launches += 8;
     HX_CUDA(cudaGetLastError());
     // The plane buffer is sized by a bound instead of the scan total (no device->host round trip, so chunks of long
     // reads can overlap their copies like the short ones): a group's frame spans the ranks of its 32 rank-sorted
     // reads plus one read, and the rank ranges of consecutive groups do not overlap.
     const int64_t total_sites_bound = (int64_t)N + 1 + ng * ((int64_t)W + 1);
-    if ((rc = grow(&s->planes, &s->cap_planes, 2 * total_sites_bound + 2, st))) return rc;
+    HX_CUDA(s->planes.grow(sizeof(uint4) * (2 * total_sites_bound + 2), st));
 
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
     const int64_t want = (ng * 32 + 255) / 256;
     const int tgrid = (int)(want < (int64_t)sms * 8 ? want : (int64_t)sms * 8);
-    k_lr_transpose<<<tgrid, 256, 0, st>>>(d_rank, d_off, d_codes, n_reads, N, W, s->g_lo, s->g_len, s->g_off,
-                                          s->planes, hx_cnt_ref(h), h->d_totals, h->d_err, sorted_flag);
-    k_lr_site_index<<<(N + 255) / 256, 256, 0, st>>>(s->g_lo, s->g_hipm, ng, N, s->first_reach, s->first_after);
+    k_lr_transpose<<<tgrid, 256, 0, st>>>(d_rank, d_off, d_codes, n_reads, N, W, s->g_lo.p, s->g_len.p, s->g_off.p,
+                                          s->planes.p, hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag);
+    k_lr_site_index<<<(N + 255) / 256, 256, 0, st>>>(s->g_lo.p, s->g_hipm.p, ng, N, s->first_reach.p, s->first_after.p);
     const int nib = (N + LR_TI - 1) / LR_TI;
     const int njb = (W + LR_TI - 1) / LR_TJ + 1;            // J0 = I0 + jb*TJ must reach pi + W for the last row
     // measured (B200, ONT-like reads): with ~10 reads per SNP rank the cp.async-staged tiles win (9.2 vs
     // 11.3 ms for 100k reads), with ~2 per rank the per-group barrier costs more than it hides (3.8 vs 1.4 ms)
     if (n_reads >= 6 * (int64_t)N)
         k_lr_tiles_staged<<<(unsigned)((int64_t)nib * njb), LR_TI * LR_TJ, 0, st>>>(
-            s->planes, s->g_off, s->g_lo, s->g_len, s->first_reach, s->first_after, N, W, njb, hx_cnt_ref(h),
-            h->d_totals, sorted_flag);
+            s->planes.p, s->g_off.p, s->g_lo.p, s->g_len.p, s->first_reach.p, s->first_after.p, N, W, njb, hx_cnt_ref(h),
+            h->d_totals.p, sorted_flag);
     else
         k_lr_tiles<<<(unsigned)((int64_t)nib * njb), LR_TI * LR_TJ, 0, st>>>(
-            s->planes, s->g_off, s->g_lo, s->g_len, s->first_reach, s->first_after, N, W, njb, hx_cnt_ref(h),
-            h->d_totals, sorted_flag);
-    h->launches += 3;
+            s->planes.p, s->g_off.p, s->g_lo.p, s->g_len.p, s->first_reach.p, s->first_after.p, N, W, njb, hx_cnt_ref(h),
+            h->d_totals.p, sorted_flag);
+    h->use.launches += 3;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }

@@ -925,17 +925,6 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
     }
 }
 
-template <typename T>
-int l2_grow(T **p, int64_t *cap, int64_t need, cudaStream_t st) {
-    if (*cap >= need) return HX_OK;
-    if (*p) cudaFreeAsync(*p, st);
-    *p = nullptr;
-    *cap = 0;
-    HX_CUDA(cudaMallocAsync((void **)p, sizeof(T) * (size_t)need, st));
-    *cap = need;
-    return HX_OK;
-}
-
 }  // namespace
 
 #ifdef L2_PROFILE
@@ -951,17 +940,16 @@ extern "C" int hx_debug_l2_prof(unsigned long long *out, int reset) {
 
 // Scratch owned by the matrix for this path (freed in hx_destroy through hx_l2_free).
 struct hx_l2_scratch {
-    int32_t *keys = nullptr, *hist = nullptr, *bstart = nullptr, *perm = nullptr, *chunk_eb = nullptr, *part = nullptr;
-    uint8_t *onehot = nullptr;
-    int64_t cap_keys = 0, cap_hist = 0, cap_bstart = 0, cap_perm = 0, cap_ceb = 0, cap_part = 0, cap_onehot = 0;
+    HxDevBuf<int32_t> keys, hist, bstart, perm, chunk_eb, part;
+    HxDevBuf<uint8_t> onehot;
 };
 
 void hx_l2_free(hx_matrix *h) {
     hx_l2_scratch *s = (hx_l2_scratch *)h->l2_scratch;
     if (!s) return;
-    void *ptrs[] = {s->keys, s->hist, s->bstart, s->perm, s->chunk_eb, s->part, s->onehot};
-    for (void *p : ptrs)
-        if (p) cudaFreeAsync(p, h->stream);
+    cudaStream_t st = h->stream;
+    s->keys.release(st); s->hist.release(st); s->bstart.release(st); s->perm.release(st); s->chunk_eb.release(st);
+    s->part.release(st); s->onehot.release(st);
     delete s;
     h->l2_scratch = nullptr;
 }
@@ -986,53 +974,52 @@ int hx_launch_ingest_lumma(hx_matrix *h, const int32_t *d_rank, const int64_t *d
     constexpr int ITEMS = 16;
     const int64_t nscan = nbins + 1;
     const int64_t nblk = (nscan + 256 * ITEMS - 1) / (256 * ITEMS);
-    int rc;
-    if ((rc = l2_grow(&s->keys, &s->cap_keys, n_reads, st))) return rc;
-    if ((rc = l2_grow(&s->hist, &s->cap_hist, 2 * nscan + 4, st))) return rc;        // histogram | cursors | tile counter
-    if ((rc = l2_grow(&s->bstart, &s->cap_bstart, nscan, st))) return rc;
-    if ((rc = l2_grow(&s->perm, &s->cap_perm, max_chunks * 32, st))) return rc;
-    if ((rc = l2_grow(&s->chunk_eb, &s->cap_ceb, max_chunks, st))) return rc;
-    if ((rc = l2_grow(&s->part, &s->cap_part, nblk, st))) return rc;
+    HX_CUDA(s->keys.grow(sizeof(int32_t) * n_reads, st));
+    HX_CUDA(s->hist.grow(sizeof(int32_t) * (2 * nscan + 4), st));         // histogram | cursors | tile counter
+    HX_CUDA(s->bstart.grow(sizeof(int32_t) * nscan, st));
+    HX_CUDA(s->perm.grow(sizeof(int32_t) * max_chunks * 32, st));
+    HX_CUDA(s->chunk_eb.grow(sizeof(int32_t) * max_chunks, st));
+    HX_CUDA(s->part.grow(sizeof(int32_t) * nblk, st));
     const int64_t onehot_bytes = max_chunks * g.SP * (int64_t)L2_SLAB;
-    if ((rc = l2_grow(&s->onehot, &s->cap_onehot, onehot_bytes + L2P_G * (int64_t)L2_SLAB, st))) return rc;   // + zero slabs
-    int32_t *cursor = s->hist + nscan;
+    HX_CUDA(s->onehot.grow(onehot_bytes + L2P_G * (int64_t)L2_SLAB, st));  // + zero slabs
+    int32_t *cursor = s->hist.p + nscan;
 
-    HX_CUDA(hx_fill_async(s->hist, 0, sizeof(int32_t) * (size_t)(2 * nscan + 4), st));
-    HX_CUDA(hx_fill_async(s->perm, 0xff, sizeof(int32_t) * (size_t)(max_chunks * 32), st));
+    HX_CUDA(hx_fill_async(s->hist.p, 0, sizeof(int32_t) * (size_t)(2 * nscan + 4), st));
+    HX_CUDA(hx_fill_async(s->perm.p, 0xff, sizeof(int32_t) * (size_t)(max_chunks * 32), st));
     const unsigned rgrid = (unsigned)((n_reads + 255) / 256);
-    k_l2_keys<<<rgrid, 256, 0, st>>>(d_rank, d_off, n_reads, g, s->keys, s->hist, h->d_err, go);
-    k_l2_pad<<<(unsigned)((g.NB + 255) / 256), 256, 0, st>>>(s->hist, g, go);
-    k_scan_partials<int32_t, 0, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(s->hist, nscan, s->part);
-    k_scan_spine<int32_t, 0><<<1, 32, 0, st>>>(s->part, nblk, nullptr);
-    k_scan_apply<int32_t, 0, ITEMS, true><<<(unsigned)nblk, 256, 0, st>>>(s->hist, nscan, s->part, s->bstart);
-    k_l2_scatter<<<rgrid, 256, 0, st>>>(s->keys, n_reads, s->bstart, cursor, s->perm, go);
-    k_l2_onehot<<<(unsigned)((max_chunks * 32 + 255) / 256), 256, 0, st>>>(d_rank, d_off, d_codes, s->perm, s->bstart, g,
-                                                                           s->onehot, s->chunk_eb, hx_cnt_ref(h),
-                                                                           h->d_totals, h->d_err, go);
-    k_l2_slabs<<<dim3((unsigned)max_chunks, (unsigned)((g.SP + 7) / 8)), 256, 0, st>>>(d_rank, d_off, d_codes, s->perm, s->bstart, g,
-                                                                                     s->onehot, h->d_totals, h->d_err, go);
+    k_l2_keys<<<rgrid, 256, 0, st>>>(d_rank, d_off, n_reads, g, s->keys.p, s->hist.p, h->d_err.p, go);
+    k_l2_pad<<<(unsigned)((g.NB + 255) / 256), 256, 0, st>>>(s->hist.p, g, go);
+    k_scan_partials<int32_t, 0, ITEMS><<<(unsigned)nblk, 256, 0, st>>>(s->hist.p, nscan, s->part.p);
+    k_scan_spine<int32_t, 0><<<1, 32, 0, st>>>(s->part.p, nblk, nullptr);
+    k_scan_apply<int32_t, 0, ITEMS, true><<<(unsigned)nblk, 256, 0, st>>>(s->hist.p, nscan, s->part.p, s->bstart.p);
+    k_l2_scatter<<<rgrid, 256, 0, st>>>(s->keys.p, n_reads, s->bstart.p, cursor, s->perm.p, go);
+    k_l2_onehot<<<(unsigned)((max_chunks * 32 + 255) / 256), 256, 0, st>>>(d_rank, d_off, d_codes, s->perm.p, s->bstart.p, g,
+                                                                           s->onehot.p, s->chunk_eb.p, hx_cnt_ref(h),
+                                                                           h->d_totals.p, h->d_err.p, go);
+    k_l2_slabs<<<dim3((unsigned)max_chunks, (unsigned)((g.SP + 7) / 8)), 256, 0, st>>>(d_rank, d_off, d_codes, s->perm.p, s->bstart.p, g,
+                                                                                     s->onehot.p, h->d_totals.p, h->d_err.p, go);
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    if (h->ingest_sms > 0 && h->ingest_sms < sms) sms = h->ingest_sms;
+    if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
     const bool fused = h->peer_world > 1;
-    const bool fresh = !fused && h->cnt_fresh;
+    const bool fresh = !fused && h->use.cnt_fresh;
     static const bool pairs_on = getenv("HX_LUMMA_PAIRS") && !strcmp(getenv("HX_LUMMA_PAIRS"), "1");
     if (!fused && sms >= 2 && pairs_on && g.SP <= 62) {
         // CTA pairs (cta_group::2): one cluster of two per TPC
-        uint8_t *zero_slabs = s->onehot + onehot_bytes;
+        uint8_t *zero_slabs = s->onehot.p + onehot_bytes;
         HX_CUDA(hx_fill_async(zero_slabs, 0, L2P_G * (size_t)L2_SLAB, st));
         const size_t smem = (size_t)L2P_STAGES * L2P_STAGE_BYTES + (size_t)L2_EP_WARPS * L2_STG_WORDS * 4 + 1024;
         auto kern = fresh ? k_l2_tiles2<true> : k_l2_tiles2<false>;
         HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<sms & ~1, L2P_THREADS, smem, st>>>(s->onehot, zero_slabs, s->bstart, g, hx_cnt_ref(h), h->d_totals, go);
-        h->launches++;
+        kern<<<sms & ~1, L2P_THREADS, smem, st>>>(s->onehot.p, zero_slabs, s->bstart.p, g, hx_cnt_ref(h), h->d_totals.p, go);
+        h->use.launches++;
     } else {
         const size_t smem = (size_t)L2_STAGES * L2_STAGE_BYTES + (size_t)L2_EP_WARPS * L2_STG_WORDS * 4 + 1024;
         auto kern = fused ? k_l2_tiles<true, false> : (fresh ? k_l2_tiles<false, true> : k_l2_tiles<false, false>);
         HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<sms, L2_THREADS, smem, st>>>(s->onehot, s->bstart, g, hx_cnt_ref(h), h->d_totals, go);
+        kern<<<sms, L2_THREADS, smem, st>>>(s->onehot.p, s->bstart.p, g, hx_cnt_ref(h), h->d_totals.p, go);
     }
-    h->launches += 11;
+    h->use.launches += 11;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }

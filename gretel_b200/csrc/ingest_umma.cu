@@ -686,18 +686,18 @@ int hx_launch_ingest_umma(hx_matrix *h, const int32_t *d_rank, const int64_t *d_
                           int64_t n_reads, const int64_t *run_end, const int *sorted_flag) {
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    if (h->ingest_sms > 0 && h->ingest_sms < sms) sms = h->ingest_sms;
+    if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
     const int kmax = h->W + 1;
     const bool fused = h->peer_world > 1;
     const size_t smem = UmLayout{kmax}.bytes();
     int64_t grid = sms;
     const int64_t max_useful = (n_reads + 255) / 256;          // no thinner than 256 reads per CTA
     if (grid > max_useful) grid = max_useful;
-    int32_t *run_rank = reinterpret_cast<int32_t *>(h->d_run_list);
-    int64_t *run_stop = reinterpret_cast<int64_t *>(h->d_run_list) + (((size_t)h->N + 2 + 1) / 2);
+    int32_t *run_rank = reinterpret_cast<int32_t *>(h->d_run_list.p);
+    int64_t *run_stop = reinterpret_cast<int64_t *>(h->d_run_list.p) + (((size_t)h->N + 2 + 1) / 2);
     int *n_runs = reinterpret_cast<int *>(run_stop + (size_t)h->N + 2);
     k_run_list<<<1, 1024, 0, h->stream>>>(run_end, h->N, run_rank, run_stop, n_runs);
-    h->launches++;
+    h->use.launches++;
     // slices hold equal shares of (alleles + read_w * reads + rank_w * ranks spanned) - the per-allele, per-read and
     // per-run costs of the kernel (config 3, tuned on the B200: 16 / 8192 gives 0.330 ms per step, equal read counts
     // 0.373); a read carries at most kmax alleles, so a slice holds at most (kmax + read_w) / read_w times its even
@@ -709,25 +709,20 @@ int hx_launch_ingest_umma(hx_matrix *h, const int32_t *d_rank, const int64_t *d_
     const int64_t jobs_cap = per / 32 + std::min<int64_t>((int64_t)h->N + 2, per) + 2;
     HX_CHECK_ARG(jobs_cap < ((int64_t)1 << 31) && per < ((int64_t)1 << 31));
     const int64_t jobs_bytes = jobs_cap * grid * (int64_t)sizeof(int4);
-    if (jobs_bytes > h->cap_jobs) {
-        if (h->d_jobs) cudaFreeAsync(h->d_jobs, h->stream);
-        h->d_jobs = nullptr; h->cap_jobs = 0;
-        HX_CUDA(cudaMallocAsync(&h->d_jobs, (size_t)(jobs_bytes + jobs_bytes / 8), h->stream));
-        h->cap_jobs = jobs_bytes + jobs_bytes / 8;
-    }
+    if (jobs_bytes > h->d_jobs.cap) HX_CUDA(h->d_jobs.grow(jobs_bytes + jobs_bytes / 8, h->stream));   // with headroom
 #define HX_UM_LAUNCH(CH_)                                                                                       \
     do {                                                                                                        \
         auto kern = fused ? k1_umma<CH_, true> : k1_umma<CH_, false>;                                           \
         HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
         kern<<<(unsigned)grid, UM_THREADS, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax, \
-                                                              hx_cnt_ref(h), h->d_totals, h->d_err, sorted_flag, \
+                                                              hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag, \
                                                               run_rank, run_stop, n_runs,                       \
-                                                              reinterpret_cast<int4 *>(h->d_jobs), (int)jobs_cap, read_w, rank_w); \
+                                                              h->d_jobs.p, (int)jobs_cap, read_w, rank_w); \
     } while (0)
     if (kmax <= 16) HX_UM_LAUNCH(4);
     else HX_UM_LAUNCH(8);
 #undef HX_UM_LAUNCH
-    h->launches++;
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }

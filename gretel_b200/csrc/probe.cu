@@ -64,7 +64,7 @@ int hx_probe_expected_rows(hx_matrix *h, const int32_t *d_rank, const int64_t *d
     HX_CUDA(cudaSetDevice(h->device));
     k_probe_expected_rows<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(
         d_rank, d_off, d_codes, n_reads, h->N, h->W, reinterpret_cast<unsigned long long *>(d_rows));
-    h->launches++;
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }
@@ -75,7 +75,7 @@ int hx_counts_row_sums(hx_matrix *h, uint64_t *d_rows) {
     HX_CUDA(cudaSetDevice(h->device));
     k_counts_row_sums<<<(unsigned)(h->N + 2), 256, 0, h->stream>>>(h->cnt, (int64_t)h->W * HX_CELL, (int64_t)h->N + 2,
                                                                reinterpret_cast<unsigned long long *>(d_rows));
-    h->launches++;
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }

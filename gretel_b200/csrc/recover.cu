@@ -919,28 +919,17 @@ __global__ void k_reweight_matrix(float *__restrict__ band, int64_t n, double ra
     }
 }
 
-int ensure_buf(void **p, int64_t *cap, int64_t need_bytes, cudaStream_t st) {
-    if (*cap >= need_bytes) return HX_OK;
-    if (*p) cudaFreeAsync(*p, st);
-    *p = nullptr;
-    *cap = 0;
-    HX_CUDA(cudaMallocAsync(p, (size_t)need_bytes, st));
-    *cap = need_bytes;
-    return HX_OK;
-}
-
 int launch_reweight(hx_matrix *h, const uint8_t *d_path, const double *d_ratio, double ratio,
                     double *d_removed) {
     constexpr int BLOCK = 256;
     const int64_t cells = ((int64_t)h->N + 1) * h->W;
     const int64_t grid = (cells + BLOCK - 1) / BLOCK;
-    int rc = ensure_buf((void **)&h->d_partials, &h->cap_partials, grid * (int64_t)sizeof(double), h->stream);
-    if (rc) return rc;
-    k_reweight_path<BLOCK><<<(unsigned)grid, BLOCK, 0, h->stream>>>(h->band, h->N, h->W, d_path, d_ratio,
-                                                                    ratio, h->d_partials, h->d_flags);
-    k_sum_partials<<<1, 1024, 0, h->stream>>>(h->d_partials, grid, d_removed);
-    h->launches += 2;
-    h->counts_dirty = true;
+    HX_CUDA(h->d_partials.grow(grid * (int64_t)sizeof(double), h->stream));
+    k_reweight_path<BLOCK><<<(unsigned)grid, BLOCK, 0, h->stream>>>(h->band.p, h->N, h->W, d_path, d_ratio,
+                                                                    ratio, h->d_partials.p, h->d_flags.p);
+    k_sum_partials<<<1, 1024, 0, h->stream>>>(h->d_partials.p, grid, d_removed);
+    h->use.launches += 2;
+    h->use.counts_dirty = true;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }
@@ -948,7 +937,7 @@ int launch_reweight(hx_matrix *h, const uint8_t *d_path, const double *d_ratio, 
 // the ordered sums of every haplotype enqueued so far are done before anything later on the main stream
 int join_sums(hx_matrix *cur) {
     for (int b = 0; b < 2; ++b)
-        if (cur->sum_busy[b]) { HX_CUDA(cudaStreamWaitEvent(cur->stream, cur->sum_done[b], 0)); cur->sum_busy[b] = false; }
+        if (cur->use.sum_busy[b]) { HX_CUDA(cudaStreamWaitEvent(cur->stream, cur->sum_done[b], 0)); cur->use.sum_busy[b] = false; }
     return HX_OK;
 }
 
@@ -969,16 +958,14 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
     const int64_t n_all = n_terms + ((int64_t)N + 2) * 8;
     const int64_t n_termsq = ((int64_t)N + 2) * Lq * HX_NSYM * 8;
     const int64_t n_allq = n_termsq + ((int64_t)N + 2) * 8;
-    rc = ensure_buf((void **)&cur->d_terms, &cur->cap_terms, (n_all + (use_q ? (n_allq + 1) / 2 + 8 : 0)) * (int64_t)sizeof(double),
-                    cur->stream);
-    if (rc) return rc;
-    double *logm = cur->d_terms + n_terms;
-    int32_t *termsq = use_q ? reinterpret_cast<int32_t *>(cur->d_terms + n_all) : nullptr;
+    HX_CUDA(cur->d_terms.grow((n_all + (use_q ? (n_allq + 1) / 2 + 8 : 0)) * (int64_t)sizeof(double), cur->stream));
+    double *logm = cur->d_terms.p + n_terms;
+    int32_t *termsq = use_q ? reinterpret_cast<int32_t *>(cur->d_terms.p + n_all) : nullptr;
     int32_t *logmq = use_q ? termsq + n_termsq : nullptr;
     const int64_t tthreads = (int64_t)(N + 1) * (Lw > Lq ? Lw : Lq) * 8;
-    k_walk_terms<<<(unsigned)((tthreads + 255) / 256), 256, 0, cur->stream>>>(cur->band, cur->vseen, N, cur->W, Lw,
-                                                                              flags, cur->d_terms, termsq, Lq,
-                                                                              cur->d_flags + 2);
+    k_walk_terms<<<(unsigned)((tthreads + 255) / 256), 256, 0, cur->stream>>>(cur->band.p, cur->vseen.p, N, cur->W, Lw,
+                                                                              flags, cur->d_terms.p, termsq, Lq,
+                                                                              cur->d_flags.p + 2);
     // parallel-in-time walk (k_walk_q): blocks of sites walked concurrently from a guessed history, then verified
     int n_blocks = 1, blk_len = N > 0 ? N : 1, warm = 0;
     static const int blocks_env = getenv("HX_WALK_BLOCKS") ? atoi(getenv("HX_WALK_BLOCKS")) : 0;   // 1 = sequential
@@ -990,18 +977,17 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
         n_blocks = (N + blk_len - 1) / blk_len;
     }
     const int spec_stride = blk_len + warm;
-    rc = ensure_buf((void **)&cur->d_spec, &cur->cap_spec, (int64_t)n_blocks * HX_WALK_CAND * spec_stride + (int64_t)N + 2 + 8 * (int64_t)n_blocks * HX_WALK_CAND + 64,
-                    cur->stream);
-    if (rc) return rc;
-    uint8_t *spec = cur->d_spec;
+    HX_CUDA(cur->d_spec.grow((int64_t)n_blocks * HX_WALK_CAND * spec_stride + (int64_t)N + 2 + 8 * (int64_t)n_blocks * HX_WALK_CAND + 64,
+                             cur->stream));
+    uint8_t *spec = cur->d_spec.p;
     uint8_t *guess = spec + (size_t)n_blocks * HX_WALK_CAND * spec_stride;
     const uint8_t *paths0 = d_path - (size_t)n_prev * ((size_t)N + 1);              // the haplotypes found so far (hx_recover)
     int *spec_ok = reinterpret_cast<int *>(reinterpret_cast<uintptr_t>(guess + (size_t)N + 2 + 15) & ~(uintptr_t)15);
     int *cand_idx = spec_ok + (size_t)n_blocks * HX_WALK_CAND;
-    k_walk_logm<<<(N + 1 + 127) / 128, 128, 0, cur->stream>>>(cur->scnt, N, flags, logm, logmq, guess);
+    k_walk_logm<<<(N + 1 + 127) / 128, 128, 0, cur->stream>>>(cur->scnt.p, N, flags, logm, logmq, guess);
     if (n_blocks > 1) {
         k_walk_pick<<<n_blocks, 32, 0, cur->stream>>>(paths0, n_prev, N, L, blk_len, cand_idx);
-        cur->launches++;
+        cur->use.launches++;
     }
     // sites per staged chunk: three chunks (terms + log-marginals) must fit in shared memory
     const int64_t site_bytes = (int64_t)Lw * 448 + 64;
@@ -1016,14 +1002,14 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
     case NIT:                                                                                                       \
         HX_CUDA(cudaFuncSetAttribute(k_walk_q<NIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qsmem));      \
         k_walk_q<NIT><<<1 + (n_blocks - 1) * HX_WALK_CAND, 32, qsmem, cur->stream>>>(                                  \
-            termsq, logmq, cur->d_terms, logm, N, L, Cq, blk_len, warm, guess, paths0, cand_idx, spec, spec_stride,    \
-            spec_ok, d_path, cur->d_flags);                                                                         \
+            termsq, logmq, cur->d_terms.p, logm, N, L, Cq, blk_len, warm, guess, paths0, cand_idx, spec, spec_stride,  \
+            spec_ok, d_path, cur->d_flags.p);                                                                       \
         if (n_blocks > 1) {                                                                                         \
             HX_CUDA(cudaFuncSetAttribute(k_walk_fix<NIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qsmem)); \
-            k_walk_fix<NIT><<<1, 32, qsmem, cur->stream>>>(termsq, logmq, cur->d_terms, logm, N, L, Cq, blk_len, warm, \
+            k_walk_fix<NIT><<<1, 32, qsmem, cur->stream>>>(termsq, logmq, cur->d_terms.p, logm, N, L, Cq, blk_len, warm, \
                                                            n_blocks, paths0, cand_idx, spec, spec_stride, spec_ok,     \
-                                                           d_path, cur->d_flags);                                       \
-            cur->launches++;                                                                                        \
+                                                           d_path, cur->d_flags.p);                                     \
+            cur->use.launches++;                                                                                    \
         }                                                                                                           \
         break;
         switch (nit) {
@@ -1032,31 +1018,31 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
         }
 #undef HX_WALK_Q
     } else if (C < 1) {
-        k_walk_wide<<<1, 256, 0, cur->stream>>>(cur->d_terms, logm, cur->vseen, N, L, Lw, flags, d_path, cur->d_flags);
+        k_walk_wide<<<1, 256, 0, cur->stream>>>(cur->d_terms.p, logm, cur->vseen.p, N, L, Lw, flags, d_path, cur->d_flags.p);
     } else {
         const size_t wsmem = (size_t)3 * C * site_bytes;
         HX_CUDA(cudaFuncSetAttribute(k_walk_tables, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
-        k_walk_tables<<<1, 32, wsmem, cur->stream>>>(cur->d_terms, logm, cur->vseen, N, L, Lw, flags, C, d_path,
-                                                     cur->d_flags);
+        k_walk_tables<<<1, 32, wsmem, cur->stream>>>(cur->d_terms.p, logm, cur->vseen.p, N, L, Lw, flags, C, d_path,
+                                                     cur->d_flags.p);
     }
-    cur->launches += 2;
+    cur->use.launches += 2;
     // per-site values of this haplotype: two alternating buffers, so that the ordered sums of haplotype `it` (side
     // stream) may still be running while haplotype it+1 is walked
-    double *site = cur->d_site + (size_t)(it & 1) * 3 * ((size_t)N + 2);
+    double *site = cur->d_site.p + (size_t)(it & 1) * 3 * ((size_t)N + 2);
     if (!cur->sum_stream) {
         HX_CUDA(cudaStreamCreateWithFlags(&cur->sum_stream, cudaStreamNonBlocking));
         for (int b = 0; b < 2; ++b) HX_CUDA(cudaEventCreateWithFlags(&cur->sum_done[b], cudaEventDisableTiming));
         HX_CUDA(cudaEventCreateWithFlags(&cur->site_ready, cudaEventDisableTiming));
     }
-    if (cur->sum_busy[it & 1]) HX_CUDA(cudaStreamWaitEvent(cur->stream, cur->sum_done[it & 1], 0));
-    k_path_stats<<<(N + 255) / 256, 256, 0, cur->stream>>>(cur->scnt, orig->scnt, N, d_path, site, cur->d_flags);
-    k_path_min<<<1, 1024, 0, cur->stream>>>(site, N, min_remove, d_stats, cur->d_flags);
+    if (cur->use.sum_busy[it & 1]) HX_CUDA(cudaStreamWaitEvent(cur->stream, cur->sum_done[it & 1], 0));
+    k_path_stats<<<(N + 255) / 256, 256, 0, cur->stream>>>(cur->scnt.p, orig->scnt.p, N, d_path, site, cur->d_flags.p);
+    k_path_min<<<1, 1024, 0, cur->stream>>>(site, N, min_remove, d_stats, cur->d_flags.p);
     HX_CUDA(cudaEventRecord(cur->site_ready, cur->stream));
     HX_CUDA(cudaStreamWaitEvent(cur->sum_stream, cur->site_ready, 0));
     k_path_sum<<<1, 256, 0, cur->sum_stream>>>(site, N, d_stats);
     HX_CUDA(cudaEventRecord(cur->sum_done[it & 1], cur->sum_stream));
-    cur->sum_busy[it & 1] = true;
-    cur->launches += 4;
+    cur->use.sum_busy[it & 1] = true;
+    cur->use.launches += 4;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }
@@ -1067,17 +1053,17 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
 extern "C" int hx_debug_walk_redone(hx_matrix *h, int *n) {
     if (!h || !n) return HX_E_ARG;
     if (cudaSetDevice(h->device) != cudaSuccess) return HX_E_CUDA;
-    if (cudaMemcpyAsync(n, h->d_flags + 3, sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return HX_E_CUDA;
+    if (cudaMemcpyAsync(n, h->d_flags.p + 3, sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return HX_E_CUDA;
     if (cudaStreamSynchronize(h->stream) != cudaSuccess) return HX_E_CUDA;
     return HX_OK;
 }
 
 int hx_ensure_counts(hx_matrix *h) {
-    if (!h->counts_dirty) return HX_OK;
-    k_site_counts<<<(h->N + 1 + 127) / 128, 128, 0, h->stream>>>(h->band, h->N, h->W, h->scnt, h->vseen);
-    h->launches++;
+    if (!h->use.counts_dirty) return HX_OK;
+    k_site_counts<<<(h->N + 1 + 127) / 128, 128, 0, h->stream>>>(h->band.p, h->N, h->W, h->scnt.p, h->vseen.p);
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
-    h->counts_dirty = false;
+    h->use.counts_dirty = false;
     return HX_OK;
 }
 
@@ -1089,7 +1075,7 @@ int hx_counts_all(hx_matrix *h, double *out) {
     HX_CUDA(cudaSetDevice(h->device));
     int rc = hx_ensure_counts(h);
     if (rc) return rc;
-    HX_CUDA(cudaMemcpyAsync(out, h->scnt, sizeof(double) * 8 * ((size_t)h->N + 1), cudaMemcpyDeviceToHost,
+    HX_CUDA(cudaMemcpyAsync(out, h->scnt.p, sizeof(double) * 8 * ((size_t)h->N + 1), cudaMemcpyDeviceToHost,
                             h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     return HX_OK;
@@ -1101,7 +1087,7 @@ int hx_marginal_of_at(hx_matrix *h, int sym, int32_t pos, double *out) {
     int rc = hx_ensure_counts(h);
     if (rc) return rc;
     double row[8];
-    HX_CUDA(cudaMemcpyAsync(row, h->scnt + (size_t)pos * 8, sizeof(row), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(row, h->scnt.p + (size_t)pos * 8, sizeof(row), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     *out = row[7] == 0 ? 0.0 : row[sym] / row[7];
     return HX_OK;
@@ -1113,14 +1099,13 @@ int hx_edge_weights_at(hx_matrix *h, int32_t snp, const uint8_t *path, int32_t L
     HX_CUDA(cudaSetDevice(h->device));
     int rc = hx_ensure_counts(h);
     if (rc) return rc;
-    rc = ensure_buf((void **)&h->d_path, &h->cap_path, (int64_t)h->N + 2, h->stream);
-    if (rc) return rc;
-    HX_CUDA(cudaMemcpyAsync(h->d_path, path, (size_t)snp, cudaMemcpyHostToDevice, h->stream));
-    k_edge_one<<<1, 32, 0, h->stream>>>(h->band, h->scnt, h->vseen, h->W, L, flags, snp, h->d_path, h->d_misc);
-    h->launches++;
+    HX_CUDA(h->d_path.grow((int64_t)h->N + 2, h->stream));
+    HX_CUDA(cudaMemcpyAsync(h->d_path.p, path, (size_t)snp, cudaMemcpyHostToDevice, h->stream));
+    k_edge_one<<<1, 32, 0, h->stream>>>(h->band.p, h->scnt.p, h->vseen.p, h->W, L, flags, snp, h->d_path.p, h->d_misc.p);
+    h->use.launches++;
     HX_CUDA(cudaGetLastError());
     double res[9];
-    HX_CUDA(cudaMemcpyAsync(res, h->d_misc, sizeof(res), cudaMemcpyDeviceToHost, h->stream));
+    HX_CUDA(cudaMemcpyAsync(res, h->d_misc.p, sizeof(res), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     for (int s = 0; s < 7; ++s) weights[s] = res[s];
     *total = res[7];
@@ -1134,33 +1119,31 @@ int hx_generate_path(hx_matrix *cur, hx_matrix *orig, int32_t L, int flags, uint
     HX_CHECK_ARG(cur->N == orig->N && cur->device == orig->device && L >= 0 && L <= HX_MAX_L);
     HX_CUDA(cudaSetDevice(cur->device));
     const int N = cur->N;
-    int rc = ensure_buf((void **)&cur->d_path, &cur->cap_path, (int64_t)N + 2, cur->stream);
-    if (rc) return rc;
-    rc = ensure_buf((void **)&cur->d_stats, &cur->cap_stats, 8 * (int64_t)sizeof(double), cur->stream);
-    if (rc) return rc;
+    HX_CUDA(cur->d_path.grow((int64_t)N + 2, cur->stream));
+    HX_CUDA(cur->d_stats.grow(8 * (int64_t)sizeof(double), cur->stream));
     // orig's counts are produced on orig's stream; order them before our walk
-    if (orig->stream != cur->stream && orig->counts_dirty) {
-        rc = hx_ensure_counts(orig);
+    if (orig->stream != cur->stream && orig->use.counts_dirty) {
+        const int rc = hx_ensure_counts(orig);
         if (rc) return rc;
         HX_CUDA(cudaStreamSynchronize(orig->stream));
     }
-    HX_CUDA(cudaMemsetAsync(cur->d_flags, 0, 3 * sizeof(int), cur->stream));
+    HX_CUDA(cudaMemsetAsync(cur->d_flags.p, 0, 3 * sizeof(int), cur->stream));
     HX_CUDA(cudaEventRecord(cur->ev0, cur->stream));
     // (the single-haplotype entry point: stats[5] must start at 0 for the hole test of the ordered sums)
-    HX_CUDA(cudaMemsetAsync(cur->d_stats, 0, 8 * sizeof(double), cur->stream));
-    rc = launch_generate(cur, orig, L, flags, cur->d_path, cur->d_stats, 0.0);
+    HX_CUDA(cudaMemsetAsync(cur->d_stats.p, 0, 8 * sizeof(double), cur->stream));
+    int rc = launch_generate(cur, orig, L, flags, cur->d_path.p, cur->d_stats.p, 0.0);
     if (rc) return rc;
     rc = join_sums(cur);
     if (rc) return rc;
     HX_CUDA(cudaEventRecord(cur->ev1, cur->stream));
-    cur->ev_rec = true;
+    cur->use.ev_rec = true;
     int hflags[2];
     double stats[8];
-    HX_CUDA(cudaMemcpyAsync(hflags, cur->d_flags, sizeof(hflags), cudaMemcpyDeviceToHost, cur->stream));
-    HX_CUDA(cudaMemcpyAsync(stats, cur->d_stats, sizeof(stats), cudaMemcpyDeviceToHost, cur->stream));
-    HX_CUDA(cudaMemcpyAsync(out_path, cur->d_path, (size_t)N + 1, cudaMemcpyDeviceToHost, cur->stream));
+    HX_CUDA(cudaMemcpyAsync(hflags, cur->d_flags.p, sizeof(hflags), cudaMemcpyDeviceToHost, cur->stream));
+    HX_CUDA(cudaMemcpyAsync(stats, cur->d_stats.p, sizeof(stats), cudaMemcpyDeviceToHost, cur->stream));
+    HX_CUDA(cudaMemcpyAsync(out_path, cur->d_path.p, (size_t)N + 1, cudaMemcpyDeviceToHost, cur->stream));
     HX_CUDA(cudaStreamSynchronize(cur->stream));
-    cudaEventElapsedTime(&cur->last_ms[1], cur->ev0, cur->ev1);
+    cudaEventElapsedTime(&cur->use.last_ms[1], cur->ev0, cur->ev1);
     if (hflags[1]) {
         *hole_site = hflags[0];
         return HX_HOLE;
@@ -1173,18 +1156,17 @@ int hx_generate_path(hx_matrix *cur, hx_matrix *orig, int32_t L, int flags, uint
 int hx_reweight_path(hx_matrix *h, const uint8_t *path, double ratio, double *removed) {
     HX_CHECK_ARG(h && path && removed);
     HX_CUDA(cudaSetDevice(h->device));
-    int rc = ensure_buf((void **)&h->d_path, &h->cap_path, (int64_t)h->N + 2, h->stream);
-    if (rc) return rc;
-    HX_CUDA(cudaMemsetAsync(h->d_flags, 0, 3 * sizeof(int), h->stream));
-    HX_CUDA(cudaMemcpyAsync(h->d_path, path, (size_t)h->N + 1, cudaMemcpyHostToDevice, h->stream));
+    HX_CUDA(h->d_path.grow((int64_t)h->N + 2, h->stream));
+    HX_CUDA(cudaMemsetAsync(h->d_flags.p, 0, 3 * sizeof(int), h->stream));
+    HX_CUDA(cudaMemcpyAsync(h->d_path.p, path, (size_t)h->N + 1, cudaMemcpyHostToDevice, h->stream));
     HX_CUDA(cudaEventRecord(h->ev0, h->stream));
-    rc = launch_reweight(h, h->d_path, nullptr, ratio, h->d_misc);
+    const int rc = launch_reweight(h, h->d_path.p, nullptr, ratio, h->d_misc.p);
     if (rc) return rc;
     HX_CUDA(cudaEventRecord(h->ev1, h->stream));
-    h->ev_rec = true;
-    HX_CUDA(cudaMemcpyAsync(removed, h->d_misc, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    h->use.ev_rec = true;
+    HX_CUDA(cudaMemcpyAsync(removed, h->d_misc.p, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
-    cudaEventElapsedTime(&h->last_ms[2], h->ev0, h->ev1);
+    cudaEventElapsedTime(&h->use.last_ms[2], h->ev0, h->ev1);
     return HX_OK;
 }
 
@@ -1196,43 +1178,41 @@ int hx_recover(hx_matrix *cur, hx_matrix *orig, int32_t L, int flags, int32_t ma
     const int64_t N = cur->N;
     *n_found = 0;
     if (max_paths == 0) return HX_OK;
-    int rc = ensure_buf((void **)&cur->d_path, &cur->cap_path, (N + 1) * (int64_t)max_paths, cur->stream);
-    if (rc) return rc;
-    rc = ensure_buf((void **)&cur->d_stats, &cur->cap_stats, 8 * (int64_t)sizeof(double) * max_paths, cur->stream);
-    if (rc) return rc;
-    if (orig->stream != cur->stream && orig->counts_dirty) {
-        rc = hx_ensure_counts(orig);
+    HX_CUDA(cur->d_path.grow((N + 1) * (int64_t)max_paths, cur->stream));
+    HX_CUDA(cur->d_stats.grow(8 * (int64_t)sizeof(double) * max_paths, cur->stream));
+    if (orig->stream != cur->stream && orig->use.counts_dirty) {
+        const int rc = hx_ensure_counts(orig);
         if (rc) return rc;
         HX_CUDA(cudaStreamSynchronize(orig->stream));
     }
-    HX_CUDA(cudaMemsetAsync(cur->d_flags, 0, 3 * sizeof(int), cur->stream));
-    HX_CUDA(cudaMemsetAsync(cur->d_stats, 0, 8 * sizeof(double) * (size_t)max_paths, cur->stream));
+    HX_CUDA(cudaMemsetAsync(cur->d_flags.p, 0, 3 * sizeof(int), cur->stream));
+    HX_CUDA(cudaMemsetAsync(cur->d_stats.p, 0, 8 * sizeof(double) * (size_t)max_paths, cur->stream));
     HX_CUDA(cudaEventRecord(cur->ev0, cur->stream));
     for (int it = 0; it < max_paths; ++it) {
-        uint8_t *dp = cur->d_path + (size_t)it * (N + 1);
-        double *ds = cur->d_stats + (size_t)it * 8;
-        rc = launch_generate(cur, orig, L, flags, dp, ds, min_remove, it, it);
+        uint8_t *dp = cur->d_path.p + (size_t)it * (N + 1);
+        double *ds = cur->d_stats.p + (size_t)it * 8;
+        int rc = launch_generate(cur, orig, L, flags, dp, ds, min_remove, it, it);
         if (rc) return rc;
         rc = launch_reweight(cur, dp, ds + 3, 0.0, ds + 4);
         if (rc) return rc;
     }
-    rc = join_sums(cur);
+    const int rc = join_sums(cur);
     if (rc) return rc;
     HX_CUDA(cudaEventRecord(cur->ev1, cur->stream));
-    cur->ev_rec = true;
+    cur->use.ev_rec = true;
     double *hs = (double *)malloc(sizeof(double) * 8 * (size_t)max_paths);
     if (!hs) return HX_E_NOMEM;
-    cudaError_t e = cudaMemcpyAsync(hs, cur->d_stats, sizeof(double) * 8 * (size_t)max_paths,
+    cudaError_t e = cudaMemcpyAsync(hs, cur->d_stats.p, sizeof(double) * 8 * (size_t)max_paths,
                                     cudaMemcpyDeviceToHost, cur->stream);
     if (e == cudaSuccess)
-        e = cudaMemcpyAsync(paths, cur->d_path, (size_t)(N + 1) * max_paths, cudaMemcpyDeviceToHost, cur->stream);
+        e = cudaMemcpyAsync(paths, cur->d_path.p, (size_t)(N + 1) * max_paths, cudaMemcpyDeviceToHost, cur->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(cur->stream);
     if (e != cudaSuccess) {
         free(hs);
         hx_set_error("hx_recover: %s", cudaGetErrorString(e));
         return HX_E_CUDA;
     }
-    cudaEventElapsedTime(&cur->last_ms[1], cur->ev0, cur->ev1);
+    cudaEventElapsedTime(&cur->use.last_ms[1], cur->ev0, cur->ev1);
     int found = 0;
     for (int it = 0; it < max_paths; ++it) {
         if (hs[(size_t)it * 8 + 5] != 1.0) break;
@@ -1248,9 +1228,9 @@ int hx_reweight_matrix(hx_matrix *h, double ratio) {
     HX_CHECK_ARG(h);
     HX_CUDA(cudaSetDevice(h->device));
     const int64_t n = h->band_elems;
-    k_reweight_matrix<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->band, n, ratio);
-    h->launches++;
-    h->counts_dirty = true;
+    k_reweight_matrix<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->band.p, n, ratio);
+    h->use.launches++;
+    h->use.counts_dirty = true;
     HX_CUDA(cudaGetLastError());
     return HX_OK;
 }

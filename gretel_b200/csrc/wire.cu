@@ -241,17 +241,6 @@ void trace_mark(int which, cudaStream_t s) {
     cudaEventRecord(g_trace.ev[g_trace.n][which], s);
 }
 
-int ensure(void **p, int64_t *cap, int64_t bytes, cudaStream_t st, bool *grew) {
-    if (bytes <= *cap && *p) return HX_OK;
-    *grew = true;
-    if (*p) cudaFreeAsync(*p, st);
-    *p = nullptr;
-    *cap = 0;
-    HX_CUDA(cudaMallocAsync(p, (size_t)bytes, st));
-    *cap = bytes;
-    return HX_OK;
-}
-
 }  // namespace
 
 void hx_wire_trace_dump() {
@@ -269,12 +258,8 @@ void hx_wire_trace_dump() {
 void hx_wire_free(hx_matrix *h) {
     for (int s = 0; s < HX_WIRE_SETS; ++s) {
         hx_wire_set &w = h->wire[s];
-        if (w.raw) cudaFreeAsync(w.raw, h->stream);
-        if (w.rank) cudaFreeAsync(w.rank, h->stream);
-        if (w.off) cudaFreeAsync(w.off, h->stream);
-        if (w.codes) cudaFreeAsync(w.codes, h->stream);
-        if (w.partials) cudaFreeAsync(w.partials, h->stream);
-        if (w.run_end) cudaFreeAsync(w.run_end, h->stream);
+        w.raw.release(h->stream); w.rank.release(h->stream); w.off.release(h->stream);
+        w.codes.release(h->stream); w.partials.release(h->stream); w.run_end.release(h->stream);
         if (w.copied) cudaEventDestroy(w.copied);
         if (w.consumed) cudaEventDestroy(w.consumed);
         if (w.decoded) cudaEventDestroy(w.decoded);
@@ -308,8 +293,8 @@ static int ingest_dense_impl(hx_matrix *h, const uint8_t *rank_delta, const int6
         if (!h->copy_stream) HX_CUDA(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
         if (!h->decode_stream) HX_CUDA(cudaStreamCreateWithFlags(&h->decode_stream, cudaStreamNonBlocking));
         cudaStream_t ds = h->decode_stream;
-        hx_wire_set &w = h->wire[h->wire_next];
-        h->wire_next = (h->wire_next + 1) % HX_WIRE_SETS;
+        hx_wire_set &w = h->wire[h->use.wire_next];
+        h->use.wire_next = (h->use.wire_next + 1) % HX_WIRE_SETS;
         const int64_t n_words = (n_codes + 15) / 16;        // 32-bit words of 2-bit alleles
         const int64_t n_words_sent = raw_codes ? 0 : n_words;
         const int64_t o_rd = 0, o_kl = o_rd + al16(n_reads), o_c2 = o_kl + al16(n_reads * klen_bytes);
@@ -328,24 +313,25 @@ static int ingest_dense_impl(hx_matrix *h, const uint8_t *rank_delta, const int6
                 HX_CUDA(cudaEventCreateWithFlags(&ws.decoded, cudaEventDisableTiming));
             }
             bool grew = false;
-            auto room = [](int64_t b) { return b + b / 8 + 256; };
-            int rc = HX_OK;
-            if (raw_bytes > ws.cap_raw) rc = ensure((void **)&ws.raw, &ws.cap_raw, room(raw_bytes), st, &grew);
-            if (!rc && 4 * n_reads + 16 > ws.cap_rank) rc = ensure((void **)&ws.rank, &ws.cap_rank, room(4 * n_reads + 16), st, &grew);
-            if (!rc && 8 * (n_reads + 1) + 16 > ws.cap_off) rc = ensure((void **)&ws.off, &ws.cap_off, room(8 * (n_reads + 1) + 16), st, &grew);
-            if (!rc && n_words * 16 + 32 > ws.cap_codes) rc = ensure((void **)&ws.codes, &ws.cap_codes, room(n_words * 16 + 32), st, &grew);
-            if (!rc && 16 * nblk + 32 > ws.cap_partials) rc = ensure((void **)&ws.partials, &ws.cap_partials, room(16 * nblk + 32), st, &grew);
-            if (!rc && 8 * ((int64_t)h->N + 2) > ws.cap_run_end) rc = ensure((void **)&ws.run_end, &ws.cap_run_end, 8 * ((int64_t)h->N + 2), st, &grew);
-            if (rc) return rc;
+            // a buffer too small for `need` bytes grows to `need` plus headroom
+            auto fit = [&](auto &buf, int64_t need) {
+                return need > buf.cap ? buf.grow(need + need / 8 + 256, st, &grew) : cudaSuccess;
+            };
+            HX_CUDA(fit(ws.raw, raw_bytes));
+            HX_CUDA(fit(ws.rank, 4 * n_reads + 16));
+            HX_CUDA(fit(ws.off, 8 * (n_reads + 1) + 16));
+            HX_CUDA(fit(ws.codes, n_words * 16 + 32));
+            HX_CUDA(fit(ws.partials, 16 * nblk + 32));
+            HX_CUDA(ws.run_end.grow(8 * ((int64_t)h->N + 2), st, &grew));
             if (grew) HX_CUDA(cudaEventRecord(ws.consumed, st));
         }
         cudaStream_t cs = h->copy_stream;
         HX_CUDA(cudaStreamWaitEvent(cs, w.consumed, 0));
         trace_mark(0, cs);
-        uint8_t *raw = static_cast<uint8_t *>(w.raw);
+        uint8_t *raw = w.raw.p;
         // util.dense_packed lays the arrays out in one host buffer exactly like the staging set: one copy
         const uint8_t *hb = rank_delta;
-        if (raw_codes && n_codes) HX_CUDA(cudaMemcpyAsync(w.codes, raw_codes, (size_t)n_codes, cudaMemcpyHostToDevice, cs));
+        if (raw_codes && n_codes) HX_CUDA(cudaMemcpyAsync(w.codes.p, raw_codes, (size_t)n_codes, cudaMemcpyHostToDevice, cs));
         const bool blob = (const uint8_t *)klen == hb + o_kl && (n_codes == 0 || raw_codes || codes2 == hb + o_c2) &&
                           (n_exc == 0 || (const uint8_t *)exc_pos == hb + o_ex) &&
                           (n_esc == 0 || ((const uint8_t *)esc_idx == hb + o_ei && (const uint8_t *)esc_delta == hb + o_ed));
@@ -367,32 +353,32 @@ static int ingest_dense_impl(hx_matrix *h, const uint8_t *rank_delta, const int6
         HX_CUDA(cudaEventRecord(w.copied, cs));
         // the decode runs on its own stream: it overlaps the previous chunk's expansion and the next chunk's copy
         HX_CUDA(cudaStreamWaitEvent(ds, w.copied, 0));
-        int *ok = reinterpret_cast<int *>(w.partials + 2 * nblk);          // behind the block partials
+        int *ok = reinterpret_cast<int *>(w.partials.p + 2 * nblk);        // behind the block partials
         const int64_t *d_ei = reinterpret_cast<const int64_t *>(raw + o_ei);
         const int32_t *d_ed = reinterpret_cast<const int32_t *>(raw + o_ed);
-        HX_CUDA(hx_fill_async(w.run_end, 0xff, sizeof(int64_t) * ((size_t)h->N + 2), ds));   // -1 = rank without reads
-        h->launches++;
+        HX_CUDA(hx_fill_async(w.run_end.p, 0xff, sizeof(int64_t) * ((size_t)h->N + 2), ds));   // -1 = rank without reads
+        h->use.launches++;
         if (klen_bytes == 1) {
-            k_dense_partials<1><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials);
-            k_dense_spine<<<1, 1024, 0, ds>>>(w.partials, nblk, n_codes, ok, h->d_err);
-            k_dense_apply<1><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials,
-                                                            w.rank, w.off, h->N, w.run_end);
+            k_dense_partials<1><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials.p);
+            k_dense_spine<<<1, 1024, 0, ds>>>(w.partials.p, nblk, n_codes, ok, h->d_err.p);
+            k_dense_apply<1><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials.p,
+                                                            w.rank.p, w.off.p, h->N, w.run_end.p);
         } else {
-            k_dense_partials<2><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials);
-            k_dense_spine<<<1, 1024, 0, ds>>>(w.partials, nblk, n_codes, ok, h->d_err);
-            k_dense_apply<2><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials,
-                                                            w.rank, w.off, h->N, w.run_end);
+            k_dense_partials<2><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials.p);
+            k_dense_spine<<<1, 1024, 0, ds>>>(w.partials.p, nblk, n_codes, ok, h->d_err.p);
+            k_dense_apply<2><<<(unsigned)nblk, 256, 0, ds>>>(raw + o_rd, raw + o_kl, n_reads, d_ei, d_ed, n_esc, w.partials.p,
+                                                            w.rank.p, w.off.p, h->N, w.run_end.p);
         }
-        h->launches += 3;
+        h->use.launches += 3;
         if (n_words_sent) {
             k_unpack_2bit<<<(unsigned)((n_words + 255) / 256), 256, 0, ds>>>(reinterpret_cast<const uint32_t *>(raw + o_c2),
-                                                                            n_words, reinterpret_cast<uint4 *>(w.codes));
-            h->launches++;
+                                                                            n_words, reinterpret_cast<uint4 *>(w.codes.p));
+            h->use.launches++;
         }
         if (n_exc) {
             k_patch_exceptions<<<(unsigned)((n_exc + 255) / 256), 256, 0, ds>>>(
-                reinterpret_cast<const uint32_t *>(raw + o_ex), n_exc, n_codes, w.codes, h->d_err);
-            h->launches++;
+                reinterpret_cast<const uint32_t *>(raw + o_ex), n_exc, n_codes, w.codes.p, h->d_err.p);
+            h->use.launches++;
         }
         HX_CUDA(cudaGetLastError());
         trace_mark(2, ds);
@@ -401,7 +387,7 @@ static int ingest_dense_impl(hx_matrix *h, const uint8_t *rank_delta, const int6
         int rc = hx_ensure_counts_buffer(h);
         if (rc) return rc;
         trace_mark(4, st);
-        rc = hx_launch_ingest_presorted(h, w.rank, w.off, w.codes, n_reads, w.run_end, ok);
+        rc = hx_launch_ingest_presorted(h, w.rank.p, w.off.p, w.codes.p, n_reads, w.run_end.p, ok);
         if (rc) return rc;
         trace_mark(3, st);
         if (g_trace_on && g_trace.n < WireTrace::MAXC) g_trace.bytes[g_trace.n++] = raw_bytes;
