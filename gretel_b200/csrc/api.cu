@@ -148,7 +148,9 @@ void free_all(hx_matrix *h) {
     h->s_rank.release(st); h->s_off.release(st); h->s_codes.release(st);
     h->s_klen.release(st); h->s_codes4.release(st); h->s_scan.release(st);
     h->scnt.release(st); h->vseen.release(st); h->d_path.release(st); h->d_stats.release(st); h->d_site.release(st);
-    h->d_partials.release(st); h->d_spec.release(st); h->d_terms.release(st); h->d_flags.release(st);
+    h->terms.release(st); h->logm.release(st); h->termsq.release(st); h->logmq.release(st);
+    h->spec.release(st); h->guess.release(st); h->spec_ok.release(st); h->cand_idx.release(st);
+    h->d_partials.release(st); h->d_flags.release(st);
     h->d_run_end.release(st); h->d_run_list.release(st); h->d_jobs.release(st); h->d_misc.release(st);
     h->d_pack.release(st);
     if (st) cudaStreamSynchronize(st);
@@ -224,7 +226,7 @@ int reset_parked(hx_matrix *h) {
     HX_CUDA(hx_fill_async(h->band.p, 0, sizeof(float) * (size_t)h->band_elems, h->stream));
     HX_CUDA(hx_fill_async(h->d_totals.p, 0, 8 * sizeof(unsigned long long), h->stream));
     HX_CUDA(hx_fill_async(h->d_err.p, 0, sizeof(int), h->stream));
-    HX_CUDA(hx_fill_async(h->d_flags.p, 0, 8 * sizeof(int), h->stream));
+    HX_CUDA(hx_fill_async(h->d_flags.p, 0, sizeof(hx_dev_flags), h->stream));
     h->use = {};
     return HX_OK;
 }
@@ -278,8 +280,8 @@ int hx_create(int32_t n_snps, int32_t band_w, int32_t device, hx_matrix **out) {
     HX_TRY(h->scnt.grow(sizeof(double) * 8 * ((size_t)n_snps + 2), h->stream));
     HX_TRY(h->vseen.grow(sizeof(int32_t) * ((size_t)n_snps + 2), h->stream));
     HX_TRY(h->d_site.grow(sizeof(double) * 6 * ((size_t)n_snps + 2), h->stream));
-    HX_TRY(h->d_flags.grow(8 * sizeof(int), h->stream));
-    HX_TRY(hx_fill_async(h->d_flags.p, 0, 8 * sizeof(int), h->stream));
+    HX_TRY(h->d_flags.grow(sizeof(hx_dev_flags), h->stream));
+    HX_TRY(hx_fill_async(h->d_flags.p, 0, sizeof(hx_dev_flags), h->stream));
     HX_TRY(h->d_misc.grow(32 * sizeof(double), h->stream));
     HX_TRY(h->d_run_end.grow(sizeof(int64_t) * ((size_t)n_snps + 2), h->stream));
     HX_TRY(h->d_run_list.grow(sizeof(int64_t) * (((size_t)n_snps + 3) / 2 + (size_t)n_snps + 2 + 2), h->stream));
@@ -389,7 +391,7 @@ int hx_ingest_totals(hx_matrix *h, int64_t totals[4]) {
     int *he = (int *)(hp + 8);
     HX_CUDA(cudaMemcpyAsync(hp, h->d_totals.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaMemcpyAsync(he, h->d_err.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    if (h->use.prepass_ran) HX_CUDA(cudaMemcpyAsync(he + 1, h->d_flags.p + 4, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (h->use.prepass_ran) HX_CUDA(cudaMemcpyAsync(he + 1, &h->d_flags.p->ingest_sorted, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     HX_CUDA(cudaStreamSynchronize(h->stream));
     if (h->use.prepass_ran && he[1] == 0) hx_note_unsorted();
     hx_wire_trace_dump();
@@ -594,7 +596,7 @@ int hx_counts_max(hx_matrix *h, uint32_t *max_count) {
     HX_CUDA(cudaSetDevice(h->device));
     int rc = hx_ensure_counts_buffer(h);
     if (rc) return rc;
-    uint32_t *d_out = reinterpret_cast<uint32_t *>(h->d_flags.p + 6);
+    uint32_t *d_out = &h->d_flags.p->counts_max;
     HX_CUDA(hx_fill_async(d_out, 0, sizeof(uint32_t), h->stream));
     k_counts_max<<<592, 256, 0, h->stream>>>(h->cnt, h->cnt_elems, d_out);
     h->use.launches++;

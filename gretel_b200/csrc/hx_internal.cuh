@@ -54,6 +54,28 @@ struct HxDevBuf {
     }
 };
 
+// The device flag word of a matrix (hx_matrix::d_flags), shared by recovery and ingestion.
+struct hx_dev_flags {
+    int hole_site;                   // recovery: the site without a candidate (0 once a walk reached site N)
+    int hole;                        // recovery: a walk met a hole; every later recovery kernel of the launch is a no-op
+    int q_unsafe;                    // recovery: a walk term does not fit the fixed-point tables
+    int walk_redone;                 // sites the parallel-in-time walk walked again since hx_create (hx_debug_walk_redone)
+    int ingest_sorted;               // ingestion: the pre-pass verdict, non-zero = reads sorted by rank
+    int fallback_go;                 // ingestion: non-zero = the counting-sort fallback runs
+    uint32_t counts_max;             // hx_counts_max
+    int pad;
+};
+static_assert(sizeof(hx_dev_flags) == 8 * sizeof(int), "hx_dev_flags is one int[8]");
+
+// What recovery reports for one haplotype (hx_matrix::d_stats).
+struct hx_hap_stats {
+    double hp_current, hp_original;  // ordered log10 sums of the path's marginals in the current / original matrix
+    double min_marginal, ratio, removed;
+    double done;                     // 1.0: the walk reached site N and the statistics are complete
+    double pad[2];
+};
+static_assert(sizeof(hx_hap_stats) == 64, "hx_hap_stats is one double[8]");
+
 #define HX_WIRE_SETS 3
 // One staging set of the dense wire format (wire.cu): raw shipped bytes + the rebuilt packed arrays
 struct hx_wire_set {
@@ -87,14 +109,19 @@ struct hx_matrix {
     HxDevBuf<double> scnt;           // (N+2)*8 per-site counts + total
     HxDevBuf<int32_t> vseen;         // (N+2) valid symbols seen per site
     HxDevBuf<uint8_t> d_path;        // path buffer(s)
-    HxDevBuf<double> d_stats;        // per-iteration stats
+    HxDevBuf<hx_hap_stats> d_stats;  // per-haplotype stats
     HxDevBuf<double> d_site;         // 2 x 3*(N+2) per-site log10 marginal (cur), (orig), marginal (alternating haplotypes)
     cudaStream_t sum_stream;         // the ordered log10 sums of a haplotype run here, off the critical path
     cudaEvent_t sum_done[2], site_ready;
-    HxDevBuf<double> d_terms;        // walk tables: (N+2)*Lw*49 log10 lookback terms + (N+2)*8 log10 marginals
-    HxDevBuf<uint8_t> d_spec;        // speculative block paths, majority-allele guess and block flags of the walk
+    // walk tables (recover.cu): (N+2)*Lw*56 log10 lookback terms, (N+2)*8 log10 marginals, and their int32
+    // fixed-point twins for the quantised walk
+    HxDevBuf<double> terms, logm;
+    HxDevBuf<int32_t> termsq, logmq;
+    // parallel-in-time walk: speculative block paths, the majority-allele guess, per-start results and start picks
+    HxDevBuf<uint8_t> spec, guess;
+    HxDevBuf<int> spec_ok, cand_idx;
     HxDevBuf<double> d_partials;     // block partials of the reweight reduction
-    HxDevBuf<int> d_flags;           // [0] hole site / abort flag, [1..] misc
+    HxDevBuf<hx_dev_flags> d_flags;
     HxDevBuf<int64_t> d_run_end;     // (N+1) end (exclusive) of the run of reads with each rank
     HxDevBuf<int64_t> d_run_list;    // compact run list for the tensor-core kernel: ranks (int32), stops (int64), count
     HxDevBuf<int4> d_jobs;           // per-CTA job tables of the tensor-core kernel (ingest_umma.cu)
@@ -113,7 +140,7 @@ struct hx_matrix {
         bool counts_dirty = true;    // scnt / vseen do not reflect the band yet
         bool cnt_fresh = false;      // cnt is still all zero (nothing ingested / received since it was cleared)
         bool ev_rec = false;         // ev0/ev1 have been recorded at least once
-        bool prepass_ran = false;    // d_flags[4] holds the sortedness verdict of the last ingestion launch
+        bool prepass_ran = false;    // d_flags->ingest_sorted holds the sortedness verdict of the last ingestion launch
         int wire_next = 0;           // the next staging set of the dense wire format
         bool sum_busy[2] = {};       // sum_done[b] marks ordered sums not yet joined into the main stream
         float last_ms[3] = {};
@@ -168,6 +195,34 @@ static inline cudaError_t hx_fill_async(void *p, int byte, size_t bytes, cudaStr
 __host__ __device__ __forceinline__ int64_t hx_cell_off(int64_t W, int64_t pi, int64_t pj) {
     return (pj * W + (pj - pi - 1)) * HX_CELL;
 }
+
+#ifdef __CUDACC__
+// mbarriers and 1-D TMA bulk copies into this CTA's shared memory (addresses are shared-window addresses)
+__device__ __forceinline__ uint32_t hx_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void hx_mbar_init(uint32_t bar, int count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
+}
+__device__ __forceinline__ void hx_mbar_expect_tx(uint32_t bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void hx_mbar_wait(uint32_t bar, uint32_t parity) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "HX_WAIT_%=:\n\t"
+        "mbarrier.try_wait.parity.acquire.cta.shared::cta.b64 p, [%0], %1;\n\t"
+        "@p bra HX_DONE_%=;\n\t"
+        "bra HX_WAIT_%=;\n\t"
+        "HX_DONE_%=:\n\t}" ::"r"(bar),
+        "r"(parity)
+        : "memory");
+}
+// src must be 16-byte aligned, bytes a multiple of 16
+__device__ __forceinline__ void hx_bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
+                 "l"(src), "r"(bytes), "r"(bar)
+                 : "memory");
+}
+#endif
 
 // ingest.cu
 int hx_launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_off,

@@ -531,8 +531,8 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
     for (size_t w = threadIdx.x; w < (size_t)rows * cells * 4; w += blockDim.x) tile[w] = make_uint4(0, 0, 0, 0);
     if (threadIdx.x == 0) {
         for (int b = 0; b < WS_NBUF; ++b) {
-            ws_mbar_init(ws_smem_u32(&s_full[b]), bw);
-            ws_mbar_init(ws_smem_u32(&s_empty[b]), pw);
+            hx_mbar_init(hx_smem_u32(&s_full[b]), bw);
+            hx_mbar_init(hx_smem_u32(&s_empty[b]), pw);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -571,7 +571,7 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
             const int r = run_r;
             const int nb = (bn + 31) >> 5;
             const int b = bi % WS_NBUF;
-            ws_mbar_wait(ws_smem_u32(&s_empty[b]), ((bi / WS_NBUF) & 1) ^ 1);
+            hx_mbar_wait(hx_smem_u32(&s_empty[b]), ((bi / WS_NBUF) & 1) ^ 1);
             int *gk = gk0 + b * 32;
             const int64_t run_stop = bstart + bn;
             for (int g = bwid; g < nb; g += bw) {
@@ -620,7 +620,7 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
                 }
             }
             __syncwarp();
-            if (lane == 0) ws_mbar_arrive(ws_smem_u32(&s_full[b]));
+            if (lane == 0) ws_mbar_arrive(hx_smem_u32(&s_full[b]));
         }
     } else {
         // ================================ pair owners =======================================
@@ -686,7 +686,7 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
 #pragma unroll
                     for (int x = 0; x < 16; ++x) acc[q][x] = 0;
             }
-            ws_mbar_wait(ws_smem_u32(&s_full[b]), (bi / WS_NBUF) & 1);
+            hx_mbar_wait(hx_smem_u32(&s_full[b]), (bi / WS_NBUF) & 1);
             const int *gk = gk0 + b * 32;
             const int bkm = __reduce_max_sync(0xffffffffu, lane < nb ? gk[lane] : 0);
             run_kmax = max(run_kmax, bkm);
@@ -696,7 +696,7 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
                                                t1[q], t2[q], nb, kmax);
             }
             __syncwarp();
-            if (lane == 0) ws_mbar_arrive(ws_smem_u32(&s_empty[b]));
+            if (lane == 0) ws_mbar_arrive(hx_smem_u32(&s_empty[b]));
             if (last) {
 #pragma unroll
                 for (int q = 0; q < NP; ++q) {
@@ -774,7 +774,8 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
     if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
-    const int *sorted_flag = presorted ? ok : h->d_flags.p + 4;
+    int *const verdict = &h->d_flags.p->ingest_sorted;      // the sortedness pre-pass writes its verdict here
+    const int *sorted_flag = presorted ? ok : verdict;
     constexpr int GBLOCK = 256;
     const int64_t gwant = (n_reads + (GBLOCK / 32) - 1) / (GBLOCK / 32);
     const int ggrid = (int)(gwant < (int64_t)sms * 8 ? gwant : (int64_t)sms * 8);
@@ -808,8 +809,8 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
         if (rc) return rc;
     } else if (use_long) {
         if (!presorted) {
-            HX_CUDA(hx_fill_async(h->d_flags.p + 4, 1, sizeof(int), h->stream));     // non-zero = sorted
-            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, h->d_flags.p + 4,
+            HX_CUDA(hx_fill_async(verdict, 1, sizeof(int), h->stream));     // non-zero = sorted
+            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, verdict,
                                                                                 run_end, h->d_err.p);
             h->use.launches++;
         }
@@ -827,8 +828,8 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
     } else {
         if (!presorted) {
             // flag: non-zero = sorted; run_end: -1 = no reads of that rank (the tensor-core kernel walks it)
-            k_prepass_init<<<(unsigned)((h->N + 2 + 255) / 256), 256, 0, h->stream>>>(h->d_flags.p + 4, run_end, use_umma ? h->N + 2 : 0);
-            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, h->d_flags.p + 4,
+            k_prepass_init<<<(unsigned)((h->N + 2 + 255) / 256), 256, 0, h->stream>>>(verdict, run_end, use_umma ? h->N + 2 : 0);
+            k_prepass<<<(unsigned)((n_reads + 255) / 256), 256, 0, h->stream>>>(d_rank, n_reads, h->N, verdict,
                                                                                 run_end, h->d_err.p);
             h->use.launches += 2;
         }
@@ -897,9 +898,9 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
         h->use.launches++;
         // fallback for unsorted input: runs only when the flag says the bit-sliced kernel declined
         if (lumma_fallback) {
-            k_flag_not<<<1, 32, 0, h->stream>>>(h->d_flags.p + 4, h->d_flags.p + 5);
+            k_flag_not<<<1, 32, 0, h->stream>>>(verdict, &h->d_flags.p->fallback_go);
             h->use.launches++;
-            int rc = hx_launch_ingest_lumma(h, d_rank, d_off, d_codes, n_reads, h->d_flags.p + 5);
+            int rc = hx_launch_ingest_lumma(h, d_rank, d_off, d_codes, n_reads, &h->d_flags.p->fallback_go);
             if (rc) return rc;
         } else if (!presorted) {
             k1_pairs_red<GBLOCK><<<ggrid, GBLOCK, 0, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W,

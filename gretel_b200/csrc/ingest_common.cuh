@@ -1,5 +1,5 @@
 // Device helpers shared by the ingestion kernels (ingest.cu, ingest_umma.cu): totals, the per-read side path
-// for rare alleles (N, -, _), L2 prefetch and the mbarrier wrappers.
+// for rare alleles (N, -, _), L2 prefetch and the mbarrier arrive / back-off wait.
 #pragma once
 #include "hx_internal.cuh"
 
@@ -121,25 +121,10 @@ __device__ __forceinline__ void hx_weighted_slice(const int32_t *__restrict__ ra
     hi = s_lohi[1];
 }
 
-__device__ __forceinline__ uint32_t ws_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void ws_mbar_init(uint32_t bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
 __device__ __forceinline__ void ws_mbar_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.release.cta.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
-__device__ __forceinline__ void ws_mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WS_WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.acquire.cta.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra WS_DONE_%=;\n\t"
-        "bra WS_WAIT_%=;\n\t"
-        "WS_DONE_%=:\n\t}" ::"r"(bar),
-        "r"(parity)
-        : "memory");
-}
-// the same with a back-off between polls: for waits that normally last microseconds (many warps waiting)
+// hx_mbar_wait with a back-off between polls: for waits that normally last microseconds (many warps waiting)
 __device__ __forceinline__ void ws_mbar_wait_sleep(uint32_t bar, uint32_t parity) {
     for (;;) {
         uint32_t done;

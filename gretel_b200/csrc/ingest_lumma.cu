@@ -235,14 +235,6 @@ __device__ __forceinline__ void l2_commit(uint32_t bar) {
 }
 __device__ __forceinline__ void l2_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void l2_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void l2_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void l2_bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
 __device__ __forceinline__ void l2_ld32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile(
         "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
@@ -365,22 +357,22 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
     HxCnt cnt = cnt_in;
     if (!FUSED) { cnt.world = 1; cnt.rows_per = 1; cnt.peer = nullptr; }
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint32_t stage0 = ws_smem_u32(l2_smem);
+    const uint32_t stage0 = hx_smem_u32(l2_smem);
     uint32_t *const staging = reinterpret_cast<uint32_t *>(l2_smem + (size_t)L2_STAGES * L2_STAGE_BYTES);
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < L2_STAGES; ++s) {
-            ws_mbar_init(ws_smem_u32(&s_full[s]), 1);
-            ws_mbar_init(ws_smem_u32(&s_empty[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_full[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_empty[s]), 1);
         }
         for (int s = 0; s < 2; ++s) {
-            ws_mbar_init(ws_smem_u32(&s_acc_full[s]), 1);
-            ws_mbar_init(ws_smem_u32(&s_acc_empty[s]), L2_EP_WARPS);
+            hx_mbar_init(hx_smem_u32(&s_acc_full[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_acc_empty[s]), L2_EP_WARPS);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(ws_smem_u32(&s_tmem)),
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(hx_smem_u32(&s_tmem)),
                      "r"(512u)
                      : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -400,7 +392,7 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
         // pieces k = w (mod L2_PW), always into stage w.
         const int64_t n_tiles = (int64_t)g.NB * g.nq;
         const int SPB = g.SPB();
-        const uint32_t bar_full = ws_smem_u32(&s_full[warp]), bar_empty = ws_smem_u32(&s_empty[warp]);
+        const uint32_t bar_full = hx_smem_u32(&s_full[warp]), bar_empty = hx_smem_u32(&s_empty[warp]);
         const uint32_t dst0 = stage0 + (uint32_t)warp * L2_STAGE_BYTES;
         int4 *const runs = s_runs[warp];
         int2 *const pend = s_pend[warp];                 // the stage being collected: up to L2_G chunks (slab of block I, nch | b1)
@@ -420,18 +412,18 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
                 const unsigned b1mask = __ballot_sync(0xffffffffu, slot < n_pend && op == 2 && b1);   // bit 3*slot+2
                 const unsigned n_copies = __popc(__ballot_sync(0xffffffffu, mine));
                 if (lane == 0) {
-                    ws_mbar_wait(bar_empty, ph ^ 1);
+                    hx_mbar_wait(bar_empty, ph ^ 1);
                     // meta: I | q, chunks, B0 present, last, per-chunk "B1 present"
                     unsigned b1bits = 0;
 #pragma unroll
                     for (int i = 0; i < L2_G; ++i) b1bits |= ((b1mask >> (3 * i + 2)) & 1u) << i;
-                    asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(ws_smem_u32(&s_meta[warp][0])), "r"(p_I),
+                    asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(hx_smem_u32(&s_meta[warp][0])), "r"(p_I),
                                  "r"(p_q | (n_pend << 20) | ((b0 | (last << 2)) << 24) | (b1bits << 28))
                                  : "memory");
 #ifdef L2_NOCOPY
-                    l2_expect_tx(bar_full, 0);
+                    hx_mbar_expect_tx(bar_full, 0);
 #else
-                    l2_expect_tx(bar_full, L2_SLAB * n_copies);
+                    hx_mbar_expect_tx(bar_full, L2_SLAB * n_copies);
 #endif
                 }
                 __syncwarp();
@@ -441,7 +433,7 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
                 if (mine) {
 #endif
                     const int slab = c.x + (op ? (2 * p_q - p_I + op - 1) * nch : 0);
-                    l2_bulk_g2s(dst0 + (uint32_t)(op * L2_G + slot) * L2_SLAB, onehot + (size_t)slab * L2_SLAB, L2_SLAB, bar_full);
+                    hx_bulk_g2s(dst0 + (uint32_t)(op * L2_G + slot) * L2_SLAB, onehot + (size_t)slab * L2_SLAB, L2_SLAB, bar_full);
                 }
                 ph ^= 1;
             }
@@ -491,8 +483,8 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
             if (n_pend) emit(1);
         }
         if (turn == (unsigned)warp && lane == 0) {                   // the warp whose turn it is tells the MMA thread to stop
-            ws_mbar_wait(bar_empty, ph ^ 1);
-            asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(ws_smem_u32(&s_meta[warp][0])), "r"(0), "r"(8 << 24) : "memory");
+            hx_mbar_wait(bar_empty, ph ^ 1);
+            asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(hx_smem_u32(&s_meta[warp][0])), "r"(0), "r"(8 << 24) : "memory");
             ws_mbar_arrive(bar_full);
         }
     } else if (warp == L2_PW) {
@@ -509,12 +501,12 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
 #ifdef L2_PROFILE
                 const long long c0 = clock64();
 #endif
-                ws_mbar_wait(ws_smem_u32(&s_full[stage]), ph);
+                hx_mbar_wait(hx_smem_u32(&s_full[stage]), ph);
 #ifdef L2_PROFILE
                 const long long c1 = clock64(); pw += c1 - c0; pn++;
 #endif
                 int m_I, m_w;
-                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(m_I), "=r"(m_w) : "r"(ws_smem_u32(&s_meta[stage][0])) : "memory");
+                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(m_I), "=r"(m_w) : "r"(hx_smem_u32(&s_meta[stage][0])) : "memory");
                 const int m_q = m_w & 0xfffff, m_flags = (m_w >> 24) & 15, n = (m_w >> 20) & 15;
                 const unsigned m_b1 = (unsigned)m_w >> 28;
                 if (m_flags & 8) {
@@ -522,16 +514,16 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
                     atomicAdd(&l2_prof[0], pw); atomicAdd(&l2_prof[1], pi_); atomicAdd(&l2_prof[2], pa); atomicAdd(&l2_prof[3], pn); atomicAdd(&l2_prof[4], pm);
                     atomicAdd(&l2_prof[5], (unsigned long long)(clock64() - t_begin));
 #endif
-                    ws_mbar_wait(ws_smem_u32(&s_acc_empty[acc]), acc_ph[acc] ^ 1);
+                    hx_mbar_wait(hx_smem_u32(&s_acc_empty[acc]), acc_ph[acc] ^ 1);
                     s_tile[acc][3] = 1;
-                    ws_mbar_arrive(ws_smem_u32(&s_acc_full[acc]));
+                    ws_mbar_arrive(hx_smem_u32(&s_acc_full[acc]));
                     break;
                 }
                 if (new_tile) {
 #ifdef L2_PROFILE
                     const long long c2 = clock64();
 #endif
-                    ws_mbar_wait(ws_smem_u32(&s_acc_empty[acc]), acc_ph[acc] ^ 1);
+                    hx_mbar_wait(hx_smem_u32(&s_acc_empty[acc]), acc_ph[acc] ^ 1);
 #ifdef L2_PROFILE
                     pa += clock64() - c2;
 #endif
@@ -553,11 +545,11 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
 #ifdef L2_PROFILE
                 pi_ += clock64() - c3; pm += n * ((m_flags & 1) != 0) + __popc(m_b1);
 #endif
-                l2_commit(ws_smem_u32(&s_empty[stage]));
+                l2_commit(hx_smem_u32(&s_empty[stage]));
                 if (m_flags & 4) {
                     s_tile[acc][0] = m_I; s_tile[acc][1] = m_q; s_tile[acc][2] = has; s_tile[acc][3] = 0;
                     asm volatile("fence.acq_rel.cta;" ::: "memory");
-                    l2_commit(ws_smem_u32(&s_acc_full[acc]));
+                    l2_commit(hx_smem_u32(&s_acc_full[acc]));
                     acc_ph[acc] ^= 1;
                     acc ^= 1;
                     new_tile = true;
@@ -571,7 +563,7 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
         uint32_t *const stg = staging + (size_t)ew * L2_STG_WORDS;
         unsigned acc = 0, acc_ph[2] = {0, 0};
         for (;;) {
-            ws_mbar_wait_sleep(ws_smem_u32(&s_acc_full[acc]), acc_ph[acc]);
+            ws_mbar_wait_sleep(hx_smem_u32(&s_acc_full[acc]), acc_ph[acc]);
             acc_ph[acc] ^= 1;
             l2_fence_after();
             if (s_tile[acc][3]) break;
@@ -579,7 +571,7 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
             l2_epilogue_tile<FUSED, FRESH>(tmem_base + acc * 256u, I, q, has, stg, lane, qd, hsel, cnt, g, crumbs);
             l2_fence_before();
             __syncwarp();
-            if (lane == 0) ws_mbar_arrive(ws_smem_u32(&s_acc_empty[acc]));
+            if (lane == 0) ws_mbar_arrive(hx_smem_u32(&s_acc_empty[acc]));
             acc ^= 1;
         }
     }
@@ -665,25 +657,25 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
     uint32_t rank;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
     const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-    const uint32_t stage0 = ws_smem_u32(l2_smem);
+    const uint32_t stage0 = hx_smem_u32(l2_smem);
     uint32_t *const staging = reinterpret_cast<uint32_t *>(l2_smem + (size_t)L2P_STAGES * L2P_STAGE_BYTES);
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < L2P_STAGES; ++s) {
-            ws_mbar_init(ws_smem_u32(&s_full[s]), 1);
-            ws_mbar_init(ws_smem_u32(&s_empty[s]), 1);
-            ws_mbar_init(ws_smem_u32(&s_peer_full[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_full[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_empty[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_peer_full[s]), 1);
         }
         for (int s = 0; s < 2; ++s) {
-            ws_mbar_init(ws_smem_u32(&s_acc_full[s]), 1);
-            ws_mbar_init(ws_smem_u32(&s_acc_empty_local[s]), L2_EP_WARPS);
-            ws_mbar_init(ws_smem_u32(&s_acc_empty_pair[s]), 2 * L2_EP_WARPS);
-            ws_mbar_init(ws_smem_u32(&s_tile_ready[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_acc_full[s]), 1);
+            hx_mbar_init(hx_smem_u32(&s_acc_empty_local[s]), L2_EP_WARPS);
+            hx_mbar_init(hx_smem_u32(&s_acc_empty_pair[s]), 2 * L2_EP_WARPS);
+            hx_mbar_init(hx_smem_u32(&s_tile_ready[s]), 1);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(ws_smem_u32(&s_tmem)),
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(hx_smem_u32(&s_tmem)),
                      "r"(512u)
                      : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
@@ -703,11 +695,11 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
         const int nq = g.nq;
         const int64_t n_tiles = (int64_t)((g.NB + 1) >> 1) * nq;
         const int SPB = g.SPB();
-        const uint32_t bar_full = ws_smem_u32(&s_full[warp]), bar_empty = ws_smem_u32(&s_empty[warp]);
+        const uint32_t bar_full = hx_smem_u32(&s_full[warp]), bar_empty = hx_smem_u32(&s_empty[warp]);
         const uint32_t dst0 = stage0 + (uint32_t)warp * L2P_STAGE_BYTES;
         int4 *const runs = s_runs[warp];
         int4 *const pend = s_pend[warp];                 // chunk: slab of its first block, nch, first block, reaches 2q+1
-        const uint32_t peer_full_at_leader = l2_mapa(ws_smem_u32(&s_peer_full[warp]), 0);
+        const uint32_t peer_full_at_leader = l2_mapa(hx_smem_u32(&s_peer_full[warp]), 0);
         unsigned ph = 0, gturn = 0;                      // phase of my stage; (stages sent so far by all warps) mod L2P_PW
         int n_pend = 0, p_Ip = 0, p_q = 0;
         auto emit = [&](int last) {                      // called by the stage's owner only
@@ -717,10 +709,10 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
                 const bool mine = slot < n_pend;
                 if (lane == 0) {
                     l2_wait_cluster(bar_empty, ph ^ 1);
-                    asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(ws_smem_u32(&s_meta[warp][0])), "r"(p_Ip),
+                    asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(hx_smem_u32(&s_meta[warp][0])), "r"(p_Ip),
                                  "r"(p_q | (n_pend << 20) | (last << 24))
                                  : "memory");
-                    l2_expect_tx(bar_full, 2 * L2_SLAB * (uint32_t)n_pend);
+                    hx_mbar_expect_tx(bar_full, 2 * L2_SLAB * (uint32_t)n_pend);
                 }
                 __syncwarp();
                 if (mine) {
@@ -730,7 +722,7 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
                     bool have = c.z <= blk;
                     if (rank == 1) have = have && (op == 0 ? (p_q > p_Ip || c.w) : (c.w != 0));
                     const uint8_t *src = have ? onehot + ((size_t)c.x + (size_t)(blk - c.z) * c.y) * L2_SLAB : zero_slabs;
-                    l2_bulk_g2s(dst0 + (uint32_t)(op * L2P_G + slot) * L2_SLAB, src, L2_SLAB, bar_full);
+                    hx_bulk_g2s(dst0 + (uint32_t)(op * L2P_G + slot) * L2_SLAB, src, L2_SLAB, bar_full);
                 }
                 // the second CTA tells the leader when its half of the stage has landed: each producer warp forwards its
                 // own stage (a remote arrive costs its issuer several hundred cycles - one forwarding thread for all
@@ -811,7 +803,7 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
         }
         if (gturn == (unsigned)warp && lane == 0) {                  // the warp whose turn it is tells warp L2P_PW to stop
             l2_wait_cluster(bar_empty, ph ^ 1);
-            asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(ws_smem_u32(&s_meta[warp][0])), "r"(0), "r"(8 << 24) : "memory");
+            asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(hx_smem_u32(&s_meta[warp][0])), "r"(0), "r"(8 << 24) : "memory");
             ws_mbar_arrive(bar_full);
         }
     } else if (warp == L2P_PW) {
@@ -819,7 +811,7 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
         if (lane == 0) {
             unsigned stage = 0, ph = 0, acc = 0, acc_ph[2] = {0, 0};
             bool new_tile = true, first = true;
-            const uint32_t acc_empty = ws_smem_u32(rank == 0 ? &s_acc_empty_pair[0] : &s_acc_empty_local[0]);
+            const uint32_t acc_empty = hx_smem_u32(rank == 0 ? &s_acc_empty_pair[0] : &s_acc_empty_local[0]);
 #ifdef L2_PROFILE
             unsigned long long pw = 0, pp = 0, pi_ = 0, pa = 0, pn = 0, pm = 0;
             const long long t_begin = clock64();
@@ -828,12 +820,12 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
 #ifdef L2_PROFILE
                 const long long c0 = clock64();
 #endif
-                l2_wait_cluster(ws_smem_u32(&s_full[stage]), ph);
+                l2_wait_cluster(hx_smem_u32(&s_full[stage]), ph);
 #ifdef L2_PROFILE
                 pw += clock64() - c0; pn++;
 #endif
                 int m_Ip, m_w;
-                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(m_Ip), "=r"(m_w) : "r"(ws_smem_u32(&s_meta[stage][0])) : "memory");
+                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(m_Ip), "=r"(m_w) : "r"(hx_smem_u32(&s_meta[stage][0])) : "memory");
                 const int m_q = m_w & 0xfffff, m_flags = m_w >> 24, n = (m_w >> 20) & 15;
                 if (m_flags & 8) {
 #ifdef L2_PROFILE
@@ -842,8 +834,8 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
 #endif
                     l2_wait_cluster(acc_empty + 8u * acc, acc_ph[acc] ^ 1);
                     s_tile[acc][3] = 1;
-                    ws_mbar_arrive(ws_smem_u32(&s_tile_ready[acc]));
-                    ws_mbar_arrive(ws_smem_u32(&s_acc_full[acc]));
+                    ws_mbar_arrive(hx_smem_u32(&s_tile_ready[acc]));
+                    ws_mbar_arrive(hx_smem_u32(&s_acc_full[acc]));
                     break;
                 }
                 if (new_tile) {
@@ -859,13 +851,13 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
                 }
                 if (m_flags & 1) {                                   // the tile's last stage: say which tile it was
                     s_tile[acc][0] = 2 * m_Ip + (int)rank; s_tile[acc][1] = m_q; s_tile[acc][2] = 3; s_tile[acc][3] = 0;
-                    ws_mbar_arrive(ws_smem_u32(&s_tile_ready[acc]));
+                    ws_mbar_arrive(hx_smem_u32(&s_tile_ready[acc]));
                 }
                 if (rank == 0) {
 #ifdef L2_PROFILE
                     const long long c3 = clock64();
 #endif
-                    l2_wait_cluster(ws_smem_u32(&s_peer_full[stage]), ph);
+                    l2_wait_cluster(hx_smem_u32(&s_peer_full[stage]), ph);
 #ifdef L2_PROFILE
                     const long long c4 = clock64(); pp += c4 - c3;
 #endif
@@ -881,8 +873,8 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
 #ifdef L2_PROFILE
                     pi_ += clock64() - c4; pm += n;
 #endif
-                    l2_commit2(ws_smem_u32(&s_empty[stage]));
-                    if (m_flags & 1) l2_commit2(ws_smem_u32(&s_acc_full[acc]));
+                    l2_commit2(hx_smem_u32(&s_empty[stage]));
+                    if (m_flags & 1) l2_commit2(hx_smem_u32(&s_acc_full[acc]));
                 }
                 if (m_flags & 1) {
                     acc_ph[acc] ^= 1;
@@ -896,11 +888,11 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
         // ============================== epilogue (each CTA drains its own 128 TMEM lanes) ======================
         const int ew = warp - (L2P_PW + 1), qd = warp & 3, hsel = ew >> 2;
         uint32_t *const stg = staging + (size_t)ew * L2_STG_WORDS;
-        const uint32_t pair_bar0 = l2_mapa(ws_smem_u32(&s_acc_empty_pair[0]), 0);
+        const uint32_t pair_bar0 = l2_mapa(hx_smem_u32(&s_acc_empty_pair[0]), 0);
         unsigned acc = 0, acc_ph[2] = {0, 0};
         for (;;) {
-            l2_wait_cluster(ws_smem_u32(&s_acc_full[acc]), acc_ph[acc]);
-            l2_wait_cluster(ws_smem_u32(&s_tile_ready[acc]), acc_ph[acc]);      // (warp L2P_PW has said which tile it is)
+            l2_wait_cluster(hx_smem_u32(&s_acc_full[acc]), acc_ph[acc]);
+            l2_wait_cluster(hx_smem_u32(&s_tile_ready[acc]), acc_ph[acc]);      // (warp L2P_PW has said which tile it is)
             acc_ph[acc] ^= 1;
             l2_fence_after();
             if (s_tile[acc][3]) break;
@@ -910,7 +902,7 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
             l2_fence_before();
             __syncwarp();
             if (lane == 0) {
-                ws_mbar_arrive(ws_smem_u32(&s_acc_empty_local[acc]));
+                ws_mbar_arrive(hx_smem_u32(&s_acc_empty_local[acc]));
                 l2_remote_arrive(pair_bar0 + 8u * acc);
             }
             acc ^= 1;

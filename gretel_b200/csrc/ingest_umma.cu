@@ -280,7 +280,7 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
     if (lo >= hi) return;
 
     const int rows = kmax + 1, cells = kmax - 1;
-    const uint32_t x_saddr = ws_smem_u32(um_smem);
+    const uint32_t x_saddr = hx_smem_u32(um_smem);
     uint4 *const tile = reinterpret_cast<uint4 *>(um_smem + (size_t)UM_EXP_WARPS * SLOTB);
     uint32_t *const tile32 = reinterpret_cast<uint32_t *>(tile);
 
@@ -288,12 +288,12 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
     if (threadIdx.x == 0) {
         s_runs_read = 0;
         for (int s = 0; s < UM_NACC; ++s) s_runkg[s] = 0;
-        for (int e = 0; e < UM_EXP_WARPS; ++e) ws_mbar_init(ws_smem_u32(&s_slot[e]), 1);
-        for (int s = 0; s < UM_NACC; ++s) ws_mbar_init(ws_smem_u32(&s_acc_full[s]), UM_ACC_COUNT);
+        for (int e = 0; e < UM_EXP_WARPS; ++e) hx_mbar_init(hx_smem_u32(&s_slot[e]), 1);
+        for (int s = 0; s < UM_NACC; ++s) hx_mbar_init(hx_smem_u32(&s_acc_full[s]), UM_ACC_COUNT);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(ws_smem_u32(&s_tmem)),
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(hx_smem_u32(&s_tmem)),
                      "r"((uint32_t)UM_TMEM_COLS)
                      : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -401,10 +401,10 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
         // slot's mbarrier (slot reusable) and to the run's accumulator barrier (run complete).
         const int e = warp - UM_RD_WARPS;
         const uint32_t slot_addr = x_saddr + (uint32_t)e * SLOTB;
-        const uint32_t slot_bar = ws_smem_u32(&s_slot[e]);
+        const uint32_t slot_bar = hx_smem_u32(&s_slot[e]);
         const uint64_t desc = um_desc(slot_addr, LBO);
         const uint32_t idesc0 = um_idesc(0);
-        const uint32_t accfull_addr = ws_smem_u32(&s_acc_full[0]);
+        const uint32_t accfull_addr = hx_smem_u32(&s_acc_full[0]);
         const uint32_t rowaddr = slot_addr + (uint32_t)(lane >> 3) * LBO + (uint32_t)(lane & 7) * 16u;
 #ifndef UM_PF_READS
 #define UM_PF_READS 2048
@@ -422,7 +422,7 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
             o = 0; o1 = 0;
             if (lane < (j.y & 0xff)) { const int64_t *p = off + lo + j.x + lane; o = p[0]; o1 = p[1]; }
         };
-        const uint32_t runs_addr = ws_smem_u32(&s_runs_read);
+        const uint32_t runs_addr = hx_smem_u32(&s_runs_read);
         int ji = e;
         int4 cur = get_job(ji);
         int64_t o, o1;
@@ -473,7 +473,7 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
                 const unsigned need = cur_ri - UM_NACC + 1;
                 while (um_ld_acquire(runs_addr) < need) __nanosleep(UM_GATE_NS);
             }
-            ws_mbar_wait(slot_bar, (njobs & 1) ^ 1);
+            hx_mbar_wait(slot_bar, (njobs & 1) ^ 1);
             um_fence_after();
             UM_T(tE);
             uint32_t rare_or, x0;
@@ -574,11 +574,11 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
             // the stage is complete after UM_ACC_COUNT arrivals: one per group (the expanders' commits) plus the rest here
             if (threadIdx.x == 0) {
                 const uint32_t ng = (uint32_t)((wk.n + 31) >> 5);
-                asm volatile("mbarrier.arrive.release.cta.shared::cta.b64 _, [%0], %1;" ::"r"(ws_smem_u32(&s_acc_full[s])),
+                asm volatile("mbarrier.arrive.release.cta.shared::cta.b64 _, [%0], %1;" ::"r"(hx_smem_u32(&s_acc_full[s])),
                              "r"(UM_ACC_COUNT - ng)
                              : "memory");
             }
-            ws_mbar_wait(ws_smem_u32(&s_acc_full[s]), (ri / UM_NACC) & 1);
+            hx_mbar_wait(hx_smem_u32(&s_acc_full[s]), (ri / UM_NACC) & 1);
             um_fence_after();
             UM_T(r2);
             const int kg = *reinterpret_cast<volatile int *>(&s_runkg[s]);
@@ -613,7 +613,7 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
             ws_pair_barrier(npt);                // tile adds and zeroing done
             if (threadIdx.x == 0) {
                 s_runkg[s] = 0;
-                asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(ws_smem_u32(&s_runs_read)), "r"(ri + 1) : "memory");
+                asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(hx_smem_u32(&s_runs_read)), "r"(ri + 1) : "memory");
             }
             UM_T(r3);
             UM_ACC(0, r1 - r0); UM_ACC(1, r2 - r1); UM_ACC(2, r3 - r2); UM_ACC(3, 1);

@@ -11,6 +11,7 @@
 // operation order as oracle/hansel_oracle.c, compiled with -fmad=false so that +,-,*,/
 // round exactly like the CPU; log10 and 10**x are evaluated exactly as glibc does (glibc_math.cuh).
 #include <limits.h>
+#include <stddef.h>
 #include <stdlib.h>
 #include <math.h>
 
@@ -41,13 +42,34 @@ __global__ void k_site_counts(const float *__restrict__ band, int N, int W,
     vseen[p] = v;
 }
 
+// ---- the lookback terms of Hansel.get_edge_weights_at ------------------------------------
+// log10((1 + H[a,s]) / (V + sum_a' H[a',s])) of one band cell, V valid symbols seen; 0.0 where the Laplace
+// denominator is 0, i.e. the term is dropped.
+__device__ __forceinline__ double lookback_term(const float *__restrict__ cell, unsigned a, int s, int v) {
+    double sup = 0.0;
+#pragma unroll
+    for (int a2 = 0; a2 < HX_NSYM; ++a2) sup += (double)cell[a2 * HX_NSYM + s];
+    const double den = (double)v + sup;
+    return den != 0 ? hx_gl_log10((1.0 + (double)cell[a * HX_NSYM + s]) / den) : 0.0;
+}
+
+// acc + the terms of lookbacks l = from, from + step, ... <= lmax beyond the band, in that order.  Their cells are
+// zero, so each term is log10(1 / V), dropped where V = 0.
+__device__ __forceinline__ double add_beyond_band(double acc, const int32_t *__restrict__ vseen, int flags, int snp,
+                                                  int from, int lmax, int step = 1) {
+    for (int l = from; l <= lmax; l += step) {
+        const int v = (flags & HX_F_VSITE_TO) ? vseen[snp] : vseen[snp - l];
+        if (v != 0) acc += hx_gl_log10(1.0 / (double)v);
+    }
+    return acc;
+}
+
 // ---- branch weights at one site (lanes 0..6 = candidate symbols) ----------------------
 // Returns this lane's unnormalised weight; *cand_mask gets the candidate set.
 __device__ __forceinline__ double edge_weight_lane(const float *__restrict__ band,
                                                    const double *__restrict__ scnt,
                                                    const int32_t *__restrict__ vseen, int W, int L,
-                                                   int flags, int snp, const uint8_t *hist,
-                                                   unsigned hist_mask, unsigned *cand_mask) {
+                                                   int flags, int snp, const uint8_t *hist, unsigned *cand_mask) {
     const int lane = threadIdx.x & 31;
     const int s = lane;
     double c = 0.0;
@@ -59,22 +81,13 @@ __device__ __forceinline__ double edge_weight_lane(const float *__restrict__ ban
     if (cand) {
         double lw = hx_gl_log10(c / total);
         const int lmax = L < snp ? L : snp;
+        const int lt = lmax < W ? lmax : W;
         const int v_to = vseen[snp];
-        for (int l = 1; l <= lmax; ++l) {
+        for (int l = 1; l <= lt; ++l) {
             const int pf = snp - l;
-            double obs = 0.0, sup = 0.0;
-            if (l <= W) {
-                const float *cell = band + hx_cell_off(W, pf, snp);
-                const unsigned a = hist[pf & hist_mask];
-                obs = (double)cell[a * HX_NSYM + s];
-#pragma unroll
-                for (int a2 = 0; a2 < HX_NSYM; ++a2) sup += (double)cell[a2 * HX_NSYM + s];
-            }
-            const int v = (flags & HX_F_VSITE_TO) ? v_to : vseen[pf];
-            const double den = (double)v + sup;
-            if (den != 0) lw += hx_gl_log10((1.0 + obs) / den);
+            lw += lookback_term(band + hx_cell_off(W, pf, snp), hist[pf], s, (flags & HX_F_VSITE_TO) ? v_to : vseen[pf]);
         }
-        ws = hx_gl_pow10(lw);
+        ws = hx_gl_pow10(add_beyond_band(lw, vseen, flags, snp, lt + 1, lmax));
     }
     *cand_mask = __ballot_sync(0xffffffffu, cand);
     return ws;
@@ -110,7 +123,7 @@ k_edge_one(const float *__restrict__ band, const double *__restrict__ scnt,
            const int32_t *__restrict__ vseen, int W, int L, int flags, int snp,
            const uint8_t *__restrict__ path, double *__restrict__ out /* [7] w, [7] total, [8] mask */) {
     unsigned cmask;
-    const double ws = edge_weight_lane(band, scnt, vseen, W, L, flags, snp, path, 0xffffffffu, &cmask);
+    const double ws = edge_weight_lane(band, scnt, vseen, W, L, flags, snp, path, &cmask);
     double wn, tw;
     (void)normalise_and_pick(ws, cmask, &wn, &tw);
     const int lane = threadIdx.x;
@@ -150,18 +163,11 @@ __global__ void k_walk_terms(const float *__restrict__ band, const int32_t *__re
         return;
     }
     const float *cell = band + hx_cell_off(W, pf, snp);
-    double obs[HX_NSYM], sup = 0.0;
-#pragma unroll
-    for (int a = 0; a < HX_NSYM; ++a) {
-        obs[a] = (double)cell[a * HX_NSYM + s];
-        sup += obs[a];
-    }
     const int v = (flags & HX_F_VSITE_TO) ? vseen[snp] : vseen[pf];
-    const double den = (double)v + sup;
     bool unsafe = false;
 #pragma unroll
     for (int a = 0; a < HX_NSYM; ++a) {
-        const double t = den != 0 ? hx_gl_log10((1.0 + obs[a]) / den) : 0.0;
+        const double t = lookback_term(cell, a, s, v);
         out[a * 8] = t;
         if (outq) {
             unsafe |= !(fabs(t) < 15.0);
@@ -194,95 +200,134 @@ __global__ void k_walk_logm(const double *__restrict__ scnt, int N, int flags, d
     if (guess) guess[snp] = (uint8_t)gsym;
 }
 
-// ---- TMA / mbarrier helpers (1-D bulk copies of the walk tables into shared memory) -------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t}" ::"r"(bar),
-        "r"(parity)
-        : "memory");
+// ---- staged walk tables ------------------------------------------------------------------------------------------
+// Three shared-memory buffers that TMA bulk copies fill with the walk tables of up to C consecutive sites each: first
+// the terms of all three buffers ([C][rows][7][8] T each), then their log-marginal rows ([C][8] T each); one mbarrier
+// per buffer.  Chunk k of a range holds sites first + kC, ...  A CTA may stage several ranges through the same buffers
+// (walk_q_range), so chunk k is the CTA's use number use0 + k: its buffer is that modulo 3, its phase that / 3, mod 2.
+template <class T>
+struct TableRing {
+    static constexpr uint32_t ROW = 8 * sizeof(T);          // bytes of one log-marginal row
+    const T *terms, *logm;                                   // global tables: rows*56 and 8 T per site
+    uint32_t sm, bars;                                       // shared addresses of buffer 0 and mbarrier 0
+    uint32_t site_bytes, chunk_bytes;                        // terms of one site, of one buffer
+    int rows, C, first, last, nchunks;
+    uint32_t use0;
+
+    // lane 0, once per CTA before any use
+    __device__ static void init(unsigned long long *bars) {
+        for (int b = 0; b < 3; ++b) hx_mbar_init(hx_smem_u32(&bars[b]), 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __device__ TableRing(const T *terms_, const T *logm_, int rows_, int C_, int first_, int last_, void *smem,
+                         unsigned long long *bars_, uint32_t use0_)
+        : terms(terms_), logm(logm_), sm(hx_smem_u32(smem)), bars(hx_smem_u32(bars_)),
+          site_bytes((uint32_t)rows_ * 56u * (uint32_t)sizeof(T)), chunk_bytes((uint32_t)C_ * site_bytes), rows(rows_),
+          C(C_), first(first_), last(last_), nchunks((last_ - first_ + 1 + C_ - 1) / C_), use0(use0_) {}
+    __device__ int buf(int k) const { return (int)((use0 + (uint32_t)k) % 3u); }
+    __device__ uint32_t terms_at(int k) const { return sm + (uint32_t)buf(k) * chunk_bytes; }
+    __device__ uint32_t logm_at(int k) const { return sm + 3u * chunk_bytes + (uint32_t)buf(k) * C * ROW; }
+    // lane 0: stage chunk k into its buffer (nothing past the last chunk)
+    __device__ void issue(int k) const {
+        if (k >= nchunks) return;
+        const int s0 = first + k * C;
+        const int ns = min(C, last - s0 + 1);
+        const uint32_t bar = bars + 8u * (uint32_t)buf(k);
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier reads of this buffer are done
+        hx_mbar_expect_tx(bar, (uint32_t)ns * (site_bytes + ROW));
+        hx_bulk_g2s(terms_at(k), terms + (int64_t)s0 * rows * 56, (uint32_t)ns * site_bytes, bar);
+        hx_bulk_g2s(logm_at(k), logm + (int64_t)s0 * 8, (uint32_t)ns * ROW, bar);
+    }
+    __device__ void wait(int k) const {
+        hx_mbar_wait(bars + 8u * (uint32_t)buf(k), ((use0 + (uint32_t)k) / 3u) & 1u);
+    }
+    // before a CTA leaves early at chunk k: the copies still in flight must land before its shared memory is released
+    __device__ void drain_after(int k) const {
+        for (int k2 = k + 1; k2 <= k + 2 && k2 < nchunks; ++k2) wait(k2);
+    }
+};
+
+// The pick at one site of the float64 walks: lane = candidate symbol, every lane of the warp calls it.  `lwf` is the
+// lane's log weight summed in any order.  The reference's ordered sum, 10**x and normalisation
+// (Hansel.get_edge_weights_at) only matter for the argmax when two candidates are within rounding of each other, so
+// they are evaluated only then (and whenever 10**x could under/overflow); otherwise the largest log weight wins
+// outright.  The exact evaluation reads the log-marginal row `lmrow`, the site's terms `tab` ([lt][7][8]) and the
+// chosen symbols in `ring`.  CAND_ONLY keeps the other lanes out of it: faster where `tab` is in global memory
+// (k_walk_wide), slower where it is in shared memory (k_walk_tables), measured on a B200.  Returns the symbol, or -1
+// for a site without a candidate (gretel.py:176-180).
+template <bool CAND_ONLY>
+__device__ __forceinline__ int pick_site(double lwf, unsigned cmask, const double *lmrow, const double *tab,
+                                         const uint8_t *ring, int snp, int lt, int lmax,
+                                         const int32_t *__restrict__ vseen, int flags) {
+    const int lane = threadIdx.x & 31;
+    const bool cand = lane < HX_NSYM && ((cmask >> lane) & 1u);
+    // best log weight over the 7 candidate lanes (butterfly), then who is within 1e-6 of it
+    const double key = cand ? lwf : -INFINITY;
+    double best = key;
+#pragma unroll
+    for (int o = 4; o > 0; o >>= 1) best = fmax(best, __shfl_xor_sync(0xffffffffu, best, o));
+    best = __shfl_sync(0xffffffffu, best, 0);    // lanes 8..31 hold -inf: make the branch below warp-uniform
+    const unsigned near = __ballot_sync(0xffffffffu, cand && key >= best - 1e-6);
+    if (cmask == 0) return -1;
+    if (__popc(near) == 1 && best > -300.0 && best < 300.0) return __ffs(near) - 1;   // a clear winner
+    // exact evaluation in the reference's order: ((log10 P(s) + t1) + t2) + ...
+    const int s = CAND_ONLY || lane < HX_NSYM ? lane : 0;     // lanes 7..31 repeat symbol 0's sums, which are not used
+    double lw = 0.0;
+    if (!CAND_ONLY || cand) {
+        lw = lmrow[s];
+        for (int l = 1; l <= lt; ++l) lw += tab[((l - 1) * HX_NSYM + ring[(snp - l) & (HX_RING - 1)]) * 8 + s];
+        lw = add_beyond_band(lw, vseen, flags, snp, lt + 1, lmax);
+    }
+    const double ws = cand ? hx_gl_pow10(lw) : 0.0;
+    double wn, tw;
+    return normalise_and_pick(ws, cmask, &wn, &tw);
 }
 
 // The walk over the precomputed tables: one warp, lanes 0..6 = candidate symbols, strictly
-// sequential over sites.  The tables of the next sites are staged into shared memory by TMA
-// bulk copies (three chunks of C sites in flight, one mbarrier each), so the dependent chain
-// per site is: previous choice -> one shared-memory load -> one add -> 7-way argmax.
-// The reference's ordered sum, 10**x and normalisation (Hansel.get_edge_weights_at) only
-// matter for the argmax when two candidates are within rounding of each other, so they are
-// evaluated only then (and whenever 10**x could under/overflow); otherwise the largest
-// log-weight wins outright.
+// sequential over sites.  The tables of the next sites are staged into shared memory (TableRing, three chunks of C
+// sites in flight), so the dependent chain per site is: previous choice -> one shared-memory load -> one add ->
+// 7-way argmax (pick_site).
 __global__ void __launch_bounds__(32)
 k_walk_tables(const double *__restrict__ terms, const double *__restrict__ logm,
               const int32_t *__restrict__ vseen, int N, int L, int Lw, int flags, int C,
-              uint8_t *__restrict__ path, int *__restrict__ flagsd) {
+              uint8_t *__restrict__ path, hx_dev_flags *__restrict__ df) {
     extern __shared__ __align__(128) unsigned char smraw[];
     __shared__ __align__(8) unsigned long long bars[3];
     __shared__ uint8_t ring[HX_RING];
     const int lane = threadIdx.x;
     const int s = lane < HX_NSYM ? lane : 0;
-    if (flagsd[1]) return;
-    const uint32_t site_t_bytes = (uint32_t)Lw * 448u;                 // terms of one site
-    const uint32_t chunk_t_bytes = (uint32_t)C * site_t_bytes;
-    double *const sm_terms = reinterpret_cast<double *>(smraw);                        // [3][C][Lw][7][8]
-    double *const sm_logm = reinterpret_cast<double *>(smraw + 3 * (size_t)chunk_t_bytes);   // [3][C][8]
-    const int nchunks = (N + C - 1) / C;
+    if (df->hole) return;
+    const TableRing<double> tr(terms, logm, Lw, C, 1, N, smraw, bars, 0);
+    const double *const sm_terms = reinterpret_cast<const double *>(smraw);                        // [3][C][Lw][7][8]
+    const double *const sm_logm = sm_terms + 3 * (size_t)(tr.chunk_bytes / 8);                      // [3][C][8]
     if (lane == 0) {
         ring[0] = HX_SYM_GAP;
         path[0] = HX_SYM_GAP;
-        for (int b = 0; b < 3; ++b) mbar_init(smem_u32(&bars[b]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        TableRing<double>::init(bars);
     }
     __syncwarp();
-    auto issue = [&](int k) {        // lane 0: stage chunk k (sites 1+kC ..) into buffer k%3
-        if (k >= nchunks) return;
-        const int b = k % 3;
-        const int first = 1 + k * C;
-        const int ns = min(C, N - first + 1);
-        const uint32_t bar = smem_u32(&bars[b]);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier reads of this buffer are done
-        mbar_expect_tx(bar, (uint32_t)ns * (site_t_bytes + 64u));
-        bulk_g2s(smem_u32(sm_terms) + (uint32_t)b * chunk_t_bytes, terms + (int64_t)first * Lw * 56,
-                 (uint32_t)ns * site_t_bytes, bar);
-        bulk_g2s(smem_u32(sm_logm) + (uint32_t)b * C * 64u, logm + (int64_t)first * 8, (uint32_t)ns * 64u, bar);
-    };
-    if (lane == 0) { issue(0); issue(1); }
+    if (lane == 0) { tr.issue(0); tr.issue(1); }
     unsigned last = HX_SYM_GAP;
     unsigned long long hist = HX_SYM_GAP;               // 4 bits per chosen symbol, newest in bits 0..3
-    for (int k = 0; k < nchunks; ++k) {
+    for (int k = 0; k < tr.nchunks; ++k) {
         __syncwarp();
-        if (lane == 0) issue(k + 2);
-        mbar_wait(smem_u32(&bars[k % 3]), (uint32_t)((k / 3) & 1));
+        if (lane == 0) tr.issue(k + 2);
+        tr.wait(k);
         const int first = 1 + k * C;
         const int ns = min(C, N - first + 1);
-        const double *ct = sm_terms + (size_t)(k % 3) * (chunk_t_bytes / 8);
-        const double *cl = sm_logm + (size_t)(k % 3) * C * 8;
+        const double *ct = sm_terms + (size_t)tr.buf(k) * (tr.chunk_bytes / 8);
+        const double *cl = sm_logm + (size_t)tr.buf(k) * C * 8;
         for (int j = 0; j < ns; ++j) {
             const int snp = first + j;
-            const double *base = ct + (size_t)j * Lw * 56 + s;
+            const double *tab = ct + (size_t)j * Lw * 56;
+            const double *base = tab + s;
             const double lm = cl[j * 8 + s];
             const unsigned cmask = (unsigned)cl[j * 8 + 7];
-            const bool cand = lane < HX_NSYM && ((cmask >> lane) & 1u);
             const int lmax = L < snp ? L : snp;
             const int lt = lmax < Lw ? lmax : Lw;
             // the only load that depends on the previous choice
             const double v1 = lt >= 1 ? base[last * 8] : 0.0;
-            // everything else, in any order (two accumulators); exactness is restored below if needed
+            // everything else, in any order (two accumulators); pick_site restores exactness if needed
             double p0 = lm, p1 = 0.0;
             {
                 const int n16 = lt < 16 ? lt : 16;
@@ -300,44 +345,11 @@ k_walk_tables(const double *__restrict__ terms, const double *__restrict__ logm,
                     if (l & 1) p1 += v; else p0 += v;
                 }
             }
-            double tail = 0.0;                           // lookback beyond the band: cells are zero
-            for (int l = lt + 1; l <= lmax; ++l) {
-                const int v = (flags & HX_F_VSITE_TO) ? vseen[snp] : vseen[snp - l];
-                if (v != 0) tail += hx_gl_log10(1.0 / (double)v);
-            }
-            const double lwf = (p0 + p1) + tail + v1;
-            // best log-weight over the 7 candidate lanes (butterfly), then who is within 1e-6 of it
-            const double key = cand ? lwf : -INFINITY;
-            double best = key;
-#pragma unroll
-            for (int o = 4; o > 0; o >>= 1) best = fmax(best, __shfl_xor_sync(0xffffffffu, best, o));
-            best = __shfl_sync(0xffffffffu, best, 0);    // lanes 8..31 hold -inf: make the branch below warp-uniform
-            const unsigned near = __ballot_sync(0xffffffffu, cand && key >= best - 1e-6);
-            int next;
-            if (cmask == 0) {
-                next = -1;
-            } else if (__popc(near) == 1 && best > -300.0 && best < 300.0) {
-                next = __ffs(near) - 1;                  // a clear winner: no other candidate within rounding
-            } else {
-                // exact evaluation in the reference's order: ((log10 P(s) + t1) + t2) + ...
-                double lw = lm;
-                for (int l = 1; l <= lt; ++l) {
-                    const unsigned a = l == 1 ? last : (unsigned)ring[(snp - l) & (HX_RING - 1)];
-                    lw += base[((l - 1) * HX_NSYM + a) * 8];
-                }
-                for (int l = lt + 1; l <= lmax; ++l) {
-                    const int v = (flags & HX_F_VSITE_TO) ? vseen[snp] : vseen[snp - l];
-                    if (v != 0) lw += hx_gl_log10(1.0 / (double)v);
-                }
-                const double ws = cand ? hx_gl_pow10(lw) : 0.0;
-                double wn, tw;
-                next = normalise_and_pick(ws, cmask, &wn, &tw);
-            }
+            const double lwf = (p0 + p1) + add_beyond_band(0.0, vseen, flags, snp, lt + 1, lmax) + v1;
+            const int next = pick_site<false>(lwf, cmask, cl + j * 8, tab, ring, snp, lt, lmax, vseen, flags);
             if (next < 0) {                              // gretel.py:176-180
-                if (lane == 0) { flagsd[0] = snp; flagsd[1] = 1; }
-                // let the bulk copies already in flight land before this CTA's shared memory is released
-                for (int k2 = k + 1; k2 <= k + 2 && k2 < nchunks; ++k2)
-                    mbar_wait(smem_u32(&bars[k2 % 3]), (uint32_t)((k2 / 3) & 1));
+                if (lane == 0) { df->hole_site = snp; df->hole = 1; }
+                tr.drain_after(k);
                 return;
             }
             last = (unsigned)next;
@@ -346,7 +358,7 @@ k_walk_tables(const double *__restrict__ terms, const double *__restrict__ logm,
             __syncwarp();
         }
     }
-    if (lane == 0) flagsd[0] = 0;
+    if (lane == 0) df->hole_site = 0;
 }
 
 __device__ __forceinline__ int lds32(uint32_t addr) {
@@ -366,29 +378,10 @@ __device__ __forceinline__ int walk_q_range(const int32_t *__restrict__ termsq, 
     constexpr int Lq = 4 * NIT + 1;
     constexpr uint32_t site_t_bytes = (uint32_t)Lq * 224u;             // int32 terms of one site
     const int lane = threadIdx.x & 31;
-    const uint32_t chunk_t_bytes = (uint32_t)C * site_t_bytes;
-    const uint32_t sm_terms = smem_u32(smraw);                                   // [3][C][Lq][7][8] int32
-    const uint32_t sm_logm = sm_terms + 3u * chunk_t_bytes;                      // [3][C][8] int32
-    const int n_sites = s_end - s_begin + 1;
-    const int nchunks = (n_sites + C - 1) / C;
-    // the three mbarriers are reused by consecutive ranges of one CTA: a buffer's phase is counted over all uses
-    const uint32_t use0 = bar_uses;
-    auto parity_of = [&](int k) { return (uint32_t)(((use0 + (uint32_t)k) / 3u) & 1u); };
-    auto buf_of = [&](int k) { return (int)((use0 + (uint32_t)k) % 3u); };
-    auto issue = [&](int k) {
-        if (k >= nchunks) return;
-        const int b = buf_of(k);
-        const int first = s_begin + k * C;
-        const int ns = min(C, s_end - first + 1);
-        const uint32_t bar = smem_u32(&bars[b]);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_expect_tx(bar, (uint32_t)ns * (site_t_bytes + 32u));
-        bulk_g2s(sm_terms + (uint32_t)b * chunk_t_bytes, termsq + (int64_t)first * Lq * 56,
-                 (uint32_t)ns * site_t_bytes, bar);
-        bulk_g2s(sm_logm + (uint32_t)b * C * 32u, logmq + (int64_t)first * 8, (uint32_t)ns * 32u, bar);
-    };
+    const TableRing<int32_t> tr(termsq, logmq, Lq, C, s_begin, s_end, smraw, bars, bar_uses);
+    const int nchunks = tr.nchunks;
     __syncwarp();
-    if (lane == 0) { issue(0); issue(1); }
+    if (lane == 0) { tr.issue(0); tr.issue(1); }
     bar_uses += (uint32_t)nchunks;
     const uint32_t q4 = 4u * (uint32_t)(lane & 7);
     const uint32_t g = (uint32_t)lane >> 3;
@@ -410,18 +403,18 @@ __device__ __forceinline__ int walk_q_range(const int32_t *__restrict__ termsq, 
     unsigned mine = 0;                                      // lane's slot of the 32-site output block
     const int margin_q = 168;                               // 1.6e-4 * 2^20
     const int floor_q = -300 * 1048576;                     // 10**x must stay representable
-    mbar_wait(smem_u32(&bars[buf_of(0)]), parity_of(0));
+    tr.wait(0);
     // lookback >= 2 terms of the first site (rows past the start of the region are zero), then its log marginal
     int R;
     {
-        const uint32_t site0 = sm_terms + (uint32_t)buf_of(0) * chunk_t_bytes;
+        const uint32_t site0 = tr.terms_at(0);
         int acc = 0;
 #pragma unroll
         for (int t = 0; t < NIT; ++t)
             acc += lds32(site0 + look_off + (uint32_t)t * 896u + __byte_perm(h[t], 0u, psel));
         acc += __shfl_xor_sync(0xffffffffu, acc, 8);
         acc += __shfl_xor_sync(0xffffffffu, acc, 16);
-        R = acc + lds32(sm_logm + (uint32_t)buf_of(0) * C * 32u + q4);
+        R = acc + lds32(tr.logm_at(0) + q4);
     }
     // ... and the history relative to s_begin: shift in the symbol at s_begin - 1
     uint32_t prev32 = (uint32_t)hsrc[s_begin - 1] << 5;
@@ -430,14 +423,14 @@ __device__ __forceinline__ int walk_q_range(const int32_t *__restrict__ termsq, 
     h[0] = (h[0] << 8) | prev32;
     for (int k = 0; k < nchunks; ++k) {
         __syncwarp();
-        if (lane == 0) issue(k + 2);
-        if (k + 1 < nchunks) mbar_wait(smem_u32(&bars[buf_of(k + 1)]), parity_of(k + 1));
+        if (lane == 0) tr.issue(k + 2);
+        if (k + 1 < nchunks) tr.wait(k + 1);
         const int first = s_begin + k * C;
         const int ns = min(C, s_end - first + 1);
-        const uint32_t ct_n = sm_terms + (uint32_t)buf_of(k + 1) * chunk_t_bytes;
-        const uint32_t cl_n = sm_logm + (uint32_t)buf_of(k + 1) * C * 32u;
-        uint32_t csite = sm_terms + (uint32_t)buf_of(k) * chunk_t_bytes;     // current site's table
-        uint32_t clm = sm_logm + (uint32_t)buf_of(k) * C * 32u;
+        const uint32_t ct_n = tr.terms_at(k + 1);
+        const uint32_t cl_n = tr.logm_at(k + 1);
+        uint32_t csite = tr.terms_at(k);                 // current site's table
+        uint32_t clm = tr.logm_at(k);
         for (int j = 0; j < ns; ++j) {
             const int snp = first + j;
             // ---- look ahead: lookback >= 2 terms of site snp+1 (independent of this site's choice).  After the
@@ -479,8 +472,7 @@ __device__ __forceinline__ int walk_q_range(const int32_t *__restrict__ termsq, 
                     next = normalise_and_pick(ws, cmask, &wn, &tw);
                 }
                 if (next < 0) {                          // gretel.py:176-180
-                    for (int k2 = k + 1; k2 <= k + 2 && k2 < nchunks; ++k2)
-                        mbar_wait(smem_u32(&bars[buf_of(k2)]), parity_of(k2));
+                    tr.drain_after(k);
                     return snp;
                 }
             }
@@ -555,16 +547,13 @@ __global__ void __launch_bounds__(32)
 k_walk_q(const int32_t *__restrict__ termsq, const int32_t *__restrict__ logmq, const double *__restrict__ terms,
          const double *__restrict__ logm, int N, int L, int C, int blk_len, int warm, const uint8_t *__restrict__ guess,
          const uint8_t *paths0, const int *__restrict__ cand_idx, uint8_t *spec, int spec_stride, int *__restrict__ spec_ok,
-         uint8_t *path, int *__restrict__ flagsd) {
+         uint8_t *path, hx_dev_flags *__restrict__ df) {
     extern __shared__ __align__(128) unsigned char smraw[];
     __shared__ __align__(8) unsigned long long bars[3];
     const int lane = threadIdx.x;
-    if (flagsd[1]) return;
-    const bool force_exact = flagsd[2] != 0;
-    if (lane == 0) {
-        for (int b = 0; b < 3; ++b) mbar_init(smem_u32(&bars[b]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    if (df->hole) return;
+    const bool force_exact = df->q_unsafe != 0;
+    if (lane == 0) TableRing<int32_t>::init(bars);
     __syncwarp();
     uint32_t bar_uses = 0;
     if (blockIdx.x == 0) {                                  // block 0 of the region: the walk proper
@@ -573,8 +562,8 @@ k_walk_q(const int32_t *__restrict__ termsq, const int32_t *__restrict__ logmq, 
         __syncwarp();
         const int hole = walk_q_range<NIT>(termsq, logmq, terms, logm, L, C, 1, end, path, path + 1, force_exact, smraw,
                                            bars, bar_uses);
-        if (hole && lane == 0) { flagsd[0] = hole; flagsd[1] = 1; }
-        if (!hole && lane == 0 && end == N) flagsd[0] = 0;
+        if (hole && lane == 0) { df->hole_site = hole; df->hole = 1; }
+        if (!hole && lane == 0 && end == N) df->hole_site = 0;
         return;
     }
     // speculative walks: CTA 1 + (b-1)*CAND + c = block b >= 1 from candidate history c
@@ -605,16 +594,13 @@ __global__ void __launch_bounds__(32)
 k_walk_fix(const int32_t *__restrict__ termsq, const int32_t *__restrict__ logmq, const double *__restrict__ terms,
            const double *__restrict__ logm, int N, int L, int C, int blk_len, int warm, int n_blocks,
            const uint8_t *paths0, const int *__restrict__ cand_idx, const uint8_t *__restrict__ spec, int spec_stride,
-           const int *__restrict__ spec_ok, uint8_t *path, int *__restrict__ flagsd) {
+           const int *__restrict__ spec_ok, uint8_t *path, hx_dev_flags *__restrict__ df) {
     extern __shared__ __align__(128) unsigned char smraw[];
     __shared__ __align__(8) unsigned long long bars[3];
     const int lane = threadIdx.x;
-    if (flagsd[1]) return;
-    const bool force_exact = flagsd[2] != 0;
-    if (lane == 0) {
-        for (int b = 0; b < 3; ++b) mbar_init(smem_u32(&bars[b]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    if (df->hole) return;
+    const bool force_exact = df->q_unsafe != 0;
+    if (lane == 0) TableRing<int32_t>::init(bars);
     __syncwarp();
     uint32_t bar_uses = 0;
     int redone = 0;                                          // sites walked again
@@ -659,7 +645,7 @@ k_walk_fix(const int32_t *__restrict__ termsq, const int32_t *__restrict__ logmq
             const int hole = walk_q_range<NIT>(termsq, logmq, terms, logm, L, C, sub, e, path, path + sub, force_exact,
                                                smraw, bars, bar_uses);
             if (hole) {
-                if (lane == 0) { flagsd[0] = hole; flagsd[1] = 1; }
+                if (lane == 0) { df->hole_site = hole; df->hole = 1; }
                 return;
             }
             redone += e - sub + 1;
@@ -683,22 +669,21 @@ k_walk_fix(const int32_t *__restrict__ termsq, const int32_t *__restrict__ logmq
             }
         }
     }
-    if (lane == 0) { flagsd[0] = 0; flagsd[3] += redone; }
+    if (lane == 0) { df->hole_site = 0; df->walk_redone += redone; }
 }
 
 // Wide-lookback walk (L*448 B per site does not fit the staged pipeline, e.g. ONT L ~ 300):
 // one warp per candidate symbol, lanes split the lookbacks and combine with warp shuffles;
-// warp 0 then takes the 7-way argmax.  As in k_walk_tables the reordered sum only picks a clear
-// winner; near-ties are re-evaluated in the reference's order by one lane per candidate.
+// warp 0 then takes the 7-way argmax (pick_site, as in k_walk_tables).
 __global__ void __launch_bounds__(256)
 k_walk_wide(const double *__restrict__ terms, const double *__restrict__ logm,
             const int32_t *__restrict__ vseen, int N, int L, int Lw, int flags,
-            uint8_t *__restrict__ path, int *__restrict__ flagsd) {
+            uint8_t *__restrict__ path, hx_dev_flags *__restrict__ df) {
     __shared__ uint8_t ring[HX_RING];
     __shared__ double s_lw[8];
     __shared__ int s_next;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;   // warp = candidate symbol (7 = idle helper)
-    if (flagsd[1]) return;
+    if (df->hole) return;
     if (threadIdx.x == 0) { ring[0] = HX_SYM_GAP; path[0] = HX_SYM_GAP; }
     __syncthreads();
     for (int snp = 1; snp <= N; ++snp) {
@@ -712,10 +697,7 @@ k_walk_wide(const double *__restrict__ terms, const double *__restrict__ logm,
             double p = 0.0;
             for (int l = 1 + lane; l <= lt; l += 32)
                 p += base[((l - 1) * HX_NSYM + ring[(snp - l) & (HX_RING - 1)]) * 8];
-            for (int l = lt + 1 + lane; l <= lmax; l += 32) {       // beyond the band: cells are zero
-                const int v = (flags & HX_F_VSITE_TO) ? vseen[snp] : vseen[snp - l];
-                if (v != 0) p += hx_gl_log10(1.0 / (double)v);
-            }
+            p = add_beyond_band(p, vseen, flags, snp, lt + 1 + lane, lmax, 32);
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) p += __shfl_xor_sync(0xffffffffu, p, o);
             if (lane == 0) s_lw[warp] = lmrow[warp] + p;
@@ -724,35 +706,8 @@ k_walk_wide(const double *__restrict__ terms, const double *__restrict__ logm,
         }
         __syncthreads();
         if (warp == 0) {
-            const double key = lane < HX_NSYM ? s_lw[lane] : -INFINITY;
-            double best = key;
-#pragma unroll
-            for (int o = 4; o > 0; o >>= 1) best = fmax(best, __shfl_xor_sync(0xffffffffu, best, o));
-            best = __shfl_sync(0xffffffffu, best, 0);
-            const bool lcand = lane < HX_NSYM && ((cmask >> lane) & 1u);
-            const unsigned near = __ballot_sync(0xffffffffu, lcand && key >= best - 1e-6);
-            int next;
-            if (cmask == 0) {
-                next = -1;
-            } else if (__popc(near) == 1 && best > -300.0 && best < 300.0) {
-                next = __ffs(near) - 1;
-            } else {
-                // exact evaluation in the reference's order, one lane per candidate
-                double lw = 0.0;
-                if (lcand) {
-                    const double *base = terms + ((int64_t)snp * Lw) * 56 + lane;
-                    lw = lmrow[lane];
-                    for (int l = 1; l <= lt; ++l)
-                        lw += base[((l - 1) * HX_NSYM + ring[(snp - l) & (HX_RING - 1)]) * 8];
-                    for (int l = lt + 1; l <= lmax; ++l) {
-                        const int v = (flags & HX_F_VSITE_TO) ? vseen[snp] : vseen[snp - l];
-                        if (v != 0) lw += hx_gl_log10(1.0 / (double)v);
-                    }
-                }
-                const double ws = lcand ? hx_gl_pow10(lw) : 0.0;
-                double wn, tw;
-                next = normalise_and_pick(ws, cmask, &wn, &tw);
-            }
+            const int next = pick_site<true>(s_lw[lane & 7], cmask, lmrow, terms + ((int64_t)snp * Lw) * 56, ring, snp, lt,
+                                             lmax, vseen, flags);
             if (lane == 0) {
                 s_next = next;
                 if (next >= 0) { ring[snp & (HX_RING - 1)] = (uint8_t)next; path[snp] = (uint8_t)next; }
@@ -760,19 +715,19 @@ k_walk_wide(const double *__restrict__ terms, const double *__restrict__ logm,
         }
         __syncthreads();
         if (s_next < 0) {                                  // gretel.py:176-180
-            if (threadIdx.x == 0) { flagsd[0] = snp; flagsd[1] = 1; }
+            if (threadIdx.x == 0) { df->hole_site = snp; df->hole = 1; }
             return;
         }
     }
-    if (threadIdx.x == 0) flagsd[0] = 0;
+    if (threadIdx.x == 0) df->hole_site = 0;
 }
 
 // ---- per-site marginals of the chosen path, then ordered sums -------------------------
 __global__ void k_path_stats(const double *__restrict__ scnt_cur, const double *__restrict__ scnt_orig,
                              int N, const uint8_t *__restrict__ path, double *__restrict__ site,
-                             const int *__restrict__ flagsd) {
+                             const hx_dev_flags *__restrict__ df) {
     const int snp = blockIdx.x * blockDim.x + threadIdx.x + 1;
-    if (flagsd[1] || snp > N) return;
+    if (df->hole || snp > N) return;
     const int s = path[snp];
     const double m = scnt_cur[(int64_t)snp * 8 + s] / scnt_cur[(int64_t)snp * 8 + 7];
     const double to = scnt_orig[(int64_t)snp * 8 + 7];
@@ -787,10 +742,10 @@ __global__ void k_path_stats(const double *__restrict__ scnt_cur, const double *
 // reduction on the main stream.  The two log10 sums are only reported; they are strictly ordered chains (same order
 // as gretel.py:185-186) and run on a side stream while the reweighting and the next haplotype's tables proceed.
 __global__ void __launch_bounds__(1024)
-k_path_min(const double *__restrict__ site, int N, double min_remove, double *__restrict__ stats,
-           const int *__restrict__ flagsd) {
+k_path_min(const double *__restrict__ site, int N, double min_remove, hx_hap_stats *__restrict__ stats,
+           const hx_dev_flags *__restrict__ df) {
     __shared__ double sh[32];
-    if (flagsd[1]) { if (threadIdx.x == 0) stats[5] = 0.0; return; }
+    if (df->hole) { if (threadIdx.x == 0) stats->done = 0.0; return; }
     const double *m = site + 2 * ((int64_t)N + 2);
     double acc = INFINITY;
     for (int x = 1 + threadIdx.x; x <= N; x += 1024) { const double v = m[x]; acc = v < acc ? v : acc; }
@@ -800,9 +755,9 @@ k_path_min(const double *__restrict__ site, int N, double min_remove, double *__
     __syncthreads();
     if (threadIdx.x == 0) {
         for (int w = 1; w < 32; ++w) acc = sh[w] < acc ? sh[w] : acc;
-        stats[2] = acc;                                        // min marginal
-        stats[3] = acc < min_remove ? min_remove : acc;        // cmd.py:157-160
-        stats[5] = 1.0;                                        // iteration completed
+        stats->min_marginal = acc;
+        stats->ratio = acc < min_remove ? min_remove : acc;    // cmd.py:157-160
+        stats->done = 1.0;
     }
 }
 
@@ -811,10 +766,10 @@ k_path_min(const double *__restrict__ site, int N, double min_remove, double *__
 constexpr int HX_SUM_CH = 896;
 
 __global__ void __launch_bounds__(256)
-k_path_sum(const double *__restrict__ site, int N, double *__restrict__ stats) {
+k_path_sum(const double *__restrict__ site, int N, hx_hap_stats *__restrict__ stats) {
     __shared__ double buf[2][2][HX_SUM_CH];
     const int tid = threadIdx.x;
-    if (stats[5] != 1.0) return;                               // the walk found a hole (k_path_min): nothing to sum
+    if (stats->done != 1.0) return;                            // the walk found a hole (k_path_min): nothing to sum
     const int64_t stride = (int64_t)N + 2;
     const int nch = (N + HX_SUM_CH - 1) / HX_SUM_CH;
     auto stage = [&](int c, int t0, int nt) {
@@ -845,7 +800,8 @@ k_path_sum(const double *__restrict__ site, int N, double *__restrict__ stats) {
         }
         __syncthreads();
     }
-    if (role >= 0) stats[role] = acc;                          // hp_current, hp_original
+    if (role == 0) stats->hp_current = acc;
+    if (role == 1) stats->hp_original = acc;
 }
 
 // ---- reweight ---------------------------------------------------------------------------
@@ -857,10 +813,10 @@ template <int BLOCK>
 __global__ void __launch_bounds__(BLOCK)
 k_reweight_path(float *__restrict__ band, int N, int W, const uint8_t *__restrict__ path,
                 const double *__restrict__ ratio_ptr, double ratio_val,
-                double *__restrict__ partials, const int *__restrict__ flagsd) {
+                double *__restrict__ partials, const hx_dev_flags *__restrict__ df) {
     __shared__ double sh[BLOCK / 32];
     double removed = 0.0;
-    const bool dead = flagsd[1] != 0;
+    const bool dead = df->hole != 0;
     const int64_t idx = (int64_t)blockIdx.x * BLOCK + threadIdx.x;
     const int64_t pj = 1 + idx / W;
     const int d = 1 + (int)(idx % W);
@@ -934,38 +890,67 @@ int launch_reweight(hx_matrix *h, const uint8_t *d_path, const double *d_ratio, 
     return HX_OK;
 }
 
-// the ordered sums of every haplotype enqueued so far are done before anything later on the main stream
-int join_sums(hx_matrix *cur) {
+// What the recovery entry points do before their walks: room for the paths and the stats of n haplotypes, orig's
+// counts (produced on orig's stream) ordered before the walk, the walk flags and the stats cleared (`done` must start
+// at 0 for the hole test of the ordered sums), the timing started.
+int recovery_prologue(hx_matrix *cur, hx_matrix *orig, int64_t path_bytes, int n) {
+    HX_CUDA(cur->d_path.grow(path_bytes, cur->stream));
+    HX_CUDA(cur->d_stats.grow(n * (int64_t)sizeof(hx_hap_stats), cur->stream));
+    if (orig->stream != cur->stream && orig->use.counts_dirty) {
+        const int rc = hx_ensure_counts(orig);
+        if (rc) return rc;
+        HX_CUDA(cudaStreamSynchronize(orig->stream));
+    }
+    HX_CUDA(cudaMemsetAsync(cur->d_flags.p, 0, offsetof(hx_dev_flags, walk_redone), cur->stream));
+    HX_CUDA(cudaMemsetAsync(cur->d_stats.p, 0, n * sizeof(hx_hap_stats), cur->stream));
+    HX_CUDA(cudaEventRecord(cur->ev0, cur->stream));
+    return HX_OK;
+}
+
+// ... and after them: the ordered sums of every haplotype joined into the main stream, the timing stopped, the stats of
+// n haplotypes, path_bytes of paths and (if `hole` is given) the hole flags copied back.
+int recovery_epilogue(hx_matrix *cur, hx_hap_stats *stats, int n, uint8_t *paths, int64_t path_bytes,
+                      hx_dev_flags *hole) {
     for (int b = 0; b < 2; ++b)
         if (cur->use.sum_busy[b]) { HX_CUDA(cudaStreamWaitEvent(cur->stream, cur->sum_done[b], 0)); cur->use.sum_busy[b] = false; }
+    HX_CUDA(cudaEventRecord(cur->ev1, cur->stream));
+    cur->use.ev_rec = true;
+    if (hole)
+        HX_CUDA(cudaMemcpyAsync(hole, cur->d_flags.p, offsetof(hx_dev_flags, q_unsafe), cudaMemcpyDeviceToHost, cur->stream));
+    HX_CUDA(cudaMemcpyAsync(stats, cur->d_stats.p, n * sizeof(hx_hap_stats), cudaMemcpyDeviceToHost, cur->stream));
+    HX_CUDA(cudaMemcpyAsync(paths, cur->d_path.p, (size_t)path_bytes, cudaMemcpyDeviceToHost, cur->stream));
+    HX_CUDA(cudaStreamSynchronize(cur->stream));
+    cudaEventElapsedTime(&cur->use.last_ms[1], cur->ev0, cur->ev1);
     return HX_OK;
 }
 
 int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *d_path,
-                    double *d_stats, double min_remove, int it = 0, int n_prev = 0) {
+                    hx_hap_stats *d_stats, double min_remove, int it = 0, int n_prev = 0) {
     int rc = hx_ensure_counts(cur);
     if (rc) return rc;
     rc = hx_ensure_counts(orig);
     if (rc) return rc;
     const int N = cur->N;
+    const int64_t sites = (int64_t)N + 2;
     const int Lw = L < cur->W ? (L < 1 ? 1 : L) : cur->W;          // lookbacks that stay inside the band
-    const int64_t n_terms = ((int64_t)N + 2) * Lw * HX_NSYM * 8;
     // float64 tables, then (quantised walk only) their int32 fixed-point twins with Lq >= L rows per site
-    static const bool no_q = getenv("HX_WALK_NOQ") != nullptr;   // debugging: force the float64 walk kernels
-    const bool use_q = !no_q && L >= 1 && L <= 32 && L <= cur->W;
+    const bool use_q = L >= 1 && L <= 32 && L <= cur->W;
     const int nit = use_q ? (L - 1 + 3) / 4 : 0;
     const int Lq = use_q ? 4 * nit + 1 : 0;
-    const int64_t n_all = n_terms + ((int64_t)N + 2) * 8;
-    const int64_t n_termsq = ((int64_t)N + 2) * Lq * HX_NSYM * 8;
-    const int64_t n_allq = n_termsq + ((int64_t)N + 2) * 8;
-    HX_CUDA(cur->d_terms.grow((n_all + (use_q ? (n_allq + 1) / 2 + 8 : 0)) * (int64_t)sizeof(double), cur->stream));
-    double *logm = cur->d_terms.p + n_terms;
-    int32_t *termsq = use_q ? reinterpret_cast<int32_t *>(cur->d_terms.p + n_all) : nullptr;
-    int32_t *logmq = use_q ? termsq + n_termsq : nullptr;
+    HX_CUDA(cur->terms.grow(sites * Lw * HX_NSYM * 8 * (int64_t)sizeof(double), cur->stream));
+    HX_CUDA(cur->logm.grow(sites * 8 * (int64_t)sizeof(double), cur->stream));
+    if (use_q) {
+        HX_CUDA(cur->termsq.grow(sites * Lq * HX_NSYM * 8 * (int64_t)sizeof(int32_t), cur->stream));
+        HX_CUDA(cur->logmq.grow(sites * 8 * (int64_t)sizeof(int32_t), cur->stream));
+    }
+    const double *terms = cur->terms.p, *logm = cur->logm.p;
+    int32_t *termsq = use_q ? cur->termsq.p : nullptr;
+    int32_t *logmq = use_q ? cur->logmq.p : nullptr;
+    hx_dev_flags *df = cur->d_flags.p;
     const int64_t tthreads = (int64_t)(N + 1) * (Lw > Lq ? Lw : Lq) * 8;
     k_walk_terms<<<(unsigned)((tthreads + 255) / 256), 256, 0, cur->stream>>>(cur->band.p, cur->vseen.p, N, cur->W, Lw,
-                                                                              flags, cur->d_terms.p, termsq, Lq,
-                                                                              cur->d_flags.p + 2);
+                                                                              flags, cur->terms.p, termsq, Lq,
+                                                                              &df->q_unsafe);
     // parallel-in-time walk (k_walk_q): blocks of sites walked concurrently from a guessed history, then verified
     int n_blocks = 1, blk_len = N > 0 ? N : 1, warm = 0;
     static const int blocks_env = getenv("HX_WALK_BLOCKS") ? atoi(getenv("HX_WALK_BLOCKS")) : 0;   // 1 = sequential
@@ -977,14 +962,15 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
         n_blocks = (N + blk_len - 1) / blk_len;
     }
     const int spec_stride = blk_len + warm;
-    HX_CUDA(cur->d_spec.grow((int64_t)n_blocks * HX_WALK_CAND * spec_stride + (int64_t)N + 2 + 8 * (int64_t)n_blocks * HX_WALK_CAND + 64,
-                             cur->stream));
-    uint8_t *spec = cur->d_spec.p;
-    uint8_t *guess = spec + (size_t)n_blocks * HX_WALK_CAND * spec_stride;
+    const int64_t n_starts = (int64_t)n_blocks * HX_WALK_CAND;
+    HX_CUDA(cur->spec.grow(n_starts * spec_stride, cur->stream));
+    HX_CUDA(cur->guess.grow(sites, cur->stream));
+    HX_CUDA(cur->spec_ok.grow(n_starts * (int64_t)sizeof(int), cur->stream));
+    HX_CUDA(cur->cand_idx.grow(n_starts * (int64_t)sizeof(int), cur->stream));
+    uint8_t *spec = cur->spec.p, *guess = cur->guess.p;
+    int *spec_ok = cur->spec_ok.p, *cand_idx = cur->cand_idx.p;
     const uint8_t *paths0 = d_path - (size_t)n_prev * ((size_t)N + 1);              // the haplotypes found so far (hx_recover)
-    int *spec_ok = reinterpret_cast<int *>(reinterpret_cast<uintptr_t>(guess + (size_t)N + 2 + 15) & ~(uintptr_t)15);
-    int *cand_idx = spec_ok + (size_t)n_blocks * HX_WALK_CAND;
-    k_walk_logm<<<(N + 1 + 127) / 128, 128, 0, cur->stream>>>(cur->scnt.p, N, flags, logm, logmq, guess);
+    k_walk_logm<<<(N + 1 + 127) / 128, 128, 0, cur->stream>>>(cur->scnt.p, N, flags, cur->logm.p, logmq, guess);
     if (n_blocks > 1) {
         k_walk_pick<<<n_blocks, 32, 0, cur->stream>>>(paths0, n_prev, N, L, blk_len, cand_idx);
         cur->use.launches++;
@@ -1002,13 +988,13 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
     case NIT:                                                                                                       \
         HX_CUDA(cudaFuncSetAttribute(k_walk_q<NIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qsmem));      \
         k_walk_q<NIT><<<1 + (n_blocks - 1) * HX_WALK_CAND, 32, qsmem, cur->stream>>>(                                  \
-            termsq, logmq, cur->d_terms.p, logm, N, L, Cq, blk_len, warm, guess, paths0, cand_idx, spec, spec_stride,  \
-            spec_ok, d_path, cur->d_flags.p);                                                                       \
+            termsq, logmq, terms, logm, N, L, Cq, blk_len, warm, guess, paths0, cand_idx, spec, spec_stride, spec_ok,   \
+            d_path, df);                                                                                            \
         if (n_blocks > 1) {                                                                                         \
             HX_CUDA(cudaFuncSetAttribute(k_walk_fix<NIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qsmem)); \
-            k_walk_fix<NIT><<<1, 32, qsmem, cur->stream>>>(termsq, logmq, cur->d_terms.p, logm, N, L, Cq, blk_len, warm, \
+            k_walk_fix<NIT><<<1, 32, qsmem, cur->stream>>>(termsq, logmq, terms, logm, N, L, Cq, blk_len, warm,        \
                                                            n_blocks, paths0, cand_idx, spec, spec_stride, spec_ok,     \
-                                                           d_path, cur->d_flags.p);                                     \
+                                                           d_path, df);                                                 \
             cur->use.launches++;                                                                                    \
         }                                                                                                           \
         break;
@@ -1018,12 +1004,11 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
         }
 #undef HX_WALK_Q
     } else if (C < 1) {
-        k_walk_wide<<<1, 256, 0, cur->stream>>>(cur->d_terms.p, logm, cur->vseen.p, N, L, Lw, flags, d_path, cur->d_flags.p);
+        k_walk_wide<<<1, 256, 0, cur->stream>>>(terms, logm, cur->vseen.p, N, L, Lw, flags, d_path, df);
     } else {
         const size_t wsmem = (size_t)3 * C * site_bytes;
         HX_CUDA(cudaFuncSetAttribute(k_walk_tables, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
-        k_walk_tables<<<1, 32, wsmem, cur->stream>>>(cur->d_terms.p, logm, cur->vseen.p, N, L, Lw, flags, C, d_path,
-                                                     cur->d_flags.p);
+        k_walk_tables<<<1, 32, wsmem, cur->stream>>>(terms, logm, cur->vseen.p, N, L, Lw, flags, C, d_path, df);
     }
     cur->use.launches += 2;
     // per-site values of this haplotype: two alternating buffers, so that the ordered sums of haplotype `it` (side
@@ -1035,8 +1020,8 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
         HX_CUDA(cudaEventCreateWithFlags(&cur->site_ready, cudaEventDisableTiming));
     }
     if (cur->use.sum_busy[it & 1]) HX_CUDA(cudaStreamWaitEvent(cur->stream, cur->sum_done[it & 1], 0));
-    k_path_stats<<<(N + 255) / 256, 256, 0, cur->stream>>>(cur->scnt.p, orig->scnt.p, N, d_path, site, cur->d_flags.p);
-    k_path_min<<<1, 1024, 0, cur->stream>>>(site, N, min_remove, d_stats, cur->d_flags.p);
+    k_path_stats<<<(N + 255) / 256, 256, 0, cur->stream>>>(cur->scnt.p, orig->scnt.p, N, d_path, site, df);
+    k_path_min<<<1, 1024, 0, cur->stream>>>(site, N, min_remove, d_stats, df);
     HX_CUDA(cudaEventRecord(cur->site_ready, cur->stream));
     HX_CUDA(cudaStreamWaitEvent(cur->sum_stream, cur->site_ready, 0));
     k_path_sum<<<1, 256, 0, cur->sum_stream>>>(site, N, d_stats);
@@ -1053,7 +1038,7 @@ int launch_generate(hx_matrix *cur, hx_matrix *orig, int L, int flags, uint8_t *
 extern "C" int hx_debug_walk_redone(hx_matrix *h, int *n) {
     if (!h || !n) return HX_E_ARG;
     if (cudaSetDevice(h->device) != cudaSuccess) return HX_E_CUDA;
-    if (cudaMemcpyAsync(n, h->d_flags.p + 3, sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return HX_E_CUDA;
+    if (cudaMemcpyAsync(n, &h->d_flags.p->walk_redone, sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return HX_E_CUDA;
     if (cudaStreamSynchronize(h->stream) != cudaSuccess) return HX_E_CUDA;
     return HX_OK;
 }
@@ -1118,38 +1103,21 @@ int hx_generate_path(hx_matrix *cur, hx_matrix *orig, int32_t L, int flags, uint
     HX_CHECK_ARG(cur && orig && out_path && out && hole_site);
     HX_CHECK_ARG(cur->N == orig->N && cur->device == orig->device && L >= 0 && L <= HX_MAX_L);
     HX_CUDA(cudaSetDevice(cur->device));
-    const int N = cur->N;
-    HX_CUDA(cur->d_path.grow((int64_t)N + 2, cur->stream));
-    HX_CUDA(cur->d_stats.grow(8 * (int64_t)sizeof(double), cur->stream));
-    // orig's counts are produced on orig's stream; order them before our walk
-    if (orig->stream != cur->stream && orig->use.counts_dirty) {
-        const int rc = hx_ensure_counts(orig);
-        if (rc) return rc;
-        HX_CUDA(cudaStreamSynchronize(orig->stream));
-    }
-    HX_CUDA(cudaMemsetAsync(cur->d_flags.p, 0, 3 * sizeof(int), cur->stream));
-    HX_CUDA(cudaEventRecord(cur->ev0, cur->stream));
-    // (the single-haplotype entry point: stats[5] must start at 0 for the hole test of the ordered sums)
-    HX_CUDA(cudaMemsetAsync(cur->d_stats.p, 0, 8 * sizeof(double), cur->stream));
-    int rc = launch_generate(cur, orig, L, flags, cur->d_path.p, cur->d_stats.p, 0.0);
+    const int64_t N = cur->N;
+    int rc = recovery_prologue(cur, orig, N + 2, 1);
     if (rc) return rc;
-    rc = join_sums(cur);
+    rc = launch_generate(cur, orig, L, flags, cur->d_path.p, cur->d_stats.p, 0.0);
     if (rc) return rc;
-    HX_CUDA(cudaEventRecord(cur->ev1, cur->stream));
-    cur->use.ev_rec = true;
-    int hflags[2];
-    double stats[8];
-    HX_CUDA(cudaMemcpyAsync(hflags, cur->d_flags.p, sizeof(hflags), cudaMemcpyDeviceToHost, cur->stream));
-    HX_CUDA(cudaMemcpyAsync(stats, cur->d_stats.p, sizeof(stats), cudaMemcpyDeviceToHost, cur->stream));
-    HX_CUDA(cudaMemcpyAsync(out_path, cur->d_path.p, (size_t)N + 1, cudaMemcpyDeviceToHost, cur->stream));
-    HX_CUDA(cudaStreamSynchronize(cur->stream));
-    cudaEventElapsedTime(&cur->use.last_ms[1], cur->ev0, cur->ev1);
-    if (hflags[1]) {
-        *hole_site = hflags[0];
+    hx_hap_stats st;
+    hx_dev_flags hf;
+    rc = recovery_epilogue(cur, &st, 1, out_path, N + 1, &hf);
+    if (rc) return rc;
+    if (hf.hole) {
+        *hole_site = hf.hole_site;
         return HX_HOLE;
     }
     *hole_site = 0;
-    out[0] = stats[0]; out[1] = stats[1]; out[2] = stats[2];
+    out[0] = st.hp_current; out[1] = st.hp_original; out[2] = st.min_marginal;
     return HX_OK;
 }
 
@@ -1157,7 +1125,7 @@ int hx_reweight_path(hx_matrix *h, const uint8_t *path, double ratio, double *re
     HX_CHECK_ARG(h && path && removed);
     HX_CUDA(cudaSetDevice(h->device));
     HX_CUDA(h->d_path.grow((int64_t)h->N + 2, h->stream));
-    HX_CUDA(cudaMemsetAsync(h->d_flags.p, 0, 3 * sizeof(int), h->stream));
+    HX_CUDA(cudaMemsetAsync(h->d_flags.p, 0, offsetof(hx_dev_flags, walk_redone), h->stream));
     HX_CUDA(cudaMemcpyAsync(h->d_path.p, path, (size_t)h->N + 1, cudaMemcpyHostToDevice, h->stream));
     HX_CUDA(cudaEventRecord(h->ev0, h->stream));
     const int rc = launch_reweight(h, h->d_path.p, nullptr, ratio, h->d_misc.p);
@@ -1178,48 +1146,27 @@ int hx_recover(hx_matrix *cur, hx_matrix *orig, int32_t L, int flags, int32_t ma
     const int64_t N = cur->N;
     *n_found = 0;
     if (max_paths == 0) return HX_OK;
-    HX_CUDA(cur->d_path.grow((N + 1) * (int64_t)max_paths, cur->stream));
-    HX_CUDA(cur->d_stats.grow(8 * (int64_t)sizeof(double) * max_paths, cur->stream));
-    if (orig->stream != cur->stream && orig->use.counts_dirty) {
-        const int rc = hx_ensure_counts(orig);
-        if (rc) return rc;
-        HX_CUDA(cudaStreamSynchronize(orig->stream));
-    }
-    HX_CUDA(cudaMemsetAsync(cur->d_flags.p, 0, 3 * sizeof(int), cur->stream));
-    HX_CUDA(cudaMemsetAsync(cur->d_stats.p, 0, 8 * sizeof(double) * (size_t)max_paths, cur->stream));
-    HX_CUDA(cudaEventRecord(cur->ev0, cur->stream));
+    int rc = recovery_prologue(cur, orig, (N + 1) * max_paths, max_paths);
+    if (rc) return rc;
     for (int it = 0; it < max_paths; ++it) {
         uint8_t *dp = cur->d_path.p + (size_t)it * (N + 1);
-        double *ds = cur->d_stats.p + (size_t)it * 8;
-        int rc = launch_generate(cur, orig, L, flags, dp, ds, min_remove, it, it);
+        hx_hap_stats *ds = cur->d_stats.p + it;
+        rc = launch_generate(cur, orig, L, flags, dp, ds, min_remove, it, it);
         if (rc) return rc;
-        rc = launch_reweight(cur, dp, ds + 3, 0.0, ds + 4);
+        rc = launch_reweight(cur, dp, &ds->ratio, 0.0, &ds->removed);
         if (rc) return rc;
     }
-    const int rc = join_sums(cur);
-    if (rc) return rc;
-    HX_CUDA(cudaEventRecord(cur->ev1, cur->stream));
-    cur->use.ev_rec = true;
-    double *hs = (double *)malloc(sizeof(double) * 8 * (size_t)max_paths);
+    hx_hap_stats *hs = (hx_hap_stats *)malloc(sizeof(hx_hap_stats) * (size_t)max_paths);
     if (!hs) return HX_E_NOMEM;
-    cudaError_t e = cudaMemcpyAsync(hs, cur->d_stats.p, sizeof(double) * 8 * (size_t)max_paths,
-                                    cudaMemcpyDeviceToHost, cur->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(paths, cur->d_path.p, (size_t)(N + 1) * max_paths, cudaMemcpyDeviceToHost, cur->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(cur->stream);
-    if (e != cudaSuccess) {
-        free(hs);
-        hx_set_error("hx_recover: %s", cudaGetErrorString(e));
-        return HX_E_CUDA;
-    }
-    cudaEventElapsedTime(&cur->use.last_ms[1], cur->ev0, cur->ev1);
+    rc = recovery_epilogue(cur, hs, max_paths, paths, (N + 1) * max_paths, nullptr);
     int found = 0;
-    for (int it = 0; it < max_paths; ++it) {
-        if (hs[(size_t)it * 8 + 5] != 1.0) break;
-        for (int q = 0; q < 5; ++q) stats[(size_t)it * 5 + q] = hs[(size_t)it * 8 + q];
-        found++;
+    for (; !rc && found < max_paths && hs[found].done == 1.0; ++found) {
+        const hx_hap_stats &h = hs[found];
+        double *o = stats + (size_t)found * 5;          // hanselx.h: hp_current, hp_original, min_marginal, ratio, removed
+        o[0] = h.hp_current; o[1] = h.hp_original; o[2] = h.min_marginal; o[3] = h.ratio; o[4] = h.removed;
     }
     free(hs);
+    if (rc) return rc;
     *n_found = found;
     return HX_OK;
 }

@@ -192,6 +192,32 @@ def test_walk_leaves_fixed_point_range(c_oracle):
     _walk_vs_c_oracle(c_oracle, h, band, N, W, 6, iters=2)
 
 
+def _float64_walk(W, L):
+    """Which float64 walk launch_generate runs for L > 32: k_walk_wide when three staged chunks of one site's tables
+    (Lw * 448 + 64 bytes, Lw = min(L, W)) cannot fit its 200 KiB of shared memory, k_walk_tables otherwise."""
+    Lw = min(L, W)
+    return "wide" if (200 * 1024) // (3 * (Lw * 448 + 64)) < 1 else "tables"
+
+
+@pytest.mark.parametrize("kernel,dL", [("tables", None), ("wide", 0), ("wide", 20)],
+                         ids=["tables_L100", "wide_L_W", "wide_L_W+20"])
+def test_wide_band_walks(c_oracle, kernel, dL):
+    """Reads of up to 170 SNPs make a band wide enough (W >= 153) that one site's float64 tables do not fit the staged
+    walk: k_walk_wide walks at L = W, and at L = W + 20 with lookbacks beyond the band (log10(1/V) terms).  L = 100
+    is the staged k_walk_tables inside the same band."""
+    rng = np.random.default_rng(5150)
+    N = 400
+    rank, off, codes = synth.random_packed(rng, N, 600, 170, p_special=0.05)
+    W = int(np.diff(off).max()) - 1
+    L = 100 if dL is None else W + dL
+    assert W >= 153 and _float64_walk(W, L) == kernel and (L > W) == (dL == 20)
+    band, _ = c_oracle.ingest(rank, off, codes, N, W)
+    cur = band.astype(np.float32)
+    assert c_oracle.generate_path(cur, cur.copy(), N, W, L)[0] is not None      # the first walk reaches site N
+    h = _mk(rank, off, codes, N, W)
+    _walk_vs_c_oracle(c_oracle, h, band, N, W, L, packed=(rank, off, codes))
+
+
 import glob
 
 GOLDEN_RECOVERY = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "ref_recovery_*.npz")))
