@@ -5,7 +5,8 @@
 Everything that computes (ingestion, gap check counts, recovery, reweighting) runs in the CUDA
 library; this file is host-side bookkeeping and output formatting only: PATHS de-duplication
 (cmd.py:164-179), out.fasta / snp.fasta (cmd.py:181-221) and gretel.crumbs (cmd.py:223-240,
-docs/protocol.rst:48-77).
+docs/protocol.rst:48-77), and with --support the reads carried by each haplotype (gretel.support, no reference
+counterpart).
 """
 from __future__ import annotations
 
@@ -51,6 +52,10 @@ def build_parser():
     p.add_argument("--dumpsnps", type=str, default=None)
     p.add_argument("--pepper", action="store_true")
     p.add_argument("--device", type=int, default=None)
+    p.add_argument("--support", action="store_true",
+                   help="write gretel.support: the reads each recovered haplotype carries")
+    p.add_argument("--max-mismatch", type=int, default=-1,
+                   help="--support: a read whose best haplotype has more mismatches is not assigned (-1: no limit)")
     p.add_argument("--version", action="version", version="%(prog)s " + __version__)
     return p
 
@@ -94,6 +99,17 @@ def write_outputs(dirn, PATHS, hansel, vcf_h, start, end, master=None, gapchar="
                 ",".join("%.2f" % x for x in p["hp_original"]), p["magnitude"]))
 
 
+def write_support(dirn, records, totals):
+    """gretel.support: '# reads, assigned, uninformative, over_limit, max_mismatch', then per distinct haplotype in
+    i_0 order: i_0, unique reads, shared reads, share of the reads, share / assigned."""
+    with open(dirn.rstrip("/") + "/gretel.support", "w") as fh:
+        fh.write("# %d\t%d\t%d\t%d\t%d\n" % (totals["reads"], totals["assigned"], totals["uninformative"],
+                                             totals["over_limit"], totals["max_mismatch"]))
+        for r in records:
+            fh.write("%d\t%d\t%d\t%.2f\t%.4f\n" % (r["i_0"], r["unique"], r["shared"], r["share"],
+                                                 r["share"] / totals["assigned"] if totals["assigned"] else 0.0))
+
+
 def main(argv=None):
     args = build_parser().parse_args(argv)
     if args.end == -1:
@@ -104,8 +120,9 @@ def main(argv=None):
         with open(args.dumpsnps, "w") as fh:
             for k in sorted(vcf_h["snp_fwd"].keys()):
                 fh.write("%d\t%d\t%d\n" % (vcf_h["snp_fwd"][k] + 1, k, k - args.start + 1))
+    reads = {} if args.support else None
     hansel = util.load_from_bam(args.bam, args.contig, args.start, args.end, vcf_h, n_threads=args.threads,
-                                stepper="all" if args.pepper else "samtools", device=args.device)
+                                stepper="all" if args.pepper else "samtools", device=args.device, reads=reads)
     if args.dumpmatrix:
         hansel.save_hansel_dump(args.dumpmatrix)
     gaps = gretel.gap_check(hansel, vcf_h["N"])
@@ -119,6 +136,10 @@ def main(argv=None):
     _, PATHS = gretel.recover(hansel, vcf_h["N"], max_paths=args.paths, min_remove=0.01)
     write_outputs(args.out, PATHS, hansel, vcf_h, args.start, args.end, master=args.master,
                   gapchar=args.gapchar, delchar=args.delchar)
+    if args.support:
+        records, totals = gretel.read_support(hansel, PATHS, reads["rank"], reads["off"], reads["codes"],
+                                              max_mismatch=args.max_mismatch)
+        write_support(args.out, records, totals)
     return 0
 
 

@@ -127,6 +127,10 @@ struct hx_matrix {
     HxDevBuf<int4> d_jobs;           // per-CTA job tables of the tensor-core kernel (ingest_umma.cu)
     HxDevBuf<double> d_misc;         // small outputs (weights etc.)
     HxDevBuf<uint32_t> d_pack;       // packed counts for the cross-GPU exchange (api.cu)
+    // read support (support.cu): haplotype codes and bit-planes, the sums, one chunk of reads, per-read results
+    HxDevBuf<uint8_t> a_haps; HxDevBuf<uint4> a_planes; HxDevBuf<unsigned long long> a_sums;
+    HxDevBuf<int32_t> a_rank; HxDevBuf<int64_t> a_off; HxDevBuf<uint8_t> a_codes; HxDevBuf<int32_t> a_best;
+    cudaEvent_t a_ev[2];             // times the assignment kernels (hx_last_kernel_ms which = 3)
     void *h_pinned;                  // small host buffer for D2H of scalars
     void *lr_scratch;                // long-read ingestion scratch (ingest_long.cu)
     void *l2_scratch;                // long-read tensor-core ingestion scratch (ingest_lumma.cu)
@@ -143,7 +147,7 @@ struct hx_matrix {
         bool prepass_ran = false;    // d_flags->ingest_sorted holds the sortedness verdict of the last ingestion launch
         int wire_next = 0;           // the next staging set of the dense wire format
         bool sum_busy[2] = {};       // sum_done[b] marks ordered sums not yet joined into the main stream
-        float last_ms[3] = {};
+        float last_ms[4] = {};
     } use;
 };
 
@@ -257,3 +261,5 @@ int64_t hx_lumma_scratch_bytes(const hx_matrix *h, int64_t n_reads);
 void hx_l2_free(hx_matrix *h);
 // recover.cu
 int hx_ensure_counts(hx_matrix *h);
+// support.cu
+void hx_support_free(hx_matrix *h);

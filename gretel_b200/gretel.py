@@ -8,6 +8,8 @@ from __future__ import annotations
 
 import sys
 
+import numpy as np
+
 
 def reweight_hansel_from_path(hansel, path, ratio):
     """gretel/gretel.py:13-98 -> sum of removed observations (float)."""
@@ -82,3 +84,25 @@ def recover(hansel, n_snps, max_paths=100, min_remove=0.01, original_hansel=None
 def gap_check(hansel, n_snps):
     """gretel/cmd.py:85-92: sites whose pairwise evidence total is zero."""
     return [i for i in range(0, n_snps + 1) if hansel.get_counts_at(i).get("total", 0) == 0]
+
+
+def read_support(hansel, PATHS, rank, off, codes, max_mismatch=-1):
+    """Reads carried by each recovered haplotype: the packed reads are assigned to the distinct paths of ``PATHS``
+    (Hansel.assign_reads) in ``i_0`` order, the order of out.fasta.  Returns (records, totals): one dict per path
+    with i_0, unique, shared, share and share_q32, and a dict with reads, assigned, uninformative, over_limit and
+    max_mismatch.  With no path no read is assigned: reads without an informative site are uninformative, the
+    others over the limit."""
+    keys = sorted(PATHS, key=lambda x: PATHS[x]["i_0"])
+    totals = {"reads": len(rank), "max_mismatch": int(max_mismatch)}
+    if not keys:
+        off = np.asarray(off, dtype=np.int64)
+        informative = np.concatenate([[0], np.cumsum(np.isin(codes[off[0]:off[-1]], (4, 6), invert=True))])
+        n_unin = int((np.diff(informative[off - off[0]]) == 0).sum())
+        totals.update(assigned=0, uninformative=n_unin, over_limit=len(rank) - n_unin)
+        return [], totals
+    paths = np.stack([hansel.encode_path(PATHS[k]["hansel_path"]) for k in keys])
+    res = hansel.assign_reads(paths, rank, off, codes, max_mismatch=max_mismatch)
+    totals.update(assigned=res.assigned, uninformative=res.uninformative, over_limit=res.over_limit)
+    records = [{"i_0": PATHS[k]["i_0"], "unique": int(res.unique[j]), "shared": int(res.shared[j]),
+                "share": float(res.share[j]), "share_q32": int(res.share_q32[j])} for j, k in enumerate(keys)]
+    return records, totals

@@ -31,6 +31,22 @@ def _default_device():
     return int(os.environ.get("GRETEL_B200_DEVICE", os.environ.get("LOCAL_RANK", "0")))
 
 
+class ReadSupport:
+    """What Hansel.assign_reads reports.  Per haplotype: ``unique`` (reads whose only best haplotype it is),
+    ``shared`` (reads tied between it and others), ``share_q32`` (uint64: the sum of floor(2^32/ties) over the
+    reads it is a best haplotype of) and ``share`` = share_q32 / 2^32.  Totals ``assigned``, ``uninformative``
+    (no informative site) and ``over_limit`` (fewest mismatches above max_mismatch).  With per_read: ``best_mm``
+    (fewest mismatches, -1 if uninformative), ``n_best`` (ties, 0 if uninformative), ``first_best`` (lowest best
+    haplotype, -1 unless assigned); None otherwise."""
+
+    def __init__(self, unique, shared, share_q32, assigned, uninformative, over_limit, best_mm=None, n_best=None,
+                 first_best=None):
+        self.unique, self.shared, self.share_q32 = unique, shared, share_q32
+        self.share = share_q32.astype(np.float64) / 2.0 ** 32
+        self.assigned, self.uninformative, self.over_limit = assigned, uninformative, over_limit
+        self.best_mm, self.n_best, self.first_best = best_mm, n_best, first_best
+
+
 class Hansel:
     def __init__(self, symbols, unsymbols, n_snps, band_w=None, device=None, _handle=None,
                  v_site="from", candidates_skip_unsymbols=True):
@@ -383,6 +399,30 @@ class Hansel:
         self._touch()
         return paths[:n.value], stats[:n.value]
 
+    # ---- read support ------------------------------------------------------------------------
+    def assign_reads(self, paths, rank, off, codes, max_mismatch=-1, per_read=False):
+        """Assign packed reads to the haplotypes ``paths`` (uint8 [H][N+1], as recover_codes returns them) by the
+        fewest mismatches at the read's informative sites; ties split a read equally (hx_assign_reads).  The
+        matrix supplies N and the device; its counts are not touched.  -> ReadSupport."""
+        paths = np.ascontiguousarray(paths, dtype=np.uint8)
+        if paths.ndim != 2 or paths.shape[1] != self.n_snps + 1:
+            raise ValueError("paths must be uint8 [n_haps][N+1]")
+        rank = np.ascontiguousarray(rank, dtype=np.int32)
+        off = np.ascontiguousarray(off, dtype=np.int64)
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        if len(off) != len(rank) + 1:
+            raise ValueError("off must have len(rank)+1 entries")
+        H, R = paths.shape[0], len(rank)
+        unique, shared = np.zeros(H, dtype=np.int64), np.zeros(H, dtype=np.int64)
+        share_q32 = np.zeros(H, dtype=np.uint64)
+        totals = np.zeros(3, dtype=np.int64)
+        per = [np.zeros(R, dtype=np.int32) for _ in range(3)] if per_read else [None] * 3
+        _lib.check(self._lib.hx_assign_reads(
+            self._h, paths.ctypes.data, H, rank.ctypes.data, off.ctypes.data, codes.ctypes.data, R, int(max_mismatch),
+            unique.ctypes.data, shared.ctypes.data, share_q32.ctypes.data, totals.ctypes.data,
+            *[a.ctypes.data if a is not None else None for a in per]))
+        return ReadSupport(unique, shared, share_q32, int(totals[0]), int(totals[1]), int(totals[2]), *per)
+
     # ---- bulk I/O ----------------------------------------------------------------------------
     def band(self):
         """float32 [N+2][W][7][7]; cell (pi,pj) at [pj][pj-pi-1]."""
@@ -427,7 +467,8 @@ class Hansel:
 
     def kernel_ms(self, which):
         ms = C.c_float()
-        _lib.check(self._lib.hx_last_kernel_ms(self._h, {"ingest": 0, "walk": 1, "reweight": 2}[which], C.byref(ms)))
+        _lib.check(self._lib.hx_last_kernel_ms(self._h, {"ingest": 0, "walk": 1, "reweight": 2, "assign": 3}[which],
+                                               C.byref(ms)))
         return float(ms.value)
 
     def launch_count(self):

@@ -65,7 +65,8 @@ def make_sites(rng, genome_len, n_snps):
 
 
 def generate(w: Workload, seed=None, shard=0, chunk=2_000_000):
-    """Return dict(rank, off, codes, n_snps, sites, strains, max_k, n_obs_upper)."""
+    """Return dict(rank, off, codes, n_snps, sites, strains, max_k, n_pairs, strain_of); strain_of[i] is the
+    strain read i was drawn from."""
     if seed is None:
         seed = 20260000 + w.config + 1
     # strains/sites depend on the workload seed only; reads also on the shard so that
@@ -122,7 +123,7 @@ def generate(w: Workload, seed=None, shard=0, chunk=2_000_000):
     return {
         "rank": rank.astype(np.int32), "off": off, "codes": codes, "n_snps": N,
         "sites": sites, "strains": strains, "max_k": int(k.max()) if len(k) else 0,
-        "n_pairs": int((k * (k - 1) // 2).sum()),
+        "n_pairs": int((k * (k - 1) // 2).sum()), "strain_of": strain_of,
     }
 
 

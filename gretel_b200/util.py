@@ -222,14 +222,15 @@ def set_totals(hansel, slices, crumbs, covered, quiet=True):
 
 def load_from_bam(bam_path, target_contig, start_pos, end_pos, vcf_handler, use_end_sentinels=False,
                   n_threads=1, debug_reads=False, debug_pos=False, stepper="samtools", device=None,
-                  band_w=None, max_depth=bamio.PYSAM_MAX_DEPTH, stages=None):
+                  band_w=None, max_depth=bamio.PYSAM_MAX_DEPTH, stages=None, reads=None):
     """gretel/util.py:33.  Same signature and return value; ``n_threads`` is accepted for
     compatibility (the reference's window sharding is replaced by one GPU kernel and the
     result is independent of it, cf. tests/test_test.py:35).  ``use_end_sentinels`` is an
     experimental dead branch upstream (never passed, cmd.py:78) and is rejected here.  ``max_depth``: the
     reference reads the BAM through pysam's pileup, whose buffer drops reads beyond 8000 per position
     (bamio._DepthCap); the default reproduces that, ``max_depth=0`` keeps every read.  ``stages``: dict that
-    receives per-stage seconds of the packer and of the GPU ingestion."""
+    receives per-stage seconds of the packer and of the GPU ingestion.  ``reads``: dict that receives the packed
+    reads ``rank``, ``off`` and ``codes`` (for Hansel.assign_reads)."""
     if use_end_sentinels:
         raise NotImplementedError("use_end_sentinels is never enabled by the reference (cmd.py:28,78)")
     # n_threads (the reference's number of BAM iterators, cmd.py:31) drives the native packer's threads
@@ -246,6 +247,8 @@ def load_from_bam(bam_path, target_contig, start_pos, end_pos, vcf_handler, use_
             band_w = max(band_w, vcf_handler["N"] + 1)
     h = load_from_packed(rank, off, codes, vcf_handler["N"], band_w=band_w, device=device, quiet=False,
                          n_threads=max(1, n_threads))
+    if reads is not None:
+        reads.update(rank=rank, off=off, codes=codes)
     if stages is not None:
         stages["pack_total"] = t1 - t0
         stages["gpu_ingest"] = time.perf_counter() - t1

@@ -180,6 +180,20 @@ int hx_reweight_path(hx_matrix *h, const uint8_t *path, double ratio, double *re
 int hx_recover(hx_matrix *cur, hx_matrix *orig, int32_t L, int flags, int32_t max_paths,
                double min_remove, uint8_t *paths, double *stats, int32_t *n_found);
 
+/* ---- read support ------------------------------------------------------------------ */
+/* Read support for recovered haplotypes (no reference counterpart; see DESIGN.md).  haps[n_haps*(N+1)]: paths as
+ * hx_recover writes them; reads as for hx_ingest_host (any order, any width).  max_mismatch < 0: no limit.
+ * Per-haplotype unique/shared (int64) and share_q32 (uint64) [n_haps]; totals[3] = {assigned, uninformative,
+ * over_limit}.  best_mm, n_best, first_best: int32[n_reads] each, or NULL.  Synchronous.
+ * A read goes to the haplotypes with the fewest mismatches at its informative sites (codes other than N and _);
+ * a tie splits it into floor(2^32/ties) per tied haplotype.  HX_E_READ: a read past site N or a code > 6;
+ * HX_E_ARG: a haplotype code > 6 at a site in 1..N.  The matrix supplies N, the device, the stream and scratch;
+ * its counts are neither read nor changed. */
+int hx_assign_reads(hx_matrix *h, const uint8_t *haps, int32_t n_haps,
+                    const int32_t *rank, const int64_t *off, const uint8_t *codes, int64_t n_reads,
+                    int32_t max_mismatch, int64_t *unique, int64_t *shared, uint64_t *share_q32,
+                    int64_t totals[3], int32_t *best_mm, int32_t *n_best, int32_t *first_best);
+
 /* ---- BAM -> packed reads on the CPU (the producer side of the boundary) ------------ */
 /* Replaces the pysam column pileup of gretel/util.py:112-210: multi-threaded BGZF inflate and one
  * CIGAR walk per alignment against the sorted 1-based SNP positions.  stepper: 0 = samtools,
@@ -248,7 +262,8 @@ int hx_band_to_host(hx_matrix *h, float *out /* (N+2)*W*49 */);
 int hx_band_from_host(hx_matrix *h, const float *in);
 int hx_to_dense(hx_matrix *h, float *out /* 7*7*(N+2)*(N+2) */);
 /* last kernel timings in ms measured with CUDA events on the matrix's stream:
- * which = 0 ingest, 1 generate_path walk, 2 reweight */
+ * which = 0 ingest, 1 generate_path walk, 2 reweight, 3 the assignment kernels of the last hx_assign_reads
+ * (copies excluded) */
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms);
 /* number of kernel launches issued by this matrix so far */
 int hx_launch_count(const hx_matrix *h, int64_t *n);
