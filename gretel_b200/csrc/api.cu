@@ -449,12 +449,8 @@ int hx_ingest_host(hx_matrix *h, const int32_t *rank, const int64_t *off, const 
         }
         int64_t a = 0;
         for (int c = 0; c < n_chunks; ++c) {
-            int64_t b = n_reads;
-            if (c + 1 < n_chunks) {
-                const int64_t target = off[0] + n_codes * (c + 1) / n_chunks;
-                b = std::lower_bound(off + a, off + n_reads, target) - off;
-                if (b <= a) continue;
-            }
+            const int64_t b = hx_chunk_end(off, a, n_reads, n_codes, c, n_chunks);
+            if (b <= a && c + 1 < n_chunks) continue;
             HX_CUDA(cudaMemcpyAsync(h->s_rank.p + a, rank + a, sizeof(int32_t) * (size_t)(b - a), cudaMemcpyHostToDevice, cs));
             HX_CUDA(cudaMemcpyAsync(h->s_off.p + a, off + a, sizeof(int64_t) * (size_t)(b - a + 1), cudaMemcpyHostToDevice, cs));
             HX_CUDA(cudaMemcpyAsync(h->s_codes.p + (off[a] - off[0]), codes + off[a], (size_t)(off[b] - off[a]), cudaMemcpyHostToDevice, cs));

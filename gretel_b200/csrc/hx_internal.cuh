@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <algorithm>
+
 #include "hanselx.h"
 
 #define HX_NSYM 7
@@ -27,6 +29,13 @@ struct HxCnt {
         uint32_t *base = local;
         if (world > 1) base = peer[pj / rows_per];
         return base + (pj * W + (pj - pi - 1)) * 49;
+    }
+    // The target as a kernel instantiation sees it: FUSED = false (a single-GPU build) folds the peer path away.
+    template <bool FUSED>
+    __device__ __forceinline__ HxCnt for_build() const {
+        HxCnt c = *this;
+        if (!FUSED) { c.world = 1; c.rows_per = 1; c.peer = nullptr; }
+        return c;
     }
 #endif
 };
@@ -198,6 +207,13 @@ static inline cudaError_t hx_fill_async(void *p, int byte, size_t bytes, cudaStr
 
 __host__ __device__ __forceinline__ int64_t hx_cell_off(int64_t W, int64_t pi, int64_t pj) {
     return (pj * W + (pj - pi - 1)) * HX_CELL;
+}
+
+// Host arrays sent in n_chunks chunks of about equal code counts, cut at read boundaries: the end (exclusive) of
+// chunk c, which starts at read a.  The last chunk ends at n_reads; an earlier one may come out empty (end <= a).
+static inline int64_t hx_chunk_end(const int64_t *off, int64_t a, int64_t n_reads, int64_t n_codes, int c, int n_chunks) {
+    if (c + 1 == n_chunks) return n_reads;
+    return std::lower_bound(off + a, off + n_reads, off[0] + n_codes * (c + 1) / n_chunks) - off;
 }
 
 #ifdef __CUDACC__

@@ -90,7 +90,7 @@ k1_pairs_red(const int32_t *__restrict__ rank, const int64_t *__restrict__ off,
         const int64_t k64 = off[r + 1] - o;
         if (k64 < 2) continue;                                                  // util.py:230
         const int rk = rank[r];
-        if (rk < 0 || (int64_t)rk + k64 > N || k64 - 1 > W) {
+        if (!read_fits(rk, k64, N, W)) {
             if (lane == 0) atomicOr(err, 1);
             continue;
         }
@@ -144,30 +144,6 @@ struct BsLayout {
         return tile_u4() * 16 + (size_t)2 * gb * kmax * 16 + 64 * sizeof(int) + (size_t)2 * gb * 32 * sizeof(int);
     }
 };
-
-// rows [pj_lo, pj_hi] of the tile: add every non-zero counter to HBM, clear it; returns the sum
-// flushed by this thread (every regular-cell increment is one crumb, util.py:268,276,281).
-__device__ __forceinline__ unsigned long long bs_flush_rows(uint32_t *tile32, int rows, int cells,
-                                                            int64_t pj_lo, int64_t pj_hi, int64_t W,
-                                                            const HxCnt cnt) {
-    unsigned long long sum = 0;
-    const int per_row = cells * 16;
-    int row = (int)(pj_lo % rows);
-    for (int64_t pj = pj_lo; pj <= pj_hi; ++pj) {
-        uint32_t *base = tile32 + (size_t)row * per_row;
-        for (int w = threadIdx.x; w < per_row; w += blockDim.x) {
-            const uint32_t v = base[w];
-            if (v) {
-                const int d = (w >> 4) + 1, ab = w & 15;
-                atomicAdd(cnt.cell(W, pj - d, pj) + (ab >> 2) * HX_NSYM + (ab & 3), v);
-                base[w] = 0;
-                sum += v;
-            }
-        }
-        if (++row == rows) row = 0;
-    }
-    return sum;
-}
 
 // Transposes one group of 32 reads (lane = read, kb SNPs each, codes at codes+o) into bit-planes in
 // shared memory: planes[t] = {v, b0, b1, -} with bit r of v set when read r holds A/C/G/T at site t and
@@ -283,8 +259,7 @@ k1_bitsliced(const int32_t *__restrict__ rank, const int64_t *__restrict__ off,
              int *__restrict__ err, const int *__restrict__ sorted_flag,
              const int64_t *__restrict__ run_end) {
     extern __shared__ uint4 smem4[];
-    HxCnt cnt = cnt_in;                              // single-GPU build: the peer path folds away
-    if (!FUSED) { cnt.world = 1; cnt.rows_per = 1; cnt.peer = nullptr; }
+    const HxCnt cnt = cnt_in.for_build<FUSED>();
     if (!*sorted_flag) return;                       // the generic fallback launch takes over
     const int rows = kmax + 1, cells = kmax - 1;
     uint4 *const tile = smem4;
@@ -368,7 +343,7 @@ k1_bitsliced(const int32_t *__restrict__ rank, const int64_t *__restrict__ off,
                 // rows pj <= r+1 can no longer be touched by this CTA (reads of rank >= r start at pj = r+2)
                 if ((int64_t)r + 1 > flushed_upto) {
                     const int64_t last = min((int64_t)r + 1, flushed_upto + rows - 2);
-                    t_crumbs += bs_flush_rows(tile32, rows, cells, flushed_upto + 1, last, W, cnt);
+                    t_crumbs += bs_flush_rows(tile32, rows, cells, flushed_upto + 1, last, W, cnt, blockDim.x, true);
                     flushed_upto = (int64_t)r + 1;
                     __syncthreads();                 // the retired ring slots may be reused by this run's tile add
                 }
@@ -440,7 +415,7 @@ k1_bitsliced(const int32_t *__restrict__ rank, const int64_t *__restrict__ off,
                     o = off[idx];
                     const int64_t k64 = off[idx + 1] - o;
                     if (k64 >= 2) {
-                        if (r < 0 || (int64_t)r + k64 > N || k64 - 1 > W) errbits |= 1;
+                        if (!read_fits(r, k64, N, W)) errbits |= 1;
                         else kb = (int)k64;
                     }
                     // last read of the batch: the next batch's codes start right behind it
@@ -449,24 +424,11 @@ k1_bitsliced(const int32_t *__restrict__ rank, const int64_t *__restrict__ off,
                 n_slices += kb >= 2;
                 n_codes += kb;
                 uint32_t rare_or, x0;
-                const uint8_t *__restrict__ c = codes + o;
                 const int kg = bs_build_group<KW>(codes, o, kb, planes_saddr + (uint32_t)((buf * gb + g) * kmax) * 16u,
                                                   rare_or, x0);
                 if (lane == 0) gk[g] = kg;
                 if (kb >= 2) {
-                    // start sentinel (util.py:262-266) / end sentinel (:271-275); the start rule wins
-                    const unsigned a0 = x0 & 0xffu;
-                    if (r == 0 && sym_valid_from(a0)) {
-                        atomicAdd(cnt.cell(W, 0, 1) + HX_SYM_GAP * HX_NSYM + a0, 1u);
-                        n_sent++;
-                    }
-                    if (r + kb == N && !(kb == 2 && r == 0)) {
-                        const unsigned ap = c[kb - 2], bl = c[kb - 1];
-                        if (sym_valid_from(ap) && bl <= 6) {
-                            atomicAdd(cnt.cell(W, N, N + 1) + bl * HX_NSYM + HX_SYM_GAP, 1u);
-                            n_sent++;
-                        }
-                    }
+                    add_sentinels(codes + o, x0 & 0xffu, r, kb, N, W, cnt, n_sent);
                     if (rare_or) rareq[atomicAdd(&s_rare_n[rc_build], 1)] = g * 32 + lane;
                 }
             }
@@ -478,7 +440,7 @@ k1_bitsliced(const int32_t *__restrict__ rank, const int64_t *__restrict__ off,
         { const int t = rc_clear; rc_clear = rc_cons; rc_cons = rc_build; rc_build = t; }
     }
     __syncthreads();
-    t_crumbs += bs_flush_rows(tile32, rows, cells, flushed_upto + 1, flushed_upto + rows - 1, W, cnt);
+    t_crumbs += bs_flush_rows(tile32, rows, cells, flushed_upto + 1, flushed_upto + rows - 1, W, cnt, blockDim.x, true);
     if (errbits) atomicOr(err, (int)errbits);
     // covered SNPs (util.py:239) = all codes of the kept reads minus the N and _ among them
     flush_totals(n_slices, t_crumbs + n_rcrumbs, (unsigned long long)n_codes - n_notcov, n_sent, totals);
@@ -508,8 +470,7 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
                 int *__restrict__ err, const int *__restrict__ sorted_flag,
                 const int64_t *__restrict__ run_end) {
     extern __shared__ uint4 smem4[];
-    HxCnt cnt = cnt_in;                              // single-GPU build: the peer path folds away
-    if (!FUSED) { cnt.world = 1; cnt.rows_per = 1; cnt.peer = nullptr; }
+    const HxCnt cnt = cnt_in.for_build<FUSED>();
     __shared__ __align__(8) unsigned long long s_full[WS_NBUF], s_empty[WS_NBUF];
     if (!*sorted_flag) return;                       // the generic fallback launch takes over
     const int rows = kmax + 1, cells = kmax - 1;
@@ -582,7 +543,7 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
                     o = off[idx];
                     const int64_t k64 = off[idx + 1] - o;
                     if (k64 >= 2) {
-                        if (r < 0 || (int64_t)r + k64 > N || k64 - 1 > W) errbits |= 1;
+                        if (!read_fits(r, k64, N, W)) errbits |= 1;
                         else kb = (int)k64;
                     }
                     // last read of the batch: the next batch's codes start right behind it
@@ -591,24 +552,10 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
                 n_slices += kb >= 2;
                 n_codes += kb;
                 uint32_t rare_or, x0;
-                const uint8_t *__restrict__ c = codes + o;
                 const int kg = bs_build_group<KW>(codes, o, kb, planes_saddr + (uint32_t)((b * gb + g) * kmax) * 16u,
                                                   rare_or, x0);
                 if (lane == 0) gk[g] = kg;
-                if (kb >= 2) {
-                    const unsigned a0 = x0 & 0xffu;
-                    if (r == 0 && sym_valid_from(a0)) {            // util.py:262-266
-                        atomicAdd(cnt.cell(W, 0, 1) + HX_SYM_GAP * HX_NSYM + a0, 1u);
-                        n_sent++;
-                    }
-                    if (r + kb == N && !(kb == 2 && r == 0)) {     // util.py:271-275
-                        const unsigned ap = c[kb - 2], bl = c[kb - 1];
-                        if (sym_valid_from(ap) && bl <= 6) {
-                            atomicAdd(cnt.cell(W, N, N + 1) + bl * HX_NSYM + HX_SYM_GAP, 1u);
-                            n_sent++;
-                        }
-                    }
-                }
+                if (kb >= 2) add_sentinels(codes + o, x0 & 0xffu, r, kb, N, W, cnt, n_sent);
                 // reads holding N, - or _: their pairs with such an allele are added right here by the warp
                 unsigned rm = __ballot_sync(0xffffffffu, kb >= 2 && rare_or != 0);
                 while (rm) {
@@ -657,25 +604,9 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
             if (first) {
                 ws_pair_barrier(npt);                // the previous run's tile adds are complete
                 if ((int64_t)r + 1 > flushed_upto) {
-                    const int64_t lastrow = min((int64_t)r + 1, flushed_upto + rows - 2);
                     // rows pj <= r+1 can no longer be touched by this CTA
-                    unsigned long long sum = 0;
-                    const int per_row = cells * 16;
-                    int row = (int)((flushed_upto + 1) % rows);
-                    for (int64_t pj = flushed_upto + 1; pj <= lastrow; ++pj) {
-                        uint32_t *base = tile32 + (size_t)row * per_row;
-                        for (int w = threadIdx.x; w < per_row; w += npt) {
-                            const uint32_t v = base[w];
-                            if (v) {
-                                const int d = (w >> 4) + 1, ab = w & 15;
-                                atomicAdd(cnt.cell(W, pj - d, pj) + (ab >> 2) * HX_NSYM + (ab & 3), v);
-                                base[w] = 0;
-                                sum += v;
-                            }
-                        }
-                        if (++row == rows) row = 0;
-                    }
-                    t_crumbs += sum;
+                    const int64_t lastrow = min((int64_t)r + 1, flushed_upto + rows - 2);
+                    t_crumbs += bs_flush_rows(tile32, rows, cells, flushed_upto + 1, lastrow, W, cnt, npt, true);
                     flushed_upto = (int64_t)r + 1;
                     ws_pair_barrier(npt);            // retired ring slots may be reused by this run's tile add
                 }
@@ -717,24 +648,7 @@ k1_bitsliced_ws(const int32_t *__restrict__ rank, const int64_t *__restrict__ of
             }
         }
         ws_pair_barrier(npt);
-        {
-            unsigned long long sum = 0;
-            const int per_row = cells * 16;
-            int row = (int)((flushed_upto + 1) % rows);
-            for (int64_t pj = flushed_upto + 1; pj <= flushed_upto + rows - 1; ++pj) {
-                uint32_t *base = tile32 + (size_t)row * per_row;
-                for (int w = threadIdx.x; w < per_row; w += npt) {
-                    const uint32_t v = base[w];
-                    if (v) {
-                        const int d = (w >> 4) + 1, ab = w & 15;
-                        atomicAdd(cnt.cell(W, pj - d, pj) + (ab >> 2) * HX_NSYM + (ab & 3), v);
-                        sum += v;
-                    }
-                }
-                if (++row == rows) row = 0;
-            }
-            t_crumbs += sum;
-        }
+        t_crumbs += bs_flush_rows(tile32, rows, cells, flushed_upto + 1, flushed_upto + rows - 1, W, cnt, npt, false);
     }
     if (errbits) atomicOr(err, (int)errbits);
     flush_totals(n_slices, t_crumbs + n_rcrumbs, (unsigned long long)n_codes - n_notcov, n_sent, totals);
@@ -771,9 +685,7 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
     if (n_reads <= 0) return HX_OK;
     const bool presorted = run_end != nullptr;
     if (!presorted) run_end = h->d_run_end.p;
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
+    const int sms = ingest_sm_budget(h);
     int *const verdict = &h->d_flags.p->ingest_sorted;      // the sortedness pre-pass writes its verdict here
     const int *sorted_flag = presorted ? ok : verdict;
     constexpr int GBLOCK = 256;
@@ -790,7 +702,6 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
     // 20 reads per rank 0.25 vs 0.19 ms against the bit-sliced kernel)
     const bool use_umma = use_bs && hx_umma_possible(h) &&
                           (h->use.ingest_kernel == 6 || (h->use.ingest_kernel == 0 && n_reads >= 64 * ((int64_t)h->N + 1)));
-    const bool fused = h->peer_world > 1;
     const bool use_long = !use_bs && (h->use.ingest_kernel == 3 || (h->use.ingest_kernel == 0 && kmax >= 2));
     // long-read tensor-core kernel (ingest_lumma.cu): default for wide reads unless its one-hot scratch would be huge
     const bool use_lumma = kmax >= 2 && (h->use.ingest_kernel == 7 ||
@@ -850,24 +761,15 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
             int gb = BS_GB;
             while (gb > 4 && WsLayout{kmax, gb}.bytes() > (size_t)((np == 1 ? 100 : 200) * 1024)) gb >>= 1;
             const size_t smem = WsLayout{kmax, gb}.bytes();
-#define HX_WS_LAUNCH(KW_, NP_, MAXT_, MINB_)                                                                  \
-    do {                                                                                                       \
-        auto kern = fused ? k1_bitsliced_ws<KW_, NP_, MAXT_, MINB_, true> : k1_bitsliced_ws<KW_, NP_, MAXT_, MINB_, false>; \
-        HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
-        int occ = 1;                                                                                           \
-        HX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, block, smem));                       \
-        if (occ < 1) occ = 1;                                                                                  \
-        int64_t grid = (int64_t)sms * occ;                                                                     \
-        const int64_t max_useful = (n_reads + 255) / 256;                                                      \
-        if (grid > max_useful) grid = max_useful;                                                              \
-        kern<<<(unsigned)grid, block, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax,    \
-                                                         gb, pw, hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag, \
-                                                         run_end);                                        \
-    } while (0)
-            if (np == 2) HX_WS_LAUNCH(14, 2, 1024, 1);
-            else if (kmax > 32) HX_WS_LAUNCH(14, 1, 1024, 1);
-            else HX_WS_LAUNCH(8, 1, 640, 2);
-#undef HX_WS_LAUNCH
+            const auto kern = ingest_kernel_for(h, [&](auto fused_t) {
+                constexpr bool F = decltype(fused_t)::value;
+                return np == 2 ? k1_bitsliced_ws<14, 2, 1024, 1, F>
+                               : kmax > 32 ? k1_bitsliced_ws<14, 1, 1024, 1, F> : k1_bitsliced_ws<8, 1, 640, 2, F>;
+            });
+            unsigned grid;
+            if (int rc = ingest_grid(kern, sms, block, smem, true, n_reads, &grid)) return rc;
+            kern<<<grid, block, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax, gb, pw, hx_cnt_ref(h),
+                                                   h->d_totals.p, h->d_err.p, sorted_flag, run_end);
         } else {
         int gb = BS_GB;
         while (gb > 4 && BsLayout{kmax, gb}.bytes() > (size_t)200 * 1024) gb >>= 1;
@@ -876,24 +778,15 @@ static int launch_ingest(hx_matrix *h, const int32_t *d_rank, const int64_t *d_o
         int block = ((npairs + np - 1) / np + 31) / 32 * 32;
         if (block < 128) block = 128;
         if (block > 1024) block = 1024;
-#define HX_BS_LAUNCH(KW_, NP_, MAXT_, MINB_)                                                                  \
-    do {                                                                                                       \
-        auto kern = fused ? k1_bitsliced<KW_, NP_, MAXT_, MINB_, true> : k1_bitsliced<KW_, NP_, MAXT_, MINB_, false>;       \
-        HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
-        int occ = 1;                                                                                           \
-        HX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, block, smem));                       \
-        if (occ < 1) occ = 1;                                                                                  \
-        int64_t grid = (int64_t)sms * occ;                                                                     \
-        const int64_t max_useful = (n_reads + 255) / 256;   /* no thinner than 256 reads per CTA */            \
-        if (grid > max_useful) grid = max_useful;                                                              \
-        kern<<<(unsigned)grid, block, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax,    \
-                                                         gb, hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag,   \
-                                                         run_end);                                        \
-    } while (0)
-        if (np == 2) HX_BS_LAUNCH(14, 2, 1024, 1);
-        else if (kmax > 32) HX_BS_LAUNCH(14, 1, 1024, 1);
-        else HX_BS_LAUNCH(8, 1, 512, 2);
-#undef HX_BS_LAUNCH
+        const auto kern = ingest_kernel_for(h, [&](auto fused_t) {
+            constexpr bool F = decltype(fused_t)::value;
+            return np == 2 ? k1_bitsliced<14, 2, 1024, 1, F>
+                           : kmax > 32 ? k1_bitsliced<14, 1, 1024, 1, F> : k1_bitsliced<8, 1, 512, 2, F>;
+        });
+        unsigned grid;
+        if (int rc = ingest_grid(kern, sms, block, smem, true, n_reads, &grid)) return rc;
+        kern<<<grid, block, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax, gb, hx_cnt_ref(h),
+                                               h->d_totals.p, h->d_err.p, sorted_flag, run_end);
         }
         h->use.launches++;
         // fallback for unsorted input: runs only when the flag says the bit-sliced kernel declined

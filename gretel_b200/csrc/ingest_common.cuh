@@ -1,6 +1,10 @@
-// Device helpers shared by the ingestion kernels (ingest.cu, ingest_umma.cu): totals, the per-read side path
-// for rare alleles (N, -, _), L2 prefetch and the mbarrier arrive / back-off wait.
+// Helpers shared by the ingestion kernels (ingest.cu, ingest_umma.cu, ingest_lumma.cu, ingest_long.cu): the per-read
+// rules of the reference (which reads count, the sentinels, the valid first allele), totals, the per-read side path
+// for rare alleles (N, -, _), the tile flush, L2 prefetch, the mbarrier arrive / back-off wait, and on the host the
+// launch of the persistent kernels.
 #pragma once
+#include <type_traits>
+
 #include "hx_internal.cuh"
 
 namespace {
@@ -31,6 +35,31 @@ __device__ __forceinline__ void flush_totals(unsigned long long t0, unsigned lon
 
 __device__ __forceinline__ bool sym_valid_from(unsigned a) {   // util.py:258
     return a != HX_SYM_N && a != HX_SYM_GAP && a <= 6;
+}
+
+// A read of k >= 2 SNPs (fewer are skipped, util.py:230) at rank r must lie in [0, N] and fit the band (k <= W + 1);
+// any other is an HX_E_READ error (bit 1).
+__device__ __forceinline__ bool read_fits(int r, int64_t k, int N, int W) {
+    return !(r < 0 || (int64_t)r + k > N || k - 1 > W);
+}
+
+// The start sentinel (util.py:262-266) and the end sentinel (:271-275) of a valid read of k >= 2 SNPs at rank r with
+// codes c and first code a0 = c[0]; a read of two SNPs that is both first and last gets only the start one.  Adds the
+// increments it made to n_sent (the counter is updated in place: returning them cost k_lr_transpose 7 registers).
+template <class Count>
+__device__ __forceinline__ void add_sentinels(const uint8_t *__restrict__ c, unsigned a0, int r, int k, int N,
+                                              int64_t W, const HxCnt cnt, Count &n_sent) {
+    if (r == 0 && sym_valid_from(a0)) {
+        atomicAdd(cnt.cell(W, 0, 1) + HX_SYM_GAP * HX_NSYM + a0, 1u);
+        n_sent++;
+    }
+    if (r + k == N && !(k == 2 && r == 0)) {
+        const unsigned ap = c[k - 2], bl = c[k - 1];
+        if (sym_valid_from(ap) && bl <= 6) {
+            atomicAdd(cnt.cell(W, N, N + 1) + bl * HX_NSYM + HX_SYM_GAP, 1u);
+            n_sent++;
+        }
+    }
 }
 
 
@@ -70,6 +99,33 @@ __device__ __forceinline__ void bs_rare_read(const uint8_t *__restrict__ c, int 
             }
         }
     }
+}
+
+
+// Rows [pj_lo, pj_hi] of a sliding tile (ring of `rows` band rows of cells x 16 counters, row = pj % rows, cell = d-1,
+// 16 = (a,b) in ACGT x ACGT), by the nthreads threads that call it: adds every non-zero counter to HBM and, with
+// zero, clears it; returns the sum flushed by this thread (every regular-cell increment is one crumb,
+// util.py:268,276,281).
+__device__ __forceinline__ unsigned long long bs_flush_rows(uint32_t *tile32, int rows, int cells, int64_t pj_lo,
+                                                            int64_t pj_hi, int64_t W, const HxCnt cnt, unsigned nthreads,
+                                                            bool zero) {
+    unsigned long long sum = 0;
+    const int per_row = cells * 16;
+    int row = (int)(pj_lo % rows);
+    for (int64_t pj = pj_lo; pj <= pj_hi; ++pj) {
+        uint32_t *base = tile32 + (size_t)row * per_row;
+        for (int w = threadIdx.x; w < per_row; w += nthreads) {
+            const uint32_t v = base[w];
+            if (v) {
+                const int d = (w >> 4) + 1, ab = w & 15;
+                atomicAdd(cnt.cell(W, pj - d, pj) + (ab >> 2) * HX_NSYM + (ab & 3), v);
+                if (zero) base[w] = 0;
+                sum += v;
+            }
+        }
+        if (++row == rows) row = 0;
+    }
+    return sum;
 }
 
 
@@ -141,6 +197,40 @@ __device__ __forceinline__ void ws_mbar_wait_sleep(uint32_t bar, uint32_t parity
 }
 __device__ __forceinline__ void ws_pair_barrier(int nthreads) {
     asm volatile("bar.sync 1, %0;" ::"r"(nthreads) : "memory");
+}
+
+
+// ---- host --------------------------------------------------------------------------------------------------
+
+// SMs the persistent ingestion kernels may use: all of the device's, or fewer when the matrix is told so (ingest_sms).
+inline int ingest_sm_budget(const hx_matrix *h) {
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
+    if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
+    return sms;
+}
+
+// The instantiation of a kernel templated on FUSED that serves this matrix: pick(std::true_type) when its counts go
+// to the GPUs of the fused multi-GPU exchange, pick(std::false_type) otherwise (see HxCnt::for_build).
+template <class Pick>
+auto ingest_kernel_for(const hx_matrix *h, Pick pick) {
+    return h->peer_world > 1 ? pick(std::true_type{}) : pick(std::false_type{});
+}
+
+// Prepares a persistent ingestion kernel for a launch with `block` threads and `smem` bytes of dynamic shared memory
+// and sets *grid: one CTA per SM of the budget (with `occupancy`, as many as fit on an SM), but no CTA thinner than
+// 256 reads.
+template <class Kern>
+int ingest_grid(Kern kern, int sms, int block, size_t smem, bool occupancy, int64_t n_reads, unsigned *grid) {
+    HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int occ = 1;
+    if (occupancy) {
+        HX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, block, smem));
+        if (occ < 1) occ = 1;
+    }
+    const int64_t max_useful = (n_reads + 255) / 256;
+    *grid = (unsigned)std::min((int64_t)sms * occ, max_useful);
+    return HX_OK;
 }
 
 

@@ -16,13 +16,12 @@
 #include <limits.h>
 
 #include "hx_internal.cuh"
+#include "ingest_common.cuh"
 #include "scan.cuh"
 
 namespace {
 
 constexpr int LR_TI = 16, LR_TJ = 32;
-
-__device__ __forceinline__ bool lr_valid_from(unsigned a) { return a != HX_SYM_N && a != HX_SYM_GAP && a <= 6; }
 
 // ---- group frames ------------------------------------------------------------------------
 __global__ void k_lr_frames(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, int64_t n_reads,
@@ -38,7 +37,7 @@ __global__ void k_lr_frames(const int32_t *__restrict__ rank, const int64_t *__r
         const int64_t k = off[idx + 1] - off[idx];
         const int r = rank[idx];
         if (k >= 2) {
-            if (r < 0 || (int64_t)r + k > N || k - 1 > W) atomicOr(err, 1);
+            if (!read_fits(r, k, N, W)) atomicOr(err, 1);
             else { lo = r; hi = r + (int)k; }
         }
     }
@@ -68,10 +67,7 @@ k_lr_transpose(const int32_t *__restrict__ rank, const int64_t *__restrict__ off
                const int64_t *__restrict__ g_off, uint4 *__restrict__ planes, const HxCnt cnt,
                unsigned long long *__restrict__ totals, int *__restrict__ err,
                const int *__restrict__ sorted_flag) {
-    __shared__ unsigned long long sh_tot[4];
     if (!*sorted_flag) return;                       // the generic fallback launch takes over
-    if (threadIdx.x < 4) sh_tot[threadIdx.x] = 0;
-    __syncthreads();
     const int lane = threadIdx.x & 31;
     const int64_t n_groups = (n_reads + 31) >> 5;
     const int64_t gstride = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -84,7 +80,7 @@ k_lr_transpose(const int32_t *__restrict__ rank, const int64_t *__restrict__ off
             o = off[idx];
             const int64_t k64 = off[idx + 1] - o;
             r = rank[idx];
-            if (k64 >= 2 && r >= 0 && (int64_t)r + k64 <= N && k64 - 1 <= W) k = (int)k64;
+            if (k64 >= 2 && read_fits(r, k64, N, W)) k = (int)k64;
         }
         t_slices += k >= 2;
         const int lo = g_lo[g];
@@ -113,21 +109,7 @@ k_lr_transpose(const int32_t *__restrict__ rank, const int64_t *__restrict__ off
             t_cov += (a < 4 || a == 5);
             has_gap |= (a == 6);
         }
-        if (k >= 2) {
-            // start sentinel (util.py:262-266) / end sentinel (:271-275); the start rule wins
-            const unsigned a0 = c[0];
-            if (r == 0 && lr_valid_from(a0)) {
-                atomicAdd(cnt.cell(W, 0, 1) + HX_SYM_GAP * HX_NSYM + a0, 1u);
-                t_sent++;
-            }
-            if (r + k == N && !(k == 2 && r == 0)) {
-                const unsigned ap = c[k - 2], bl = c[k - 1];
-                if (lr_valid_from(ap) && bl <= 6) {
-                    atomicAdd(cnt.cell(W, N, N + 1) + bl * HX_NSYM + HX_SYM_GAP, 1u);
-                    t_sent++;
-                }
-            }
-        }
+        if (k >= 2) add_sentinels(c, c[0], r, k, N, W, cnt, t_sent);
         // '_' as the second allele of a pair is counted (util.py:258 only rejects it as the first);
         // it has no bit-plane: the warp walks such reads position by position
         unsigned gm = __ballot_sync(0xffffffffu, has_gap);
@@ -142,7 +124,7 @@ k_lr_transpose(const int32_t *__restrict__ rank, const int64_t *__restrict__ off
                 if (c2[j] != HX_SYM_GAP) continue;          // uniform: every lane reads the same byte
                 for (int i = lane; i < j; i += 32) {
                     const unsigned a = c2[i];
-                    if (lr_valid_from(a)) {
+                    if (sym_valid_from(a)) {
                         atomicAdd(cnt.cell(W, r2 + i + 1, r2 + j + 1) + a * HX_NSYM + HX_SYM_GAP, 1u);
                         t_crumbs++;
                     }
@@ -150,21 +132,7 @@ k_lr_transpose(const int32_t *__restrict__ rank, const int64_t *__restrict__ off
             }
         }
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        t_slices += __shfl_xor_sync(0xffffffffu, t_slices, o);
-        t_cov += __shfl_xor_sync(0xffffffffu, t_cov, o);
-        t_sent += __shfl_xor_sync(0xffffffffu, t_sent, o);
-        t_crumbs += __shfl_xor_sync(0xffffffffu, t_crumbs, o);
-    }
-    if (lane == 0) {
-        if (t_slices) atomicAdd(&sh_tot[0], t_slices);
-        if (t_crumbs) atomicAdd(&sh_tot[1], t_crumbs);
-        if (t_cov) atomicAdd(&sh_tot[2], t_cov);
-        if (t_sent) atomicAdd(&sh_tot[3], t_sent);
-    }
-    __syncthreads();
-    if (threadIdx.x < 4 && sh_tot[threadIdx.x]) atomicAdd(&totals[threadIdx.x], sh_tot[threadIdx.x]);
+    flush_totals(t_slices, t_crumbs, t_cov, t_sent, totals);
 }
 
 // per site s: first group whose running-max end exceeds s (some read so far reaches s), and the

@@ -76,7 +76,7 @@ k_l2_keys(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, int
     const int r = rank[i];
     int key = -1;
     if (k >= 2) {                                                                    // util.py:230
-        if (r < 0 || (int64_t)r + k > g.N || k - 1 > g.W) atomicOr(err, 1);
+        if (!read_fits(r, k, g.N, g.W)) atomicOr(err, 1);
         else {
             const int sb = (r + 1) >> 4, eb = (r + (int)k) >> 4;
             key = sb * g.SPB() + 1 + (eb - sb);
@@ -137,21 +137,7 @@ k_l2_onehot(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, c
         const int eb = __reduce_max_sync(0xffffffffu, idx >= 0 ? (r + k) >> 4 : 0);
         if (lane == 0) chunk_eb[c] = eb;
         t_slices += idx >= 0;
-        if (k >= 2) {
-            // start sentinel (util.py:262-266) / end sentinel (:271-275); the start rule wins
-            const unsigned a0 = cd[0];
-            if (r == 0 && sym_valid_from(a0)) {
-                atomicAdd(cnt.cell(g.W, 0, 1) + HX_SYM_GAP * HX_NSYM + a0, 1u);
-                t_sent++;
-            }
-            if (r + k == g.N && !(k == 2 && r == 0)) {
-                const unsigned ap = cd[k - 2], bl = cd[k - 1];
-                if (sym_valid_from(ap) && bl <= 6) {
-                    atomicAdd(cnt.cell(g.W, g.N, g.N + 1) + bl * HX_NSYM + HX_SYM_GAP, 1u);
-                    t_sent++;
-                }
-            }
-        }
+        if (k >= 2) add_sentinels(cd, cd[0], r, k, g.N, g.W, cnt, t_sent);
     }
     flush_totals(t_slices, 0, 0, t_sent, totals);
 }
@@ -354,8 +340,7 @@ k_l2_tiles(const uint8_t *__restrict__ onehot, const int32_t *__restrict__ bstar
     __shared__ volatile int s_tile[2][4];             // (I, q, halves present, exit) of the tile in each accumulator
     __shared__ uint32_t s_tmem;
     if (go && !*go) return;
-    HxCnt cnt = cnt_in;
-    if (!FUSED) { cnt.world = 1; cnt.rows_per = 1; cnt.peer = nullptr; }
+    const HxCnt cnt = cnt_in.for_build<FUSED>();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t stage0 = hx_smem_u32(l2_smem);
     uint32_t *const staging = reinterpret_cast<uint32_t *>(l2_smem + (size_t)L2_STAGES * L2_STAGE_BYTES);
@@ -651,8 +636,7 @@ k_l2_tiles2(const uint8_t *__restrict__ onehot, const uint8_t *__restrict__ zero
     __shared__ volatile int s_tile[2][4];
     __shared__ uint32_t s_tmem;
     if (go && !*go) return;                              // (uniform over the cluster)
-    HxCnt cnt = cnt_in;
-    cnt.world = 1; cnt.rows_per = 1; cnt.peer = nullptr;
+    const HxCnt cnt = cnt_in.for_build<false>();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     uint32_t rank;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
@@ -990,9 +974,7 @@ int hx_launch_ingest_lumma(hx_matrix *h, const int32_t *d_rank, const int64_t *d
                                                                            h->d_totals.p, h->d_err.p, go);
     k_l2_slabs<<<dim3((unsigned)max_chunks, (unsigned)((g.SP + 7) / 8)), 256, 0, st>>>(d_rank, d_off, d_codes, s->perm.p, s->bstart.p, g,
                                                                                      s->onehot.p, h->d_totals.p, h->d_err.p, go);
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
+    const int sms = ingest_sm_budget(h);
     const bool fused = h->peer_world > 1;
     const bool fresh = !fused && h->use.cnt_fresh;
     static const bool pairs_on = getenv("HX_LUMMA_PAIRS") && !strcmp(getenv("HX_LUMMA_PAIRS"), "1");
@@ -1007,7 +989,10 @@ int hx_launch_ingest_lumma(hx_matrix *h, const int32_t *d_rank, const int64_t *d
         h->use.launches++;
     } else {
         const size_t smem = (size_t)L2_STAGES * L2_STAGE_BYTES + (size_t)L2_EP_WARPS * L2_STG_WORDS * 4 + 1024;
-        auto kern = fused ? k_l2_tiles<true, false> : (fresh ? k_l2_tiles<false, true> : k_l2_tiles<false, false>);
+        const auto kern = ingest_kernel_for(h, [&](auto fused_t) {
+            constexpr bool F = decltype(fused_t)::value;
+            return fresh ? k_l2_tiles<false, true> : k_l2_tiles<F, false>;      // fresh: a single-GPU build only
+        });
         HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<sms, L2_THREADS, smem, st>>>(s->onehot.p, s->bstart.p, g, hx_cnt_ref(h), h->d_totals.p, go);
     }

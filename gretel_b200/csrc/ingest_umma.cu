@@ -259,8 +259,7 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
         int jobs_cap, int read_w, int rank_w) {
     extern __shared__ __align__(1024) uint8_t um_smem[];
     UM_T(k_begin);
-    HxCnt cnt = cnt_in;                              // single-GPU build: the peer path folds away
-    if (!FUSED) { cnt.world = 1; cnt.rows_per = 1; cnt.peer = nullptr; }
+    const HxCnt cnt = cnt_in.for_build<FUSED>();
     __shared__ __align__(8) unsigned long long s_slot[UM_EXP_WARPS];   // a warp's operand slot has been read by its MMA
     __shared__ __align__(8) unsigned long long s_acc_full[UM_NACC];    // all MMAs of a run are complete
     __shared__ int s_runkg[UM_NACC];                       // widest read of the run accumulating in each stage
@@ -450,13 +449,11 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
             const int r = cur.z;
             const unsigned cur_ri = (unsigned)cur.w;
             const int s = cur_ri % UM_NACC;
-            // SNPs on my read: 0 for a lane past the run's end or a read with fewer than two; a read that leaves
-            // [0, N] or is wider than the band is an error (the same test as the other kernels)
-            const uint64_t kd = (uint64_t)(o1 - o);
-            const int klim = min(W + 1, N - r);                     // warp-uniform
+            // SNPs on my read: 0 for a lane past the run's end or a read with fewer than two
+            const int64_t kd = o1 - o;
             int kb = 0;
-            if (kd >= 2) {
-                if (r < 0 || kd > (uint64_t)(klim < 0 ? 0 : klim)) errbits |= 1;
+            if ((uint64_t)kd >= 2) {                                // offsets that decrease (kd < 0) are an error too
+                if (kd < 0 || !read_fits(r, kd, N, W)) errbits |= 1;
                 else kb = (int)kd;
             }
             n_slices += kb >= 2;
@@ -493,21 +490,7 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
             ++njobs;
             UM_T(tG);
             if (r == 0 || r + kg >= N) {                            // warp-uniform: runs at the ends of the region
-                if (kb >= 2) {
-                    const uint8_t *__restrict__ c = codes + o;
-                    const unsigned a0 = x0 & 0xffu;
-                    if (r == 0 && sym_valid_from(a0)) {            // util.py:262-266
-                        atomicAdd(cnt.cell(W, 0, 1) + HX_SYM_GAP * HX_NSYM + a0, 1u);
-                        n_sent++;
-                    }
-                    if (r + kb == N && !(kb == 2 && r == 0)) {     // util.py:271-275
-                        const unsigned ap = c[kb - 2], bl = c[kb - 1];
-                        if (sym_valid_from(ap) && bl <= 6) {
-                            atomicAdd(cnt.cell(W, N, N + 1) + bl * HX_NSYM + HX_SYM_GAP, 1u);
-                            n_sent++;
-                        }
-                    }
-                }
+                if (kb >= 2) add_sentinels(codes + o, x0 & 0xffu, r, kb, N, W, cnt, n_sent);
             }
             // reads holding N, - or _: their pairs with such an allele are added right here by the warp
             unsigned rm = __ballot_sync(0xffffffffu, kb >= 2 && rare_or != 0);
@@ -618,23 +601,7 @@ k1_umma(const int32_t *__restrict__ rank, const int64_t *__restrict__ off, const
             UM_T(r3);
             UM_ACC(0, r1 - r0); UM_ACC(1, r2 - r1); UM_ACC(2, r3 - r2); UM_ACC(3, 1);
         }
-        {
-            unsigned long long sum = 0;
-            int row = (int)((flushed_upto + 1) % rows);
-            for (int64_t pj = flushed_upto + 1; pj <= flushed_upto + rows - 1; ++pj) {
-                uint32_t *base = tile32 + (size_t)row * per_row;
-                for (int w = threadIdx.x; w < per_row; w += npt) {
-                    const uint32_t v = base[w];
-                    if (v) {
-                        const int d = (w >> 4) + 1, ab = w & 15;
-                        atomicAdd(cnt.cell(W, pj - d, pj) + (ab >> 2) * HX_NSYM + (ab & 3), v);
-                        sum += v;
-                    }
-                }
-                if (++row == rows) row = 0;
-            }
-            t_crumbs += sum;
-        }
+        t_crumbs += bs_flush_rows(tile32, rows, cells, flushed_upto + 1, flushed_upto + rows - 1, W, cnt, npt, false);
 #ifdef UM_PROFILE
         if (threadIdx.x == 0) for (int i = 0; i < 4; ++i) atomicAdd(&um_prof[16 + i], prof_acc[i]);
 #endif
@@ -684,15 +651,14 @@ bool hx_umma_possible(const hx_matrix *h) {
 // rank-sorted reads of at most 32 SNPs; run_end must hold -1 for ranks without reads (hx_launch_ingest fills it)
 int hx_launch_ingest_umma(hx_matrix *h, const int32_t *d_rank, const int64_t *d_off, const uint8_t *d_codes,
                           int64_t n_reads, const int64_t *run_end, const int *sorted_flag) {
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    if (h->use.ingest_sms > 0 && h->use.ingest_sms < sms) sms = h->use.ingest_sms;
     const int kmax = h->W + 1;
-    const bool fused = h->peer_world > 1;
     const size_t smem = UmLayout{kmax}.bytes();
-    int64_t grid = sms;
-    const int64_t max_useful = (n_reads + 255) / 256;          // no thinner than 256 reads per CTA
-    if (grid > max_useful) grid = max_useful;
+    const auto kern = ingest_kernel_for(h, [&](auto fused_t) {
+        constexpr bool F = decltype(fused_t)::value;
+        return kmax <= 16 ? k1_umma<4, F> : k1_umma<8, F>;
+    });
+    unsigned grid;
+    if (int rc = ingest_grid(kern, ingest_sm_budget(h), UM_THREADS, smem, false, n_reads, &grid)) return rc;
     int32_t *run_rank = reinterpret_cast<int32_t *>(h->d_run_list.p);
     int64_t *run_stop = reinterpret_cast<int64_t *>(h->d_run_list.p) + (((size_t)h->N + 2 + 1) / 2);
     int *n_runs = reinterpret_cast<int *>(run_stop + (size_t)h->N + 2);
@@ -710,18 +676,9 @@ int hx_launch_ingest_umma(hx_matrix *h, const int32_t *d_rank, const int64_t *d_
     HX_CHECK_ARG(jobs_cap < ((int64_t)1 << 31) && per < ((int64_t)1 << 31));
     const int64_t jobs_bytes = jobs_cap * grid * (int64_t)sizeof(int4);
     if (jobs_bytes > h->d_jobs.cap) HX_CUDA(h->d_jobs.grow(jobs_bytes + jobs_bytes / 8, h->stream));   // with headroom
-#define HX_UM_LAUNCH(CH_)                                                                                       \
-    do {                                                                                                        \
-        auto kern = fused ? k1_umma<CH_, true> : k1_umma<CH_, false>;                                           \
-        HX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-        kern<<<(unsigned)grid, UM_THREADS, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax, \
-                                                              hx_cnt_ref(h), h->d_totals.p, h->d_err.p, sorted_flag, \
-                                                              run_rank, run_stop, n_runs,                       \
-                                                              h->d_jobs.p, (int)jobs_cap, read_w, rank_w); \
-    } while (0)
-    if (kmax <= 16) HX_UM_LAUNCH(4);
-    else HX_UM_LAUNCH(8);
-#undef HX_UM_LAUNCH
+    kern<<<grid, UM_THREADS, smem, h->stream>>>(d_rank, d_off, d_codes, n_reads, h->N, h->W, kmax, hx_cnt_ref(h),
+                                                h->d_totals.p, h->d_err.p, sorted_flag, run_rank, run_stop, n_runs,
+                                                h->d_jobs.p, (int)jobs_cap, read_w, rank_w);
     h->use.launches++;
     HX_CUDA(cudaGetLastError());
     return HX_OK;

@@ -425,12 +425,8 @@ int hx_ingest_host_pipelined(hx_matrix *h, const int32_t *rank, const int64_t *o
     int64_t a = 0;
     static thread_local HxDensePlan plan;             // keeps its list buffers between chunks and calls
     for (int c = 0; c < n_chunks; ++c) {
-        int64_t b = n_reads;
-        if (c + 1 < n_chunks) {
-            const int64_t target = off[0] + n_codes * (c + 1) / n_chunks;
-            b = std::lower_bound(off + a, off + n_reads, target) - off;
-            if (b <= a) continue;
-        }
+        const int64_t b = hx_chunk_end(off, a, n_reads, n_codes, c, n_chunks);
+        if (b <= a && c + 1 < n_chunks) continue;
         HxDensePlan &P = plan;
         int rc = hx_dense_begin(off + a, b - a, nt, (int64_t)h->W + 1, &P, slim);
         if (rc) return rc;
