@@ -670,8 +670,11 @@ int hx_launch_ingest_umma(hx_matrix *h, const int32_t *d_rank, const int64_t *d_
     // share of the reads (plus the rank term's share)
     static const int read_w = [] { const char *e = getenv("HX_UM_READ_W"); const int v = e ? atoi(e) : HX_SLICE_READ_W; return v < 1 ? 1 : v; }();
     static const int rank_w = [] { const char *e = getenv("HX_UM_RANK_W"); const int v = e ? atoi(e) : HX_SLICE_RANK_W; return v < 0 ? 0 : v; }();
-    // per-CTA job tables: a slice of `per` reads holds at most per/32 full groups plus one partial group per run
-    const int64_t per = (((n_reads + grid - 1) / grid + 1) * (kmax + read_w) + ((int64_t)rank_w * (h->N + 2) + grid - 1) / grid) / read_w + 2;
+    // per-CTA job tables: a slice of `per` reads holds at most per/32 full groups plus one partial group per run.  No
+    // slice holds more than all the reads: where the rank term dominates (few CTAs, many sites, a large rank_w) the
+    // weight bound alone reaches hundreds of GB of tables
+    const int64_t per_w = (((n_reads + grid - 1) / grid + 1) * (kmax + read_w) + ((int64_t)rank_w * (h->N + 2) + grid - 1) / grid) / read_w + 2;
+    const int64_t per = std::min(per_w, n_reads);
     const int64_t jobs_cap = per / 32 + std::min<int64_t>((int64_t)h->N + 2, per) + 2;
     HX_CHECK_ARG(jobs_cap < ((int64_t)1 << 31) && per < ((int64_t)1 << 31));
     const int64_t jobs_bytes = jobs_cap * grid * (int64_t)sizeof(int4);
