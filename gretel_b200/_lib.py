@@ -58,6 +58,7 @@ SIGNATURES = {
     "hx_reweight_path": (_int, [_p, _p, _dbl, C.POINTER(_dbl)]),
     "hx_recover": (_int, [_p, _p, _i32, _int, _i32, _dbl, _p, _p, C.POINTER(_i32)]),
     "hx_assign_reads": (_int, [_p, _p, _i32, _p, _p, _p, _i64, _i32, _p, _p, _p, _p, _p, _p, _p]),
+    "hx_score_paths": (_int, [_p, _p, _i32, _i32, _int, _p, _p, _p, _p, _p, _p, _p]),
     "hx_pack_bam": (_int, [C.c_char_p, C.c_char_p, _i32, _i32, _p, _i32, _int, _int, _p]),
     "hx_pack_bam_ex": (_int, [C.c_char_p, C.c_char_p, _i32, _i32, _p, _i32, _int, _int, _i32, _p, _p]),
     "hx_pack_free": (None, [_p]),

@@ -7,7 +7,7 @@ import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_HERE)
-SOURCES = ["api.cu", "ingest.cu", "ingest_umma.cu", "ingest_long.cu", "ingest_lumma.cu", "recover.cu", "wire.cu", "probe.cu", "coverage.cu", "support.cu", "bampack.cpp"]
+SOURCES = ["api.cu", "ingest.cu", "ingest_umma.cu", "ingest_long.cu", "ingest_lumma.cu", "recover.cu", "wire.cu", "probe.cu", "coverage.cu", "support.cu", "score.cu", "bampack.cpp"]
 LIB_PATH = os.path.join(_HERE, "libhanselx.so")
 
 NVCC_FLAGS = [

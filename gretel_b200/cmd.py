@@ -6,7 +6,8 @@ Everything that computes (ingestion, gap check counts, recovery, reweighting) ru
 library; this file is host-side bookkeeping and output formatting only: PATHS de-duplication
 (cmd.py:164-179), out.fasta / snp.fasta (cmd.py:181-221) and gretel.crumbs (cmd.py:223-240,
 docs/protocol.rst:48-77), and with --support the reads carried by each haplotype (gretel.support, no reference
-counterpart).
+counterpart); with --site-weights / --score the branch weights of every recovered haplotype and of known sequences,
+site by site (gretel.sites, gretel.scores, no reference counterpart).
 """
 from __future__ import annotations
 
@@ -34,6 +35,22 @@ def read_first_fasta_record(path):
     return "".join(seq)
 
 
+def read_fasta_records(path):
+    """Every record of a FASTA file as (name, sequence); the name is the header up to the first whitespace."""
+    records, name, seq = [], None, []
+    with open(path) as fh:
+        for line in fh:
+            if line.startswith(">"):
+                if name is not None:
+                    records.append((name, "".join(seq)))
+                name, seq = (line[1:].split() or [""])[0], []
+            elif name is not None:
+                seq.append(line.strip())
+    if name is not None:
+        records.append((name, "".join(seq)))
+    return records
+
+
 def build_parser():
     p = argparse.ArgumentParser(prog="gretel", description="Gretel: A metagenomic haplotyper (B200 hot path).")
     p.add_argument("bam")
@@ -56,6 +73,13 @@ def build_parser():
                    help="write gretel.support: the reads each recovered haplotype carries")
     p.add_argument("--max-mismatch", type=int, default=-1,
                    help="--support: a read whose best haplotype has more mismatches is not assigned (-1: no limit)")
+    p.add_argument("--site-weights", action="store_true",
+                   help="write gretel.sites: per recovered haplotype and site the branch weights of its allele, of "
+                        "the best candidate and of the runner-up; and gretel.scores: per haplotype its log "
+                        "likelihood, unsupported sites and sites where another allele is preferred")
+    p.add_argument("--score", default=None, metavar="FASTA",
+                   help="also score every record of FASTA (same coordinates as --master) against the evidence, in "
+                        "gretel.scores (and gretel.sites with --site-weights)")
     p.add_argument("--version", action="version", version="%(prog)s " + __version__)
     return p
 
@@ -110,6 +134,34 @@ def write_support(dirn, records, totals):
                                                  r["share"] / totals["assigned"] if totals["assigned"] else 0.0))
 
 
+def write_scores(dirn, hansel, vcf_h, scored, site_weights):
+    """gretel.scores: per scored path (recovered ones by i_0, then FASTA records by name) loglik, unsupported sites
+    and sites whose best candidate is not the path's allele.  With site_weights, gretel.sites: per path and site
+    the site, its position, the path's allele, its weight, the best candidate (. if none), its weight and the largest
+    weight of the candidates other than the path's allele.  `scored`: (keys, paths uint8 [H][N+1], PathScores)
+    blocks as gretel.score_paths / score_sequences return them.  Weights are written in full precision (repr)."""
+    dirn = dirn.rstrip("/") + "/"
+    with open(dirn + "gretel.scores", "w") as fh:
+        fh.write("#id\tloglik\tn_unsupported\tn_disagree\n")
+        for keys, _, sc in scored:
+            for j, k in enumerate(keys):
+                fh.write("%s\t%r\t%d\t%d\n" % (k, float(sc.loglik[j]), sc.n_unsupported[j], sc.n_disagree[j]))
+    if not site_weights:
+        return
+    sym = hansel.symbols
+    with open(dirn + "gretel.sites", "w") as fh:
+        fh.write("#id\tsite\tpos\tallele\tw_hap\tbest\tw_best\tw_second\n")
+        for keys, paths, sc in scored:
+            for j, k in enumerate(keys):
+                for s in range(1, vcf_h["N"] + 1):
+                    b = int(sc.best[j, s - 1])
+                    none = b == sc.NO_CANDIDATE
+                    fh.write("%s\t%d\t%d\t%s\t%r\t%s\t%r\t%r\n" % (
+                        k, s, vcf_h["snp_rev"][s - 1], sym[paths[j][s]], float(sc.w_hap[j, s - 1]),
+                        "." if none else sym[b], 0.0 if none else float(sc.weights[j, s - 1, b]),
+                        float(sc.w_second[j, s - 1])))
+
+
 def main(argv=None):
     args = build_parser().parse_args(argv)
     if args.end == -1:
@@ -133,13 +185,20 @@ def main(argv=None):
         return 1
     if not args.quiet:
         snp_table(hansel, vcf_h)
-    _, PATHS = gretel.recover(hansel, vcf_h["N"], max_paths=args.paths, min_remove=0.01)
+    original = hansel.copy()                      # what recovery starts from: paths are scored against it
+    _, PATHS = gretel.recover(hansel, vcf_h["N"], max_paths=args.paths, min_remove=0.01, original_hansel=original)
     write_outputs(args.out, PATHS, hansel, vcf_h, args.start, args.end, master=args.master,
                   gapchar=args.gapchar, delchar=args.delchar)
     if args.support:
         records, totals = gretel.read_support(hansel, PATHS, reads["rank"], reads["off"], reads["codes"],
                                               max_mismatch=args.max_mismatch)
         write_support(args.out, records, totals)
+    if args.site_weights or args.score:
+        scored = [gretel.score_paths(original, PATHS, weights=args.site_weights)]
+        if args.score:
+            scored.append(gretel.score_sequences(original, vcf_h, read_fasta_records(args.score),
+                                                 delchar=args.delchar, weights=args.site_weights))
+        write_scores(args.out, original, vcf_h, [s for s in scored if s[0]], args.site_weights)
     return 0
 
 

@@ -141,6 +141,7 @@ void free_all(hx_matrix *h) {
     hx_l2_free(h);
     hx_wire_free(h);
     hx_support_free(h);
+    hx_score_free(h);
     if (h->d_peer_tbl) cudaFree(h->d_peer_tbl);
     cudaStream_t st = h->stream;
     h->band.release(st);
@@ -777,7 +778,7 @@ int hx_to_dense(hx_matrix *h, float *out) {
 }
 
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms) {
-    HX_CHECK_ARG(h && ms && which >= 0 && which < 4);
+    HX_CHECK_ARG(h && ms && which >= 0 && which < 5);
     *ms = h->use.last_ms[which];
     return HX_OK;
 }

@@ -72,7 +72,7 @@ struct hx_dev_flags {
     int ingest_sorted;               // ingestion: the pre-pass verdict, non-zero = reads sorted by rank
     int fallback_go;                 // ingestion: non-zero = the counting-sort fallback runs
     uint32_t counts_max;             // hx_counts_max
-    int pad;
+    int score_err;                   // path scoring: a haplotype code > 6 at a site, or not '_' at site 0
 };
 static_assert(sizeof(hx_dev_flags) == 8 * sizeof(int), "hx_dev_flags is one int[8]");
 
@@ -140,6 +140,9 @@ struct hx_matrix {
     HxDevBuf<uint8_t> a_haps; HxDevBuf<uint4> a_planes; HxDevBuf<unsigned long long> a_sums;
     HxDevBuf<int32_t> a_rank; HxDevBuf<int64_t> a_off; HxDevBuf<uint8_t> a_codes; HxDevBuf<int32_t> a_best;
     cudaEvent_t a_ev[2];             // times the assignment kernels (hx_last_kernel_ms which = 3)
+    // path scoring (score.cu): haplotype codes, per-site outputs of one chunk of haplotypes, per-haplotype sums
+    HxDevBuf<uint8_t> sc_haps, sc_best; HxDevBuf<double> sc_site, sc_ll; HxDevBuf<int32_t> sc_cnt;
+    cudaEvent_t sc_ev[2];            // times the scoring kernels (hx_last_kernel_ms which = 4)
     void *h_pinned;                  // small host buffer for D2H of scalars
     void *lr_scratch;                // long-read ingestion scratch (ingest_long.cu)
     void *l2_scratch;                // long-read tensor-core ingestion scratch (ingest_lumma.cu)
@@ -156,7 +159,7 @@ struct hx_matrix {
         bool prepass_ran = false;    // d_flags->ingest_sorted holds the sortedness verdict of the last ingestion launch
         int wire_next = 0;           // the next staging set of the dense wire format
         bool sum_busy[2] = {};       // sum_done[b] marks ordered sums not yet joined into the main stream
-        float last_ms[4] = {};
+        float last_ms[5] = {};
     } use;
 };
 
@@ -279,3 +282,5 @@ void hx_l2_free(hx_matrix *h);
 int hx_ensure_counts(hx_matrix *h);
 // support.cu
 void hx_support_free(hx_matrix *h);
+// score.cu
+void hx_score_free(hx_matrix *h);

@@ -106,3 +106,40 @@ def read_support(hansel, PATHS, rank, off, codes, max_mismatch=-1):
     records = [{"i_0": PATHS[k]["i_0"], "unique": int(res.unique[j]), "shared": int(res.shared[j]),
                 "share": float(res.share[j]), "share_q32": int(res.share_q32[j])} for j, k in enumerate(keys)]
     return records, totals
+
+
+def score_paths(hansel, PATHS, weights=False):
+    """Score the distinct recovered paths of ``PATHS`` in ``i_0`` order (the order of out.fasta) against ``hansel``
+    (Hansel.score_paths).  Score against the matrix recovery started from (``original_hansel``): recovery reweights
+    the matrix it walks.  Returns (i_0 list, paths uint8 [H][N+1], PathScores); ([], None, None) without a path."""
+    keys = sorted(PATHS, key=lambda x: PATHS[x]["i_0"])
+    if not keys:
+        return [], None, None
+    paths = np.stack([hansel.encode_path(PATHS[k]["hansel_path"]) for k in keys])
+    return [PATHS[k]["i_0"] for k in keys], paths, hansel.score_paths(paths, weights=weights)
+
+
+def sequence_path(seq, vcf_h, delchar=""):
+    """A known sequence (same coordinates as --master) as a path: '_', then per site j the character at 1-based
+    position snp_rev[j] - A, C, G or T (either case) as itself, ``delchar`` (if not empty) as '-', anything else,
+    or a position past the end of the sequence, as N.  -> uint8 [N+1]."""
+    code = {"A": 0, "C": 1, "G": 2, "T": 3}
+    out = np.full(vcf_h["N"] + 1, 4, dtype=np.uint8)
+    out[0] = 6
+    for j in range(vcf_h["N"]):
+        pos = vcf_h["snp_rev"][j]
+        ch = seq[pos - 1] if 1 <= pos <= len(seq) else ""
+        if delchar and ch == delchar:
+            out[j + 1] = 5
+        else:
+            out[j + 1] = code.get(ch.upper(), 4)
+    return out
+
+
+def score_sequences(hansel, vcf_h, fasta_records, delchar="", weights=False):
+    """Score known sequences ((name, sequence) pairs, e.g. reference strains from a panel) as paths (sequence_path)
+    against ``hansel``.  Returns (names, paths uint8 [H][N+1], PathScores); ([], None, None) without a record."""
+    if not fasta_records:
+        return [], None, None
+    paths = np.stack([sequence_path(seq, vcf_h, delchar) for _, seq in fasta_records])
+    return [name for name, _ in fasta_records], paths, hansel.score_paths(paths, weights=weights)

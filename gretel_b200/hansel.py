@@ -47,6 +47,23 @@ class ReadSupport:
         self.best_mm, self.n_best, self.first_best = best_mm, n_best, first_best
 
 
+class PathScores:
+    """What Hansel.score_paths reports for H haplotypes over sites 1..N; per-site arrays are [H][N], site s at
+    column s-1.  ``weights`` float64 [H][N][8] (the 7 normalised branch weights of Hansel.get_edge_weights_at at the
+    site given the haplotype's earlier alleles, 0 for a non-candidate, then the total) or None; ``w_hap`` the weight
+    of the haplotype's own allele (0 if it is not a candidate); ``w_second`` the largest weight of the other
+    candidates (0 if none); ``best`` uint8 the first-max candidate, the allele the recovery walk would pick there
+    (255 where there is no candidate).  Per haplotype: ``loglik`` the sum of log10(w_hap) over the sites with
+    w_hap > 0, ``n_unsupported`` the sites with w_hap = 0, ``n_disagree`` the sites where best is not the
+    haplotype's allele."""
+
+    NO_CANDIDATE = 255
+
+    def __init__(self, weights, w_hap, w_second, best, loglik, n_unsupported, n_disagree):
+        self.weights, self.w_hap, self.w_second, self.best = weights, w_hap, w_second, best
+        self.loglik, self.n_unsupported, self.n_disagree = loglik, n_unsupported, n_disagree
+
+
 class Hansel:
     def __init__(self, symbols, unsymbols, n_snps, band_w=None, device=None, _handle=None,
                  v_site="from", candidates_skip_unsymbols=True):
@@ -423,6 +440,28 @@ class Hansel:
             *[a.ctypes.data if a is not None else None for a in per]))
         return ReadSupport(unique, shared, share_q32, int(totals[0]), int(totals[1]), int(totals[2]), *per)
 
+    # ---- path scores --------------------------------------------------------------------------
+    def score_paths(self, paths, L=None, weights=False):
+        """Score the haplotypes ``paths`` (uint8 [H][N+1] as recover_codes returns them: '_' at site 0, codes 0..6)
+        against this matrix: at every site the branch weights of get_edge_weights_at given the haplotype's earlier
+        alleles, with ``L`` (default: the matrix's L) and the matrix's flags, as recovery uses them (hx_score_paths).
+        The matrix is not changed.  -> PathScores."""
+        self.finalize()
+        paths = np.ascontiguousarray(paths, dtype=np.uint8)
+        if paths.ndim != 2 or paths.shape[1] != self.n_snps + 1:
+            raise ValueError("paths must be uint8 [n_haps][N+1]")
+        H, N = paths.shape[0], self.n_snps
+        w = np.zeros((H, N, 8), dtype=np.float64) if weights else None
+        w_hap, w_second = np.zeros((H, N), dtype=np.float64), np.zeros((H, N), dtype=np.float64)
+        best = np.zeros((H, N), dtype=np.uint8)
+        loglik = np.zeros(H, dtype=np.float64)
+        n_unsup, n_dis = np.zeros(H, dtype=np.int32), np.zeros(H, dtype=np.int32)
+        _lib.check(self._lib.hx_score_paths(
+            self._h, paths.ctypes.data, H, int(self.L if L is None else L), self.flags,
+            w.ctypes.data if w is not None else None, w_hap.ctypes.data, w_second.ctypes.data, best.ctypes.data,
+            loglik.ctypes.data, n_unsup.ctypes.data, n_dis.ctypes.data))
+        return PathScores(w, w_hap, w_second, best, loglik, n_unsup, n_dis)
+
     # ---- bulk I/O ----------------------------------------------------------------------------
     def band(self):
         """float32 [N+2][W][7][7]; cell (pi,pj) at [pj][pj-pi-1]."""
@@ -467,7 +506,8 @@ class Hansel:
 
     def kernel_ms(self, which):
         ms = C.c_float()
-        _lib.check(self._lib.hx_last_kernel_ms(self._h, {"ingest": 0, "walk": 1, "reweight": 2, "assign": 3}[which],
+        _lib.check(self._lib.hx_last_kernel_ms(self._h, {"ingest": 0, "walk": 1, "reweight": 2, "assign": 3,
+                                                                "score": 4}[which],
                                                C.byref(ms)))
         return float(ms.value)
 

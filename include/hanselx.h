@@ -194,6 +194,20 @@ int hx_assign_reads(hx_matrix *h, const uint8_t *haps, int32_t n_haps,
                     int32_t max_mismatch, int64_t *unique, int64_t *shared, uint64_t *share_q32,
                     int64_t totals[3], int32_t *best_mm, int32_t *n_best, int32_t *first_best);
 
+/* ---- path scores --------------------------------------------------------------------- */
+/* Per-site branch weights of given haplotypes (no reference counterpart; DESIGN.md §4 K6).  haps[n_haps*(N+1)] as
+ * hx_recover writes them.  Every per-site output is [n_haps*N] (site s of haplotype h at h*N + s-1) and may be NULL;
+ * weights is [n_haps*N*8] (7 normalised weights, then the total) or NULL.  loglik, n_unsupported, n_disagree: [n_haps].
+ * Site s of haplotype h gets exactly what hx_edge_weights_at(s, haps[h], L, flags) reports; best = the first maximum
+ * over the candidates (255: none); w_hap = the weight of the haplotype's own allele (0 if it is not a candidate);
+ * w_second = the largest weight of the other candidates (0 if none).  loglik = the sum of log10(w_hap) over the sites
+ * with w_hap > 0 in site order; n_unsupported = the sites with w_hap = 0; n_disagree = the sites with best != the
+ * haplotype's allele.  HX_E_ARG: a code > 6, or haps[h][0] != '_'.  The matrix's band and counts are not changed.
+ * Synchronous. */
+int hx_score_paths(hx_matrix *h, const uint8_t *haps, int32_t n_haps, int32_t L, int flags,
+                   double *weights, double *w_hap, double *w_second, uint8_t *best,
+                   double *loglik, int32_t *n_unsupported, int32_t *n_disagree);
+
 /* ---- BAM -> packed reads on the CPU (the producer side of the boundary) ------------ */
 /* Replaces the pysam column pileup of gretel/util.py:112-210: multi-threaded BGZF inflate and one
  * CIGAR walk per alignment against the sorted 1-based SNP positions.  stepper: 0 = samtools,
@@ -263,7 +277,7 @@ int hx_band_from_host(hx_matrix *h, const float *in);
 int hx_to_dense(hx_matrix *h, float *out /* 7*7*(N+2)*(N+2) */);
 /* last kernel timings in ms measured with CUDA events on the matrix's stream:
  * which = 0 ingest, 1 generate_path walk, 2 reweight, 3 the assignment kernels of the last hx_assign_reads
- * (copies excluded) */
+ * (copies excluded), 4 the scoring kernels of the last hx_score_paths (copies excluded) */
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms);
 /* number of kernel launches issued by this matrix so far */
 int hx_launch_count(const hx_matrix *h, int64_t *n);
