@@ -258,7 +258,10 @@ __device__ __forceinline__ int walk_q_range(const int32_t *__restrict__ termsq, 
     }
     unsigned mine = 0;                                      // lane's slot of the 32-site output block
     const int margin_q = 168;                               // 1.6e-4 * 2^20
-    const int floor_q = -300 * 1048576;                     // 10**x must stay representable
+    // 10**x must stay representable: outside (-300, 300) the exact evaluation decides, where a weight that underflows
+    // to 0 or overflows to inf (a lookback term is positive when V = 0 and the support is below 1) changes the
+    // normalised weights and so the first-max pick
+    const int floor_q = -300 * 1048576, ceil_q = 300 * 1048576;
     tr.wait(0);
     // lookback >= 2 terms of the first site (rows past the start of the region are zero), then its log marginal
     int R;
@@ -306,7 +309,7 @@ __device__ __forceinline__ int walk_q_range(const int32_t *__restrict__ termsq, 
             const int best = __reduce_max_sync(0xffffffffu, tot);
             const unsigned near = __ballot_sync(0xffffffffu, tot >= best - margin_q) & 0xffu;
             int next = 31 - __clz(near);                     // == ffs-1 when exactly one candidate is near
-            if ((near & (near - 1)) != 0 || best <= floor_q || force_exact) {
+            if ((near & (near - 1)) != 0 || best <= floor_q || best >= ceil_q || force_exact) {
                 const unsigned cmask = (unsigned)logm[(int64_t)snp * 8 + 7];
                 if (cmask == 0) next = -1;
                 else {

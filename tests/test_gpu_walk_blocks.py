@@ -18,10 +18,10 @@ import numpy as np
 import pytest
 
 from gretel_b200 import synth
+from tests.test_gpu_recover_switches import same_stats
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-RTOL = 1e-6
 MAX_K = 40                       # SNPs per read: the band is 39 wide, so every L <= 32 takes the fixed-point walk
 N_CAND = 5                       # earlier haplotypes a block may start from (HX_WALK_CAND - 1)
 
@@ -194,11 +194,6 @@ def redone(h):
     return n.value
 
 
-def _same_stats(got, exp, what):
-    for k, (g, e) in enumerate(zip(got, exp)):
-        assert g == pytest.approx(e, rel=1e-9 if k == 4 else RTOL), "%s: statistic %d: %r != %r" % (what, k, g, e)
-
-
 def check_case(c_oracle, c, n_res=6, n_gen=2, blocks=24, hole=None):
     """Both device entry points against the oracle loop: recover_codes (resident, earlier haplotypes as starts) for
     n_res haplotypes and generate_path_codes + reweight_path_codes (no earlier haplotypes) for n_gen.  `hole`: the
@@ -221,7 +216,7 @@ def check_case(c_oracle, c, n_res=6, n_gen=2, blocks=24, hole=None):
     for k, (p, s, e) in enumerate(zip(paths, stats, want)):
         bad = np.flatnonzero(p != e["path"])
         assert bad.size == 0, "resident haplotype %d differs from site %d on (%d sites)" % (k, bad[0], bad.size)
-        _same_stats(s, e["stats"], "resident haplotype %d" % k)
+        same_stats(s, e["stats"], N, W, "resident haplotype %d" % k)
     assert np.array_equal(h.band(), bands[len(want)]), "band after recover_codes"
     h.close()
 
@@ -242,7 +237,7 @@ def check_case(c_oracle, c, n_res=6, n_gen=2, blocks=24, hole=None):
         assert bad.size == 0, "haplotype %d differs from site %d on (%d sites)" % (k, bad[0], bad.size)
         ratio = max(got[3], 0.01)
         removed = h.reweight_path_codes(got[0], ratio)
-        _same_stats(got[1:] + (ratio, removed), its[k]["stats"], "haplotype %d" % k)
+        same_stats(got[1:] + (ratio, removed), its[k]["stats"], N, W, "haplotype %d" % k)
     assert np.array_equal(h.band(), bands[min(n_gen, len(its))]), "band after generate_path_codes"
     h.close()
 
