@@ -447,7 +447,10 @@ int hx_ingest_host_pipelined(hx_matrix *h, const int32_t *rank, const int64_t *o
         if (rc) return rc;
         if (!h->pin_ev[slot]) HX_CUDA(cudaEventCreateWithFlags(&h->pin_ev[slot], cudaEventDisableTiming));
         rc = hx_dense_pack(rank + a, off + a, codes, &P, h->pin[slot]);
-        if (rc) return rc;                         // HX_E_STATE: not sorted from here on; *done_reads went out already
+        // HX_E_STATE: not sorted from here on; *done_reads went out already.  HX_E_ARG: a read has more SNPs than the
+        // SNP-count width chosen from the band (W + 1 < 256: one byte) or a code > 6 - reads the device check refuses
+        // with HX_E_READ when they reach it, so a caller sees one status for them at every input size
+        if (rc) return rc == HX_E_ARG ? HX_E_READ : rc;
         rc = ensure_pin(P.bytes, P.head_bytes);
         if (rc) return rc;
         uint8_t *blob = h->pin[slot];

@@ -67,7 +67,8 @@ int hx_sync(hx_matrix *h);
 /* Host-buffer entry point (H2D + kernel + D2H of the totals), synchronous.
  * totals[4] = { n_slices (util.py:233), n_crumbs (util.py:268,276,281),
  *               covered_snps (util.py:239), sentinel increments }.
- * Counts accumulate over calls until hx_finalize_counts(). */
+ * Counts accumulate over calls until hx_finalize_counts().  HX_E_READ for a read that leaves [0,N], is wider
+ * than the band or has a code > 6, whatever the input size and HX_HOST_PIPELINE. */
 int hx_ingest_host(hx_matrix *h, const int32_t *rank, const int64_t *off, const uint8_t *codes,
                    int64_t n_reads, int64_t totals[4]);
 /* The same, in the compact wire format (half the host->device bytes): klen[r] = SNPs on read r,
