@@ -14,6 +14,8 @@ NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",
     "-fmad=false",                 # fp64 recovery arithmetic must round like the CPU oracle
+    # no -march for the host compiler: the x86-64 baseline has no FMA, so host fp64 (the EM of hx_em_abundance) is not
+    # contracted and rounds like the Python oracle
     "-Xcompiler", "-fPIC", "-shared",
     "-Xptxas", "-v",
 ]

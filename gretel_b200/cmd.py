@@ -6,7 +6,8 @@ Everything that computes (ingestion, gap check counts, recovery, reweighting) ru
 library; this file is host-side bookkeeping and output formatting only: PATHS de-duplication
 (cmd.py:164-179), out.fasta / snp.fasta (cmd.py:181-221) and gretel.crumbs (cmd.py:223-240,
 docs/protocol.rst:48-77), and with --support the reads carried by each haplotype (gretel.support, no reference
-counterpart); with --site-weights / --score the branch weights of every recovered haplotype and of known sequences,
+counterpart); with --abundance each haplotype's share of the reads by EM over read classes (gretel.abundance, no
+reference counterpart); with --site-weights / --score the branch weights of every recovered haplotype and of known sequences,
 site by site (gretel.sites, gretel.scores, no reference counterpart).
 """
 from __future__ import annotations
@@ -71,8 +72,12 @@ def build_parser():
     p.add_argument("--device", type=int, default=None)
     p.add_argument("--support", action="store_true",
                    help="write gretel.support: the reads each recovered haplotype carries")
+    p.add_argument("--abundance", action="store_true",
+                   help="write gretel.abundance: each recovered haplotype's share of the reads, by EM over the "
+                        "classes of reads tied between the same haplotypes")
     p.add_argument("--max-mismatch", type=int, default=-1,
-                   help="--support: a read whose best haplotype has more mismatches is not assigned (-1: no limit)")
+                   help="--support, --abundance: a read whose best haplotype has more mismatches is not assigned "
+                        "(-1: no limit)")
     p.add_argument("--site-weights", action="store_true",
                    help="write gretel.sites: per recovered haplotype and site the branch weights of its allele, of "
                         "the best candidate and of the runner-up; and gretel.scores: per haplotype its log "
@@ -84,8 +89,10 @@ def build_parser():
     return p
 
 
-def snp_table(hansel, vcf_h, out=sys.stdout):
-    """cmd.py:123-145."""
+def snp_table(hansel, vcf_h, out=None):
+    """cmd.py:123-145.  ``out`` defaults to the sys.stdout of the call, not of the import (a caller that swaps
+    sys.stdout after this module was first imported still gets the table)."""
+    out = sys.stdout if out is None else out
     out.write("i\tpos\tgap\tA\tC\tG\tT\tN\t-\t_\ttot\n")
     last_rev = 0
     for i in range(0, vcf_h["N"] + 1):
@@ -134,6 +141,20 @@ def write_support(dirn, records, totals):
                                                  r["share"] / totals["assigned"] if totals["assigned"] else 0.0))
 
 
+def write_abundance(dirn, records, totals):
+    """gretel.abundance: '# reads, assigned, uninformative, over_limit, max_mismatch, classes, iterations,
+    converged, loglik' (loglik in full precision), then per distinct haplotype in i_0 order: i_0, unique reads,
+    shared reads, EM reads, EM fraction."""
+    with open(dirn.rstrip("/") + "/gretel.abundance", "w") as fh:
+        fh.write("# %d\t%d\t%d\t%d\t%d\t%d\t%d\t%d\t%r\n" % (
+            totals["reads"], totals["assigned"], totals["uninformative"], totals["over_limit"],
+            totals["max_mismatch"], totals["classes"], totals["iterations"], totals["converged"],
+            float(totals["loglik"])))
+        for r in records:
+            fh.write("%d\t%d\t%d\t%.2f\t%.6f\n" % (r["i_0"], r["unique"], r["shared"], r["em_reads"],
+                                                  r["em_fraction"]))
+
+
 def write_scores(dirn, hansel, vcf_h, scored, site_weights):
     """gretel.scores: per scored path (recovered ones by i_0, then FASTA records by name) loglik, unsupported sites
     and sites whose best candidate is not the path's allele.  With site_weights, gretel.sites: per path and site
@@ -172,7 +193,7 @@ def main(argv=None):
         with open(args.dumpsnps, "w") as fh:
             for k in sorted(vcf_h["snp_fwd"].keys()):
                 fh.write("%d\t%d\t%d\n" % (vcf_h["snp_fwd"][k] + 1, k, k - args.start + 1))
-    reads = {} if args.support else None
+    reads = {} if args.support or args.abundance else None
     hansel = util.load_from_bam(args.bam, args.contig, args.start, args.end, vcf_h, n_threads=args.threads,
                                 stepper="all" if args.pepper else "samtools", device=args.device, reads=reads)
     if args.dumpmatrix:
@@ -193,6 +214,10 @@ def main(argv=None):
         records, totals = gretel.read_support(hansel, PATHS, reads["rank"], reads["off"], reads["codes"],
                                               max_mismatch=args.max_mismatch)
         write_support(args.out, records, totals)
+    if args.abundance:
+        records, totals = gretel.abundance(hansel, PATHS, reads["rank"], reads["off"], reads["codes"],
+                                           max_mismatch=args.max_mismatch)
+        write_abundance(args.out, records, totals)
     if args.site_weights or args.score:
         scored = [gretel.score_paths(original, PATHS, weights=args.site_weights)]
         if args.score:

@@ -229,6 +229,7 @@ int reset_parked(hx_matrix *h) {
     HX_CUDA(hx_fill_async(h->d_totals.p, 0, 8 * sizeof(unsigned long long), h->stream));
     HX_CUDA(hx_fill_async(h->d_err.p, 0, sizeof(int), h->stream));
     HX_CUDA(hx_fill_async(h->d_flags.p, 0, sizeof(hx_dev_flags), h->stream));
+    hx_classes_drop(h);
     h->use = {};
     return HX_OK;
 }
@@ -778,7 +779,7 @@ int hx_to_dense(hx_matrix *h, float *out) {
 }
 
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms) {
-    HX_CHECK_ARG(h && ms && which >= 0 && which < 5);
+    HX_CHECK_ARG(h && ms && which >= 0 && which < 6);
     *ms = h->use.last_ms[which];
     return HX_OK;
 }

@@ -93,6 +93,8 @@ struct hx_wire_set {
     cudaEvent_t copied, decoded, consumed;
 };
 
+struct hx_classes;                   // host-side read classes (support.cu)
+
 struct hx_matrix {
     int32_t N, W, device;
     int64_t band_elems;              // (N+2)*W*49
@@ -139,7 +141,13 @@ struct hx_matrix {
     // read support (support.cu): haplotype codes and bit-planes, the sums, one chunk of reads, per-read results
     HxDevBuf<uint8_t> a_haps; HxDevBuf<uint4> a_planes; HxDevBuf<unsigned long long> a_sums;
     HxDevBuf<int32_t> a_rank; HxDevBuf<int64_t> a_off; HxDevBuf<uint8_t> a_codes; HxDevBuf<int32_t> a_best;
-    cudaEvent_t a_ev[2];             // times the assignment kernels (hx_last_kernel_ms which = 3)
+    cudaEvent_t a_ev[2];             // times the assignment and class kernels (hx_last_kernel_ms which = 3, 5)
+    // read classes (support.cu): per read of a chunk the tie count, member offset, (first, D) and hash of a tied read;
+    // scan partials; per sub-batch the member pool, the table (representatives, counts), the compacted classes and
+    // their members, and their two counters
+    HxDevBuf<int64_t> cl_nb, cl_moff, cl_scan; HxDevBuf<int2> cl_tie; HxDevBuf<unsigned long long> cl_hash, cl_ncls;
+    HxDevBuf<int32_t> cl_pool, cl_rep, cl_out; HxDevBuf<unsigned> cl_cnt; HxDevBuf<int4> cl_cls;
+    hx_classes *a_cls;            // host-side classes of the last successful hx_read_classes (or null)
     // path scoring (score.cu): haplotype codes, per-site outputs of one chunk of haplotypes, per-haplotype sums
     HxDevBuf<uint8_t> sc_haps, sc_best; HxDevBuf<double> sc_site, sc_ll; HxDevBuf<int32_t> sc_cnt;
     cudaEvent_t sc_ev[2];            // times the scoring kernels (hx_last_kernel_ms which = 4)
@@ -159,7 +167,7 @@ struct hx_matrix {
         bool prepass_ran = false;    // d_flags->ingest_sorted holds the sortedness verdict of the last ingestion launch
         int wire_next = 0;           // the next staging set of the dense wire format
         bool sum_busy[2] = {};       // sum_done[b] marks ordered sums not yet joined into the main stream
-        float last_ms[5] = {};
+        float last_ms[6] = {};
     } use;
 };
 
@@ -282,5 +290,6 @@ void hx_l2_free(hx_matrix *h);
 int hx_ensure_counts(hx_matrix *h);
 // support.cu
 void hx_support_free(hx_matrix *h);
+void hx_classes_drop(hx_matrix *h);      // forgets the classes of the last hx_read_classes
 // score.cu
 void hx_score_free(hx_matrix *h);

@@ -108,6 +108,38 @@ def read_support(hansel, PATHS, rank, off, codes, max_mismatch=-1):
     return records, totals
 
 
+def abundance(hansel, PATHS, rank, off, codes, max_mismatch=-1, max_iter=10000, tol=1e-12):
+    """How abundant each recovered haplotype is: the packed reads are grouped into compatibility classes over the
+    distinct paths of ``PATHS`` (Hansel.read_classes) and each path's share of the assigned reads is estimated by EM
+    over the classes (hansel.em_abundance).  Unlike read_support's equal split, a read tied between paths goes to
+    them in proportion to their estimated abundance.  Returns (records, totals): one dict per path in ``i_0`` order
+    with i_0, unique, shared, em_reads (= em_fraction * assigned) and em_fraction, and a dict with reads, assigned,
+    uninformative, over_limit, max_mismatch, classes, iterations, converged and loglik.  With no path no read is
+    assigned, as in read_support."""
+    from .hansel import em_abundance
+    keys = sorted(PATHS, key=lambda x: PATHS[x]["i_0"])
+    if not keys:
+        _, totals = read_support(hansel, PATHS, rank, off, codes, max_mismatch=max_mismatch)
+        totals.update(classes=0, iterations=0, converged=True, loglik=0.0)
+        return [], totals
+    paths = np.stack([hansel.encode_path(PATHS[k]["hansel_path"]) for k in keys])
+    cls = hansel.read_classes(paths, rank, off, codes, max_mismatch=max_mismatch)
+    em = em_abundance(len(keys), cls, max_iter=max_iter, tol=tol)
+    size = np.diff(cls.class_off)
+    of_class = np.repeat(np.arange(len(cls)), size)
+    unique = np.bincount(cls.members[size[of_class] == 1], weights=cls.count[of_class][size[of_class] == 1],
+                         minlength=len(keys)).astype(np.int64)
+    shared = np.bincount(cls.members[size[of_class] >= 2], weights=cls.count[of_class][size[of_class] >= 2],
+                         minlength=len(keys)).astype(np.int64)
+    totals = {"reads": len(rank), "assigned": cls.assigned, "uninformative": cls.uninformative,
+              "over_limit": cls.over_limit, "max_mismatch": int(max_mismatch), "classes": len(cls),
+              "iterations": em.n_iter, "converged": em.converged, "loglik": em.loglik}
+    records = [{"i_0": PATHS[k]["i_0"], "unique": int(unique[j]), "shared": int(shared[j]),
+                "em_reads": float(em.pi[j] * cls.assigned), "em_fraction": float(em.pi[j])}
+               for j, k in enumerate(keys)]
+    return records, totals
+
+
 def score_paths(hansel, PATHS, weights=False):
     """Score the distinct recovered paths of ``PATHS`` in ``i_0`` order (the order of out.fasta) against ``hansel``
     (Hansel.score_paths).  Score against the matrix recovery started from (``original_hansel``): recovery reweights

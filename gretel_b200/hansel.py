@@ -47,6 +47,54 @@ class ReadSupport:
         self.best_mm, self.n_best, self.first_best = best_mm, n_best, first_best
 
 
+class ReadClasses:
+    """What Hansel.read_classes reports: the compatibility classes of the assigned reads (DESIGN.md §4 K7) as CSR.
+    Class c has the haplotypes ``members[class_off[c]:class_off[c+1]]`` (int32, ascending), the tie set of its
+    reads, and ``count[c]`` reads (int64, >= 1); classes are ordered lexicographically by member list.  Totals
+    ``assigned`` (the sum of ``count``), ``uninformative`` and ``over_limit`` as in ReadSupport."""
+
+    def __init__(self, class_off, members, count, assigned, uninformative, over_limit):
+        self.class_off, self.members, self.count = class_off, members, count
+        self.assigned, self.uninformative, self.over_limit = assigned, uninformative, over_limit
+
+    def __len__(self):
+        return len(self.count)
+
+    def classes(self):
+        """[(member tuple, count)] in class order."""
+        o = self.class_off
+        return [(tuple(int(x) for x in self.members[o[c]:o[c + 1]]), int(self.count[c])) for c in range(len(self))]
+
+
+class Abundance:
+    """What em_abundance reports: ``pi`` float64 [n_haps] (each haplotype's share of the assigned reads), ``n_iter``
+    (iterations run), ``converged`` (the last change of pi was <= tol) and ``loglik`` (the sum over classes of
+    count * log10 of the class's summed pi)."""
+
+    def __init__(self, pi, n_iter, converged, loglik):
+        self.pi, self.n_iter, self.converged, self.loglik = pi, n_iter, converged, loglik
+
+
+def em_abundance(n_haps, classes, max_iter=10000, tol=1e-12):
+    """Each haplotype's share of the reads by EM over read classes (``classes``: a ReadClasses, or a
+    (class_off, members, count) triple), in float64 and the fixed operation order of DESIGN.md §4 K7
+    (hx_em_abundance; host code, needs no GPU).  -> Abundance."""
+    if isinstance(classes, ReadClasses):
+        classes = (classes.class_off, classes.members, classes.count)
+    class_off, members, count = classes
+    class_off = np.ascontiguousarray(class_off, dtype=np.int64)
+    members = np.ascontiguousarray(members, dtype=np.int32)
+    count = np.ascontiguousarray(count, dtype=np.int64)
+    if len(class_off) != len(count) + 1:
+        raise ValueError("class_off must have len(count)+1 entries")
+    pi = np.zeros(max(int(n_haps), 0), dtype=np.float64)
+    n_iter, conv, ll = C.c_int32(), C.c_int32(), C.c_double()
+    _lib.check(_lib.load().hx_em_abundance(int(n_haps), len(count), class_off.ctypes.data, members.ctypes.data,
+                                           count.ctypes.data, int(max_iter), float(tol), pi.ctypes.data,
+                                           C.byref(n_iter), C.byref(conv), C.byref(ll)))
+    return Abundance(pi, int(n_iter.value), bool(conv.value), float(ll.value))
+
+
 class PathScores:
     """What Hansel.score_paths reports for H haplotypes over sites 1..N; per-site arrays are [H][N], site s at
     column s-1.  ``weights`` float64 [H][N][8] (the 7 normalised branch weights of Hansel.get_edge_weights_at at the
@@ -440,6 +488,30 @@ class Hansel:
             *[a.ctypes.data if a is not None else None for a in per]))
         return ReadSupport(unique, shared, share_q32, int(totals[0]), int(totals[1]), int(totals[2]), *per)
 
+    def read_classes(self, paths, rank, off, codes, max_mismatch=-1):
+        """Group the assigned reads into compatibility classes: the reads whose tie sets B (assign_reads) are equal
+        form one class (hx_read_classes).  Inputs as for assign_reads; the matrix's counts are not touched.
+        -> ReadClasses."""
+        paths = np.ascontiguousarray(paths, dtype=np.uint8)
+        if paths.ndim != 2 or paths.shape[1] != self.n_snps + 1:
+            raise ValueError("paths must be uint8 [n_haps][N+1]")
+        rank = np.ascontiguousarray(rank, dtype=np.int32)
+        off = np.ascontiguousarray(off, dtype=np.int64)
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        if len(off) != len(rank) + 1:
+            raise ValueError("off must have len(rank)+1 entries")
+        totals = np.zeros(3, dtype=np.int64)
+        n_cls, n_mem = C.c_int64(), C.c_int64()
+        _lib.check(self._lib.hx_read_classes(
+            self._h, paths.ctypes.data, paths.shape[0], rank.ctypes.data, off.ctypes.data, codes.ctypes.data,
+            len(rank), int(max_mismatch), totals.ctypes.data, C.byref(n_cls), C.byref(n_mem)))
+        class_off = np.zeros(n_cls.value + 1, dtype=np.int64)
+        members = np.zeros(n_mem.value, dtype=np.int32)
+        count = np.zeros(n_cls.value, dtype=np.int64)
+        _lib.check(self._lib.hx_read_classes_get(self._h, class_off.ctypes.data, members.ctypes.data,
+                                                 count.ctypes.data))
+        return ReadClasses(class_off, members, count, int(totals[0]), int(totals[1]), int(totals[2]))
+
     # ---- path scores --------------------------------------------------------------------------
     def score_paths(self, paths, L=None, weights=False):
         """Score the haplotypes ``paths`` (uint8 [H][N+1] as recover_codes returns them: '_' at site 0, codes 0..6)
@@ -507,7 +579,7 @@ class Hansel:
     def kernel_ms(self, which):
         ms = C.c_float()
         _lib.check(self._lib.hx_last_kernel_ms(self._h, {"ingest": 0, "walk": 1, "reweight": 2, "assign": 3,
-                                                                "score": 4}[which],
+                                                                "score": 4, "classes": 5}[which],
                                                C.byref(ms)))
         return float(ms.value)
 

@@ -195,6 +195,31 @@ int hx_assign_reads(hx_matrix *h, const uint8_t *haps, int32_t n_haps,
                     int32_t max_mismatch, int64_t *unique, int64_t *shared, uint64_t *share_q32,
                     int64_t totals[3], int32_t *best_mm, int32_t *n_best, int32_t *first_best);
 
+/* ---- read classes and abundances -------------------------------------------------- */
+/* Compatibility classes of the assigned reads (no reference counterpart; DESIGN.md §4 K7).  Inputs, informative
+ * sites, assignment and errors as for hx_assign_reads; HX_E_ARG also for n_haps < 1.  Every assigned read adds 1 to the
+ * class keyed by its tie set B (the haplotypes at its fewest mismatches, ascending); singletons {h} are classes too.
+ * Only classes with a count >= 1 exist, ordered lexicographically by member list.  totals[3] = {assigned,
+ * uninformative, over_limit}; *n_classes and *n_members size the arrays of hx_read_classes_get.  The classes are
+ * kept in the handle until the next call (an error leaves none).  Synchronous; the band and the counts are neither
+ * read nor changed.  HX_CLASS_HASH_BITS (default 64) masks the class hash and HX_CLASS_SCRATCH_MB (default 256)
+ * bounds the scratch of one sub-batch of tied reads; neither changes any result. */
+int hx_read_classes(hx_matrix *h, const uint8_t *haps, int32_t n_haps, const int32_t *rank, const int64_t *off,
+                    const uint8_t *codes, int64_t n_reads, int32_t max_mismatch, int64_t totals[3],
+                    int64_t *n_classes, int64_t *n_members);
+/* The classes of the last hx_read_classes as CSR: class_off[n_classes+1], members[n_members] (int32), count[n_classes]
+ * (int64).  HX_E_STATE if there are none. */
+int hx_read_classes_get(hx_matrix *h, int64_t *class_off, int32_t *members, int64_t *count);
+/* EM over classes (DESIGN.md §4 K7): the share pi[n_haps] of each haplotype, in float64 in a fixed operation order,
+ * from pi = 1/n_haps for at most max_iter iterations, stopping at the first whose largest change is <= tol.
+ * *n_iter = iterations run, *converged = (that change <= tol), *loglik = sum of count * log10(sum of pi over the
+ * class).  No class (T = 0): pi = 0, n_iter = 0, loglik = 0, converged.  Host code; needs no GPU.  HX_E_ARG:
+ * n_haps < 1, tol < 0, max_iter < 0, a count < 1, a class without members, a member out of [0,n_haps), members of a
+ * class not strictly ascending, classes not strictly lexicographically ascending. */
+int hx_em_abundance(int32_t n_haps, int64_t n_classes, const int64_t *class_off, const int32_t *members,
+                    const int64_t *count, int32_t max_iter, double tol, double *pi, int32_t *n_iter,
+                    int32_t *converged, double *loglik);
+
 /* ---- path scores --------------------------------------------------------------------- */
 /* Per-site branch weights of given haplotypes (no reference counterpart; DESIGN.md §4 K6).  haps[n_haps*(N+1)] as
  * hx_recover writes them.  Every per-site output is [n_haps*N] (site s of haplotype h at h*N + s-1) and may be NULL;
@@ -278,7 +303,8 @@ int hx_band_from_host(hx_matrix *h, const float *in);
 int hx_to_dense(hx_matrix *h, float *out /* 7*7*(N+2)*(N+2) */);
 /* last kernel timings in ms measured with CUDA events on the matrix's stream:
  * which = 0 ingest, 1 generate_path walk, 2 reweight, 3 the assignment kernels of the last hx_assign_reads
- * (copies excluded), 4 the scoring kernels of the last hx_score_paths (copies excluded) */
+ * (copies excluded), 4 the scoring kernels of the last hx_score_paths (copies excluded), 5 the class kernels of the
+ * last hx_read_classes (copies excluded) */
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms);
 /* number of kernel launches issued by this matrix so far */
 int hx_launch_count(const hx_matrix *h, int64_t *n);
