@@ -12,7 +12,7 @@ HX_OK, HX_HOLE = 0, 1
 HX_E_CUDA, HX_E_ARG, HX_E_BAND, HX_E_READ, HX_E_NOMEM, HX_E_STATE = -1, -2, -3, -4, -5, -6
 HX_F_VSITE_TO, HX_F_KEEP_UNSYMBOLS = 1, 2
 
-_p, _i32, _i64, _int, _dbl, _flt = C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_double, C.c_float
+_p, _i32, _i64, _u64, _int, _dbl, _flt = C.c_void_p, C.c_int32, C.c_int64, C.c_uint64, C.c_int, C.c_double, C.c_float
 _pp = C.POINTER(C.c_void_p)
 
 # name -> (restype, argtypes); must list every symbol include/hanselx.h declares
@@ -61,6 +61,7 @@ SIGNATURES = {
     "hx_read_classes": (_int, [_p, _p, _i32, _p, _p, _p, _i64, _i32, _p, _p, _p]),
     "hx_read_classes_get": (_int, [_p, _p, _p, _p]),
     "hx_em_abundance": (_int, [_i32, _i64, _p, _p, _p, _i32, _dbl, _p, _p, _p, _p]),
+    "hx_em_bootstrap": (_int, [_p, _i32, _i64, _p, _p, _p, _i32, _u64, _i32, _dbl, _p, _p, _p, _p, _p]),
     "hx_score_paths": (_int, [_p, _p, _i32, _i32, _int, _p, _p, _p, _p, _p, _p, _p]),
     "hx_pack_bam": (_int, [C.c_char_p, C.c_char_p, _i32, _i32, _p, _i32, _int, _int, _p]),
     "hx_pack_bam_ex": (_int, [C.c_char_p, C.c_char_p, _i32, _i32, _p, _i32, _int, _int, _i32, _p, _p]),

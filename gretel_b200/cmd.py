@@ -7,7 +7,8 @@ library; this file is host-side bookkeeping and output formatting only: PATHS de
 (cmd.py:164-179), out.fasta / snp.fasta (cmd.py:181-221) and gretel.crumbs (cmd.py:223-240,
 docs/protocol.rst:48-77), and with --support the reads carried by each haplotype (gretel.support, no reference
 counterpart); with --abundance each haplotype's share of the reads by EM over read classes (gretel.abundance, no
-reference counterpart); with --site-weights / --score the branch weights of every recovered haplotype and of known sequences,
+reference counterpart), and with --bootstrap its bootstrap mean, standard deviation and 95 % interval
+(gretel.bootstrap); with --site-weights / --score the branch weights of every recovered haplotype and of known sequences,
 site by site (gretel.sites, gretel.scores, no reference counterpart).
 """
 from __future__ import annotations
@@ -75,6 +76,11 @@ def build_parser():
     p.add_argument("--abundance", action="store_true",
                    help="write gretel.abundance: each recovered haplotype's share of the reads, by EM over the "
                         "classes of reads tied between the same haplotypes")
+    p.add_argument("--bootstrap", type=int, default=0, metavar="B",
+                   help="with --abundance: also write gretel.bootstrap, the mean, standard deviation and 95 %% "
+                        "interval of each haplotype's share over B bootstrap resamples of the reads")
+    p.add_argument("--bootstrap-seed", type=int, default=0, metavar="S",
+                   help="--bootstrap: the seed of the resampling (the same seed gives the same replicates)")
     p.add_argument("--max-mismatch", type=int, default=-1,
                    help="--support, --abundance: a read whose best haplotype has more mismatches is not assigned "
                         "(-1: no limit)")
@@ -155,6 +161,16 @@ def write_abundance(dirn, records, totals):
                                                   r["em_fraction"]))
 
 
+def write_bootstrap(dirn, records, totals):
+    """gretel.bootstrap: '# replicates, seed, converged_replicates', then per distinct haplotype in i_0 order: i_0,
+    EM fraction, and the bootstrap mean, standard deviation, 2.5 % and 97.5 % quantiles of the fraction."""
+    with open(dirn.rstrip("/") + "/gretel.bootstrap", "w") as fh:
+        fh.write("# %d\t%d\t%d\n" % (totals["replicates"], totals["seed"], totals["boot_converged"]))
+        for r in records:
+            fh.write("%d\t%.6f\t%.6f\t%.6f\t%.6f\t%.6f\n" % (r["i_0"], r["em_fraction"], r["boot_mean"], r["boot_sd"],
+                                                            r["boot_lo"], r["boot_hi"]))
+
+
 def write_scores(dirn, hansel, vcf_h, scored, site_weights):
     """gretel.scores: per scored path (recovered ones by i_0, then FASTA records by name) loglik, unsupported sites
     and sites whose best candidate is not the path's allele.  With site_weights, gretel.sites: per path and site
@@ -184,7 +200,12 @@ def write_scores(dirn, hansel, vcf_h, scored, site_weights):
 
 
 def main(argv=None):
-    args = build_parser().parse_args(argv)
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if args.bootstrap < 0:
+        parser.error("--bootstrap must be >= 0")
+    if args.bootstrap > 0 and not args.abundance:
+        parser.error("--bootstrap needs --abundance")
     if args.end == -1:
         args.end = util.get_ref_len_from_bam(args.bam, args.contig)
         sys.stderr.write("[NOTE] Setting end_pos to %d" % args.end)
@@ -216,8 +237,11 @@ def main(argv=None):
         write_support(args.out, records, totals)
     if args.abundance:
         records, totals = gretel.abundance(hansel, PATHS, reads["rank"], reads["off"], reads["codes"],
-                                           max_mismatch=args.max_mismatch)
+                                           max_mismatch=args.max_mismatch, n_boot=args.bootstrap,
+                                           seed=args.bootstrap_seed)
         write_abundance(args.out, records, totals)
+        if args.bootstrap > 0:
+            write_bootstrap(args.out, records, totals)
     if args.site_weights or args.score:
         scored = [gretel.score_paths(original, PATHS, weights=args.site_weights)]
         if args.score:

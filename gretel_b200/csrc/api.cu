@@ -142,6 +142,7 @@ void free_all(hx_matrix *h) {
     hx_wire_free(h);
     hx_support_free(h);
     hx_score_free(h);
+    hx_boot_free(h);
     if (h->d_peer_tbl) cudaFree(h->d_peer_tbl);
     cudaStream_t st = h->stream;
     h->band.release(st);
@@ -779,7 +780,7 @@ int hx_to_dense(hx_matrix *h, float *out) {
 }
 
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms) {
-    HX_CHECK_ARG(h && ms && which >= 0 && which < 6);
+    HX_CHECK_ARG(h && ms && which >= 0 && which < 8);
     *ms = h->use.last_ms[which];
     return HX_OK;
 }

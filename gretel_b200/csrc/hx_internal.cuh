@@ -141,13 +141,18 @@ struct hx_matrix {
     // read support (support.cu): haplotype codes and bit-planes, the sums, one chunk of reads, per-read results
     HxDevBuf<uint8_t> a_haps; HxDevBuf<uint4> a_planes; HxDevBuf<unsigned long long> a_sums;
     HxDevBuf<int32_t> a_rank; HxDevBuf<int64_t> a_off; HxDevBuf<uint8_t> a_codes; HxDevBuf<int32_t> a_best;
-    cudaEvent_t a_ev[2];             // times the assignment and class kernels (hx_last_kernel_ms which = 3, 5)
+    cudaEvent_t a_ev[2];             // times the assignment, class and bootstrap kernels (hx_last_kernel_ms which = 3, 5-7)
     // read classes (support.cu): per read of a chunk the tie count, member offset, (first, D) and hash of a tied read;
     // scan partials; per sub-batch the member pool, the table (representatives, counts), the compacted classes and
     // their members, and their two counters
     HxDevBuf<int64_t> cl_nb, cl_moff, cl_scan; HxDevBuf<int2> cl_tie; HxDevBuf<unsigned long long> cl_hash, cl_ncls;
     HxDevBuf<int32_t> cl_pool, cl_rep, cl_out; HxDevBuf<unsigned> cl_cnt; HxDevBuf<int4> cl_cls;
     hx_classes *a_cls;            // host-side classes of the last successful hx_read_classes (or null)
+    // bootstrap (bootstrap.cu): the classes (offsets, members, counts, prefix sums of the counts), the haplotype-major
+    // lists of member entries (offsets, class of each entry); per batch of replicates the resampled counts, pi, the
+    // class sums when they do not fit in shared memory, n_iter + converged, and loglik
+    HxDevBuf<int64_t> bt_off, bt_cnt0, bt_pre, bt_hoff; HxDevBuf<int32_t> bt_mem, bt_hcls, bt_it;
+    HxDevBuf<unsigned long long> bt_cnt; HxDevBuf<double> bt_pi, bt_z, bt_ll;
     // path scoring (score.cu): haplotype codes, per-site outputs of one chunk of haplotypes, per-haplotype sums
     HxDevBuf<uint8_t> sc_haps, sc_best; HxDevBuf<double> sc_site, sc_ll; HxDevBuf<int32_t> sc_cnt;
     cudaEvent_t sc_ev[2];            // times the scoring kernels (hx_last_kernel_ms which = 4)
@@ -167,7 +172,7 @@ struct hx_matrix {
         bool prepass_ran = false;    // d_flags->ingest_sorted holds the sortedness verdict of the last ingestion launch
         int wire_next = 0;           // the next staging set of the dense wire format
         bool sum_busy[2] = {};       // sum_done[b] marks ordered sums not yet joined into the main stream
-        float last_ms[6] = {};
+        float last_ms[8] = {};
     } use;
 };
 
@@ -215,6 +220,21 @@ static inline cudaError_t hx_fill_async(void *p, int byte, size_t bytes, cudaStr
     return cudaGetLastError();
 }
 #endif
+
+// Device time of one kernel launch on the matrix's stream, added to timer `which` of hx_last_kernel_ms.
+template <class Launch>
+static int timed(hx_matrix *h, int which, Launch launch) {
+    HX_CUDA(cudaEventRecord(h->a_ev[0], h->stream));
+    launch();
+    h->use.launches++;
+    HX_CUDA(cudaGetLastError());
+    HX_CUDA(cudaEventRecord(h->a_ev[1], h->stream));
+    HX_CUDA(cudaEventSynchronize(h->a_ev[1]));
+    float ms = 0.0f;
+    HX_CUDA(cudaEventElapsedTime(&ms, h->a_ev[0], h->a_ev[1]));
+    h->use.last_ms[which] += ms;
+    return HX_OK;
+}
 
 __host__ __device__ __forceinline__ int64_t hx_cell_off(int64_t W, int64_t pi, int64_t pj) {
     return (pj * W + (pj - pi - 1)) * HX_CELL;
@@ -291,5 +311,9 @@ int hx_ensure_counts(hx_matrix *h);
 // support.cu
 void hx_support_free(hx_matrix *h);
 void hx_classes_drop(hx_matrix *h);      // forgets the classes of the last hx_read_classes
+int hx_check_classes(int32_t n_haps, int64_t n_classes, const int64_t *class_off, const int32_t *members,
+                     const int64_t *count, int64_t *total);
+// bootstrap.cu
+void hx_boot_free(hx_matrix *h);
 // score.cu
 void hx_score_free(hx_matrix *h);

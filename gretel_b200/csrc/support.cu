@@ -347,21 +347,6 @@ k_class_compact(uint32_t S, const int32_t *__restrict__ slot_rep, const unsigned
 
 }  // namespace
 
-// Device time of one kernel launch on the matrix's stream, added to timer `which` of hx_last_kernel_ms.
-template <class Launch>
-static int timed(hx_matrix *h, int which, Launch launch) {
-    HX_CUDA(cudaEventRecord(h->a_ev[0], h->stream));
-    launch();
-    h->use.launches++;
-    HX_CUDA(cudaGetLastError());
-    HX_CUDA(cudaEventRecord(h->a_ev[1], h->stream));
-    HX_CUDA(cudaEventSynchronize(h->a_ev[1]));
-    float ms = 0.0f;
-    HX_CUDA(cudaEventElapsedTime(&ms, h->a_ev[0], h->a_ev[1]));
-    h->use.last_ms[which] += ms;
-    return HX_OK;
-}
-
 void hx_support_free(hx_matrix *h) {
     cudaStream_t st = h->stream;
     h->a_haps.release(st); h->a_planes.release(st); h->a_sums.release(st);
@@ -685,14 +670,9 @@ extern "C" int hx_read_classes_get(hx_matrix *h, int64_t *class_off, int32_t *me
     return HX_OK;
 }
 
-// The EM of DESIGN.md §4 K7, in exactly its operation order, so that oracle/abundance_oracle.py reproduces it bit for
-// bit.  Host code: the classes are few.  No step may be contracted to an FMA: the x86-64 baseline the library is
-// built for has none, and build.py passes no -march that would add it.
-extern "C" int hx_em_abundance(int32_t n_haps, int64_t n_classes, const int64_t *class_off, const int32_t *members,
-                               const int64_t *count, int32_t max_iter, double tol, double *pi, int32_t *n_iter,
-                               int32_t *converged, double *loglik) {
-    HX_CHECK_ARG(n_haps >= 1 && n_classes >= 0 && max_iter >= 0 && tol >= 0.0 && pi && n_iter && converged && loglik);
-    HX_CHECK_ARG(n_classes == 0 || (class_off && members && count));
+// The CSR checks of hx_em_abundance and hx_em_bootstrap (HX_E_ARG), and T = the sum of the counts.
+int hx_check_classes(int32_t n_haps, int64_t n_classes, const int64_t *class_off, const int32_t *members,
+                     const int64_t *count, int64_t *total) {
     const int H = n_haps;
     int64_t T = 0;
     if (n_classes) HX_CHECK_ARG(class_off[0] == 0);
@@ -708,6 +688,21 @@ extern "C" int hx_em_abundance(int32_t n_haps, int64_t n_classes, const int64_t 
             HX_CHECK_ARG(std::lexicographical_compare(members + class_off[c - 1], members + a, members + a, members + b));
         T += count[c];
     }
+    *total = T;
+    return HX_OK;
+}
+
+// The EM of DESIGN.md §4 K7, in exactly its operation order, so that oracle/abundance_oracle.py reproduces it bit for
+// bit.  Host code: the classes are few.  No step may be contracted to an FMA: the x86-64 baseline the library is
+// built for has none, and build.py passes no -march that would add it.
+extern "C" int hx_em_abundance(int32_t n_haps, int64_t n_classes, const int64_t *class_off, const int32_t *members,
+                               const int64_t *count, int32_t max_iter, double tol, double *pi, int32_t *n_iter,
+                               int32_t *converged, double *loglik) {
+    HX_CHECK_ARG(n_haps >= 1 && n_classes >= 0 && max_iter >= 0 && tol >= 0.0 && pi && n_iter && converged && loglik);
+    HX_CHECK_ARG(n_classes == 0 || (class_off && members && count));
+    const int H = n_haps;
+    int64_t T = 0;
+    if (const int rc = hx_check_classes(H, n_classes, class_off, members, count, &T)) return rc;
     if (T == 0) {
         for (int h = 0; h < H; ++h) pi[h] = 0.0;
         *n_iter = 0;

@@ -108,19 +108,25 @@ def read_support(hansel, PATHS, rank, off, codes, max_mismatch=-1):
     return records, totals
 
 
-def abundance(hansel, PATHS, rank, off, codes, max_mismatch=-1, max_iter=10000, tol=1e-12):
+def abundance(hansel, PATHS, rank, off, codes, max_mismatch=-1, max_iter=10000, tol=1e-12, n_boot=0, seed=0):
     """How abundant each recovered haplotype is: the packed reads are grouped into compatibility classes over the
     distinct paths of ``PATHS`` (Hansel.read_classes) and each path's share of the assigned reads is estimated by EM
     over the classes (hansel.em_abundance).  Unlike read_support's equal split, a read tied between paths goes to
     them in proportion to their estimated abundance.  Returns (records, totals): one dict per path in ``i_0`` order
     with i_0, unique, shared, em_reads (= em_fraction * assigned) and em_fraction, and a dict with reads, assigned,
     uninformative, over_limit, max_mismatch, classes, iterations, converged and loglik.  With no path no read is
-    assigned, as in read_support."""
+    assigned, as in read_support.  With ``n_boot`` > 0 the EM is also run on ``n_boot`` bootstrap resamples of the
+    assigned reads on the GPU (Hansel.em_bootstrap with ``seed``): each record gains boot_mean, boot_sd (ddof = 1; 0
+    for one replicate), boot_lo and boot_hi (the 2.5 % and 97.5 % quantiles) of its fraction over the replicates,
+    and the totals gain replicates, seed and boot_converged (the replicates whose EM converged).  The point estimate
+    stays em_abundance's."""
     from .hansel import em_abundance
     keys = sorted(PATHS, key=lambda x: PATHS[x]["i_0"])
     if not keys:
         _, totals = read_support(hansel, PATHS, rank, off, codes, max_mismatch=max_mismatch)
         totals.update(classes=0, iterations=0, converged=True, loglik=0.0)
+        if n_boot > 0:
+            totals.update(replicates=int(n_boot), seed=int(seed), boot_converged=int(n_boot))
         return [], totals
     paths = np.stack([hansel.encode_path(PATHS[k]["hansel_path"]) for k in keys])
     cls = hansel.read_classes(paths, rank, off, codes, max_mismatch=max_mismatch)
@@ -137,7 +143,19 @@ def abundance(hansel, PATHS, rank, off, codes, max_mismatch=-1, max_iter=10000, 
     records = [{"i_0": PATHS[k]["i_0"], "unique": int(unique[j]), "shared": int(shared[j]),
                 "em_reads": float(em.pi[j] * cls.assigned), "em_fraction": float(em.pi[j])}
                for j, k in enumerate(keys)]
+    if n_boot > 0:
+        boot = hansel.em_bootstrap(len(keys), cls, n_boot, seed=seed, max_iter=max_iter, tol=tol)
+        for j, r in enumerate(records):
+            r.update(boot_summary(boot.pi[1:, j]))
+        totals.update(replicates=int(n_boot), seed=int(seed), boot_converged=int(boot.converged[1:].sum()))
     return records, totals
+
+
+def boot_summary(x):
+    """boot_mean, boot_sd (ddof = 1, 0.0 for one value), boot_lo and boot_hi (the 2.5 % and 97.5 % quantiles) of the
+    replicate fractions ``x``."""
+    return {"boot_mean": float(np.mean(x)), "boot_sd": float(np.std(x, ddof=1)) if len(x) > 1 else 0.0,
+            "boot_lo": float(np.quantile(x, 0.025)), "boot_hi": float(np.quantile(x, 0.975))}
 
 
 def score_paths(hansel, PATHS, weights=False):

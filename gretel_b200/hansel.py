@@ -79,6 +79,27 @@ def em_abundance(n_haps, classes, max_iter=10000, tol=1e-12):
     """Each haplotype's share of the reads by EM over read classes (``classes``: a ReadClasses, or a
     (class_off, members, count) triple), in float64 and the fixed operation order of DESIGN.md §4 K7
     (hx_em_abundance; host code, needs no GPU).  -> Abundance."""
+    class_off, members, count = _csr(classes)
+    pi = np.zeros(max(int(n_haps), 0), dtype=np.float64)
+    n_iter, conv, ll = C.c_int32(), C.c_int32(), C.c_double()
+    _lib.check(_lib.load().hx_em_abundance(int(n_haps), len(count), class_off.ctypes.data, members.ctypes.data,
+                                           count.ctypes.data, int(max_iter), float(tol), pi.ctypes.data,
+                                           C.byref(n_iter), C.byref(conv), C.byref(ll)))
+    return Abundance(pi, int(n_iter.value), bool(conv.value), float(ll.value))
+
+
+class Bootstrap:
+    """What Hansel.em_bootstrap reports for B replicates over H haplotypes: row 0 is the EM on the classes' counts
+    (em_abundance, bit for bit), row b >= 1 the EM on a multinomial resample of the assigned reads (DESIGN.md §4 K8).
+    ``pi`` float64 [B+1][H], ``n_iter`` int32 [B+1], ``converged`` bool [B+1], ``loglik`` float64 [B+1], and
+    ``count`` int64 [B+1][C] (each row's class counts; row 0 = the input counts) or None."""
+
+    def __init__(self, pi, n_iter, converged, loglik, count=None):
+        self.pi, self.n_iter, self.converged, self.loglik, self.count = pi, n_iter, converged, loglik, count
+
+
+def _csr(classes):
+    """A ReadClasses or (class_off, members, count) -> contiguous int64 / int32 / int64 arrays."""
     if isinstance(classes, ReadClasses):
         classes = (classes.class_off, classes.members, classes.count)
     class_off, members, count = classes
@@ -87,12 +108,7 @@ def em_abundance(n_haps, classes, max_iter=10000, tol=1e-12):
     count = np.ascontiguousarray(count, dtype=np.int64)
     if len(class_off) != len(count) + 1:
         raise ValueError("class_off must have len(count)+1 entries")
-    pi = np.zeros(max(int(n_haps), 0), dtype=np.float64)
-    n_iter, conv, ll = C.c_int32(), C.c_int32(), C.c_double()
-    _lib.check(_lib.load().hx_em_abundance(int(n_haps), len(count), class_off.ctypes.data, members.ctypes.data,
-                                           count.ctypes.data, int(max_iter), float(tol), pi.ctypes.data,
-                                           C.byref(n_iter), C.byref(conv), C.byref(ll)))
-    return Abundance(pi, int(n_iter.value), bool(conv.value), float(ll.value))
+    return class_off, members, count
 
 
 class PathScores:
@@ -512,6 +528,24 @@ class Hansel:
                                                  count.ctypes.data))
         return ReadClasses(class_off, members, count, int(totals[0]), int(totals[1]), int(totals[2]))
 
+    def em_bootstrap(self, n_haps, classes, n_boot, seed=0, max_iter=10000, tol=1e-12, counts=False):
+        """Bootstrap of the abundance EM on the GPU (hx_em_bootstrap): row 0 is em_abundance on ``classes`` (a
+        ReadClasses or a (class_off, members, count) triple), row b = 1..n_boot the same EM on the counts of a
+        resample of the assigned reads with replacement, drawn by Philox4x32-10 keyed by ``seed`` (uint64).  Every row
+        depends only on (classes, seed, b).  The matrix supplies the device; its counts are not touched.
+        -> Bootstrap (``count`` with counts=True)."""
+        class_off, members, count = _csr(classes)
+        H, R, Cn = max(int(n_haps), 0), max(int(n_boot), 0) + 1, len(count)
+        pi = np.zeros((R, H), dtype=np.float64)
+        n_iter, conv = np.zeros(R, dtype=np.int32), np.zeros(R, dtype=np.int32)
+        ll = np.zeros(R, dtype=np.float64)
+        cnt = np.zeros((R, Cn), dtype=np.int64) if counts else None
+        _lib.check(self._lib.hx_em_bootstrap(
+            self._h, int(n_haps), Cn, class_off.ctypes.data, members.ctypes.data, count.ctypes.data, int(n_boot),
+            int(seed) & 0xFFFFFFFFFFFFFFFF, int(max_iter), float(tol), pi.ctypes.data, n_iter.ctypes.data,
+            conv.ctypes.data, ll.ctypes.data, cnt.ctypes.data if counts else None))
+        return Bootstrap(pi, n_iter, conv.astype(bool), ll, cnt)
+
     # ---- path scores --------------------------------------------------------------------------
     def score_paths(self, paths, L=None, weights=False):
         """Score the haplotypes ``paths`` (uint8 [H][N+1] as recover_codes returns them: '_' at site 0, codes 0..6)
@@ -579,7 +613,8 @@ class Hansel:
     def kernel_ms(self, which):
         ms = C.c_float()
         _lib.check(self._lib.hx_last_kernel_ms(self._h, {"ingest": 0, "walk": 1, "reweight": 2, "assign": 3,
-                                                                "score": 4, "classes": 5}[which],
+                                                                "score": 4, "classes": 5, "resample": 6,
+                                                                "bootstrap_em": 7}[which],
                                                C.byref(ms)))
         return float(ms.value)
 

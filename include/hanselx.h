@@ -219,6 +219,15 @@ int hx_read_classes_get(hx_matrix *h, int64_t *class_off, int32_t *members, int6
 int hx_em_abundance(int32_t n_haps, int64_t n_classes, const int64_t *class_off, const int32_t *members,
                     const int64_t *count, int32_t max_iter, double tol, double *pi, int32_t *n_iter,
                     int32_t *converged, double *loglik);
+/* Bootstrap of the abundance EM (DESIGN.md §4 K8).  Classes, max_iter, tol and the HX_E_ARG rules as for
+ * hx_em_abundance; also HX_E_ARG for n_boot < 0.  Row 0 = the EM on count (== hx_em_abundance bit for bit); row b >= 1
+ * = the EM on count_b, the multinomial resample of the T assigned reads drawn by Philox4x32-10 keyed by seed.
+ * pi[(n_boot+1)*n_haps], n_iter / converged / loglik [n_boot+1]; boot_count[(n_boot+1)*n_classes] or NULL.
+ * Synchronous.  The band, the counts and the classes held by the handle are neither read nor changed.
+ * HX_BOOT_SCRATCH_MB (default 256) bounds the device scratch of one batch of replicates; it changes no result. */
+int hx_em_bootstrap(hx_matrix *h, int32_t n_haps, int64_t n_classes, const int64_t *class_off, const int32_t *members,
+                    const int64_t *count, int32_t n_boot, uint64_t seed, int32_t max_iter, double tol,
+                    double *pi, int32_t *n_iter, int32_t *converged, double *loglik, int64_t *boot_count);
 
 /* ---- path scores --------------------------------------------------------------------- */
 /* Per-site branch weights of given haplotypes (no reference counterpart; DESIGN.md §4 K6).  haps[n_haps*(N+1)] as
@@ -304,7 +313,8 @@ int hx_to_dense(hx_matrix *h, float *out /* 7*7*(N+2)*(N+2) */);
 /* last kernel timings in ms measured with CUDA events on the matrix's stream:
  * which = 0 ingest, 1 generate_path walk, 2 reweight, 3 the assignment kernels of the last hx_assign_reads
  * (copies excluded), 4 the scoring kernels of the last hx_score_paths (copies excluded), 5 the class kernels of the
- * last hx_read_classes (copies excluded) */
+ * last hx_read_classes (copies excluded), 6 the resampling kernels and 7 the EM kernels of the last hx_em_bootstrap
+ * (copies excluded) */
 int hx_last_kernel_ms(hx_matrix *h, int which, float *ms);
 /* number of kernel launches issued by this matrix so far */
 int hx_launch_count(const hx_matrix *h, int64_t *n);
